@@ -1,6 +1,6 @@
 """Headline benchmark: HTSAT-tiny + ResiDual (all layers) inference, clips/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): HTSAT-tiny CLAP audio encoder with ResiDual injected in every block of all four
 layers (reference-faithful doubled FFN, src/residual.py:91-96), batch 256 synthetic 10 s / 48 kHz clips per GPU,
@@ -229,10 +229,11 @@ def run_reference(args):
         print(json.dumps({"impl": "reference", "unavailable": f"no CPU reference arm for --workload {wl} (only infer and train are timed)"}), flush=True)
         return
     one, kind, desc = make_cpu_step(wl, B)
-    for _ in range(max(1, min(args.warmup, 2))):
+    warm = max(1, min(args.warmup, 2))
+    for _ in range(warm):
         one()
     t0 = time.perf_counter()
-    steps = max(1, min(args.steps, 12))
+    steps = args.steps
     for _ in range(steps):
         one()
     dt = time.perf_counter() - t0
@@ -241,7 +242,7 @@ def run_reference(args):
               f"{torch.get_num_threads()} threads")
     cfg = config_dict(256, wl)
     cfg["reference_sample"] = {"clips_per_step": B, "steps": steps, "note": "throughput of the CPU arm is per clip; 8-clip steps keep the run bounded"}
-    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": args.warmup,
+    line = {"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": steps, "warmup": warm,
             "ms_per_step": 1e3 * dt / steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
             "data": "synthetic", "config": cfg,
             "cpu_baseline": {"value": v, "unit": UNIT, "cores": torch.get_num_threads(), "kind": kind, "sample": sample},
@@ -316,6 +317,8 @@ class Workload:
             cls = torch.nn.Linear(512, 50).to(dev)
             params = [r.learnable for r in residuals.values()] + list(cls.parameters())
             opt = torch.optim.Adam(params, lr=1e-3)
+            self.trained = {f"lambda{l}": r.learnable for l, r in residuals.items()}
+            self.trained.update(classifier_weight=cls.weight, classifier_bias=cls.bias)
             labels = torch.randint(0, 50, (B,), device=dev, generator=torch.Generator(device=dev).manual_seed(5 + rank))
             self.comm = {"collective": "allreduce(sum) of one flat fp32 buffer: lambda grads + classifier grads",
                          "floats": int(sum(p.numel() for p in params)), "comm_nranks": world}
@@ -357,6 +360,25 @@ class Workload:
             self.e2e_step = lambda host: pca_step(host.to(dev, non_blocking=True)).cpu()
             self.e2e_api = "encode(want_dict=True) + MomentAccumulator.update per layer and per (layer, head); mean vector .cpu()"
             self.e2e_dtype = torch.float32
+
+    def outputs(self, out):
+        """What a caller of the step holds after it, given `out` = what step() returned: the audio embeddings; for the training step
+        the loss and the updated lambdas and classifier; for the PCA statistics every accumulator's moments {n, sum x, sum x x^T},
+        the per-(layer, head) attention moments stacked per layer."""
+        import torch
+        if self.wl == "train":
+            return dict(loss=out, **self.trained)
+        if self.wl != "pca":
+            return {"audio_embed": out}
+        res = {}
+        f64 = dict(dtype=torch.float64)
+        for l in range(4):
+            r, heads = self.res_acc[l], self.attn_acc[l]
+            res.update({f"layer{l}_residual_n": torch.tensor(float(r.n), **f64), f"layer{l}_residual_s1": r.s1, f"layer{l}_residual_s2": r.s2,
+                        f"layer{l}_attention_n": torch.tensor([float(a.n) for a in heads], **f64),
+                        f"layer{l}_attention_s1": torch.stack([a.s1 for a in heads]),
+                        f"layer{l}_attention_s2": torch.stack([a.s2 for a in heads])})
+        return res
 
     def host_batch(self):
         """Pinned host copy of this rank's clips in the dtype the e2e route takes (int16 PCM = quantize_tensor's integers)."""
@@ -402,9 +424,11 @@ class RankGuard:
             self.dist.barrier(group=self.group)
 
 
-def measure(wl, B, K, Wm, dev, rank, world, dist, do_e2e=True, do_profile=True, sampler=None, precision="bf16", guard=None):
+def measure(wl, B, K, Wm, dev, rank, world, dist, do_e2e=True, do_profile=True, sampler=None, precision="bf16", guard=None,
+            dump_dir=None):
     """W warm-up + K timed steps of workload `wl` (CUDA events, barrier + synchronize on both sides, max over ranks), then the
-    e2e leg and the per-class launch profile. Returns a dict (same on every rank except the rank-0-only profile)."""
+    e2e leg and the per-class launch profile. Returns a dict (same on every rank except the rank-0-only profile). With dump_dir,
+    rank 0 writes the outputs of the last timed step there (dump_outputs) before anything else runs on the workload."""
     import torch
     from audio_residual_b200 import lib as L
     if guard is not None:
@@ -443,6 +467,8 @@ def measure(wl, B, K, Wm, dev, rank, world, dist, do_e2e=True, do_profile=True, 
     res = {"workload": wl, "value": world * B * K / (ms_total / 1e3), "ms_per_step": ms_total / K, "steps": K, "warmup": Wm,
            "launches_per_step": int(launches_per_step), "clocks": clocks, "comm": w.comm,
            "checksum": float(out.double().abs().sum().item()), "precision": precision}
+    if dump_dir is not None and rank == 0:
+        dump_outputs(dump_dir, w.outputs(out))
 
     if do_e2e:
         host = w.host_batch()
@@ -580,6 +606,32 @@ def _measure_guarded(wl, B, K, Wm, dev, rank, world, precision, guard):
             "precision": precision, "_workload_obj": w}
 
 
+DUMP_LIMIT_BYTES = 64 * 10**6      # all files of one dump, .npy headers included
+NPY_HEADER_BYTES = 1024            # reserved per file; np.save writes 128 bytes for these shapes
+
+
+def dump_outputs(path, arrays):
+    """Writes each tensor of `arrays` as <path>/<name>.npy, float64 where the workload computes in float64 and float32 otherwise, so
+    that two builds run with the same arguments (hence the same seeded inputs and weights) can be compared output for output.
+    Smallest first, an array is stored whole when it fits its share of the budget still left; a larger one is replaced by a sample
+    of its flattened elements at indices drawn from a fixed seed, so the same elements are stored on every run."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    left = DUMP_LIMIT_BYTES
+    todo = sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(todo):
+        t = t.detach()
+        t = t.double() if t.dtype == torch.float64 else t.float()
+        fit = (left // (len(todo) - i) - NPY_HEADER_BYTES) // t.element_size()
+        if t.numel() > fit:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), fit, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        left -= a.nbytes + NPY_HEADER_BYTES
+
+
 def pin_rank_to_cores(local_rank, world):
     """One contiguous block of host cores per rank (torchrun does not pin). Measured on an 8-GPU box with 32 vCPUs: un-pinned, three
     of the eight ranks spent 20 ms per e2e call against 12.4-12.8 ms for the others - their Python threads were what their GPUs
@@ -615,7 +667,7 @@ def run_ours(args):
     if sampler is not None:
         sampler.start()          # started before warm-up so nvidia-smi is already streaming when the timed region begins
     guard = RankGuard(dist, world)
-    main = measure(wl, B, K, Wm, dev, rank, world, dist, sampler=sampler)
+    main = measure(wl, B, K, Wm, dev, rank, world, dist, sampler=sampler, dump_dir=args.dump_outputs)
     main.pop("_workload_obj", None)
     torch.cuda.empty_cache()
 
@@ -732,7 +784,13 @@ def main():
                     help="infer = the headline (BASELINE configs[1]); the others measure configs[2..4] with the same JSON contract")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the extra records (train / pca / base_fusion / fp32 at this N)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rank 0) as DIR/<name>.npy (--impl ours)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

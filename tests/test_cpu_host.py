@@ -197,10 +197,14 @@ def test_csv_schema_roundtrip(tmp_path):
 
 
 def test_real_reference_pca_fixture_schema():
-    """The reference ships real PCA pickles (residual_pca/ESC50/layer_*_evalfold_*); when mounted, they must load."""
-    p = "/root/reference/residual_pca/ESC50/layer_0_evalfold_0"
+    """The reference ships real PCA pickles (residual_pca/ESC50/layer_*_evalfold_*); they must load. This repository does not store
+    them, and oracle/build_ref.py does not snapshot them, so the test runs only against a full reference
+    checkout that oracle/refimport.py finds (ARD_REFERENCE_ROOT). The pickle schema itself is checked on every run with synthetic
+    pickles by test_load_residual_reads_reference_fixture_schema."""
+    from oracle import refimport
+    p = os.path.join(refimport.REF, "residual_pca", "ESC50", "layer_0_evalfold_0")
     if not os.path.exists(p):
-        pytest.skip("reference fixtures not mounted")
+        pytest.skip("needs a full reference checkout (ARD_REFERENCE_ROOT): its PCA pickles are not stored in this repository")
     r = load_residual(p)
     assert r.basis.shape == (96, 96) and r.mean.shape == (96,)
     assert torch.allclose(r.basis @ r.basis.T, torch.eye(96), atol=1e-4)
@@ -369,17 +373,50 @@ def test_apply_criterion_routes_custom_losses_to_the_caller():
     assert torch.equal(apply_criterion(lambda a, b: a.sum(), z, y), z.sum())
 
 
-def test_reference_snapshot_recipe(tmp_path):
-    """oracle/build_ref.py: the snapshot holds what oracle/refimport.py needs (skipped when /root/reference is not mounted)."""
+def test_reference_snapshot_recipe(tmp_path, monkeypatch):
+    """oracle/build_ref.py: the snapshot holds what oracle/refimport.py needs. The reference sources are not part of this
+    repository, so the recipe runs on a stand-in tree with the reference's layout and writes its snapshot under tmp_path."""
     from oracle import build_ref
-    if not os.path.isdir(os.path.join(build_ref.SRC, "CLAP")):
-        pytest.skip("reference tree not mounted")
+    src, dst = tmp_path / "reference", tmp_path / "_ref"
+    monkeypatch.setattr(build_ref, "SRC", str(src))
+    monkeypatch.setattr(build_ref, "DST", str(dst))
+    assert not build_ref.build(verbose=False)                      # no reference tree and no snapshot yet
+    cm = "CLAP/src/laion_clap/clap_module/"
+    for rel in (cm + "htsat.py", cm + "model.py", cm + "utils.py", cm + "model_configs/HTSAT-tiny.json", cm + "model_configs/HTSAT-base.json",
+                "CLAP/src/laion_clap/training/data.py", "src/residual.py"):
+        (src / rel).parent.mkdir(parents=True, exist_ok=True)
+        (src / rel).write_text(rel)
     assert build_ref.build(verbose=False)
     for rel in ("CLAP/src/laion_clap/clap_module/htsat.py", "CLAP/src/laion_clap/clap_module/model.py", "CLAP/src/laion_clap/training/data.py",
                 "src/residual.py", "CLAP/src/laion_clap/clap_module/model_configs/HTSAT-tiny.json"):
         assert os.path.exists(os.path.join(build_ref.DST, rel)), rel
+        assert open(os.path.join(build_ref.DST, rel)).read() == rel
     ign = open(os.path.join(ROOT, ".gitignore")).read()
     assert "oracle/_ref/" in ign                                   # reference sources never enter the history
+
+
+def test_bench_dump_outputs_budget_and_sampling(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float64 stays float64, other dtypes become float32; arrays that fit their share of the budget are
+    stored whole, larger ones as the elements at seeded indices (the same on every run); one dump's files stay within the budget."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 200_000)
+    g = torch.Generator().manual_seed(0)
+    arrays = {"n": torch.tensor(7.0, dtype=torch.float64), "small": torch.randn(10, 8, generator=g),
+              "big64": torch.randn(300, 300, generator=g, dtype=torch.float64), "big16": torch.randn(200, 200, generator=g).to(torch.bfloat16)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    total = sum(os.path.getsize(tmp_path / "a" / f) for f in os.listdir(tmp_path / "a"))
+    assert sorted(os.listdir(tmp_path / "a")) == ["big16.npy", "big64.npy", "n.npy", "small.npy"] and total <= 200_000
+    for name, t in arrays.items():
+        a, b = np.load(tmp_path / "a" / f"{name}.npy"), np.load(tmp_path / "b" / f"{name}.npy")
+        assert np.array_equal(a, b) and a.dtype == (np.float64 if t.dtype == torch.float64 else np.float32)
+        full = (t.double() if t.dtype == torch.float64 else t.float()).numpy()
+        if name in ("n", "small"):
+            assert np.array_equal(a, full)
+        else:
+            assert a.ndim == 1 and 0 < a.size < full.size
+            idx = np.sort(np.random.default_rng(0).choice(full.size, a.size, replace=False))
+            assert np.array_equal(a, full.reshape(-1)[idx])
 
 
 def test_gram_route_spectrum_equals_covariance_spectrum():

@@ -1,3 +1,3 @@
 #!/bin/bash
 # rebuild libard_b200.so from the repo root (cwd-independent)
-cd /root/repo && python __graft_entry__.py "$@"
+cd "$(dirname "$0")/.." && python __graft_entry__.py "$@"
