@@ -380,8 +380,6 @@ static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_
     if (!a->embedding) return set_error(ARD_ERR_SHAPE, "embedding output is required");
     if (a->precision != 0 && a->precision != 1) return set_error(ARD_ERR_SHAPE, "precision must be 0 (bf16) or 1 (fp32-grade), got %d", a->precision);
     const bool fp32 = a->precision == 1;
-    if (fp32 && a->save_for_backward)
-        return set_error(ARD_ERR_NOTIMPL, "the training step (save_for_backward) runs on the bf16 path; precision=1 is inference only");
     const int C0 = h->cfg.embed_dim;
     ARD_TRY(ensure_workspace(h, B));
     float* X = h->ws_x.as<float>();
@@ -389,7 +387,7 @@ static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_
     const bool train = a->save_for_backward != 0;
     h->tape_B = train ? h->tape_B : 0;   // an inference forward overwrites the head activations the backward would read
     if (train) {
-        ARD_TRY(ensure_tape(h, B));
+        ARD_TRY(ensure_tape(h, B, a->precision));
         ++h->tape_gen;
         X = h->layers[0].blocks[0].t_s;
     }
@@ -408,7 +406,7 @@ static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_
                                h->bn_shift.as<float>(), h->pe_w.as<float>(), h->pe_b.as<float>(), h->pe_g.as<float>(), h->pe_beta.as<float>(),
                                X, B, C0, s));
     }
-    // ---- swin stages
+    // ---- swin stages (fp32-grade: the training forward writes the fp32 tape there)
     if (fp32) ARD_TRY(encoder_stages_fp32(h, a, X, Y, &X, s));
     for (int l = 0; l < h->nlayers && !fp32; ++l) {
         const int C = C_of(h, l), R = R_of(l), T = R * R, depth = h->cfg.depths[l];
@@ -769,7 +767,7 @@ long long ard_workspace_bytes(const ard_handle* h) {
     if (!h) return 0;
     const DevBuf* bufs[] = {&h->ws_logmel, &h->ws_x, &h->ws_y, &h->ws_xn, &h->ws_ao, &h->ws_qkv, &h->ws_h, &h->ws_normed,
                             &h->ws_emb, &h->ws_hid, &h->ws_proj, &h->ws_tscam_a, &h->ws_tscam_y, &h->ws_wave, &h->tape, &h->bw_g,
-                            &h->bw_gs, &h->bw_t, &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small};
+                            &h->bw_gs, &h->bw_t, &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small, &h->bw_g3};
     long long t = 0;
     for (const DevBuf* b : bufs) t += (long long)b->bytes;
     return t;
@@ -862,6 +860,13 @@ int ard_window_attention_bwd(const void* qkv_bf16, const void* dout_bf16, void* 
     AttnArgs a;
     a.qkv = (const __nv_bfloat16*)qkv_bf16; a.bias_table = bias_table; a.B = B; a.H = H; a.W = W; a.C = C; a.nH = nH; a.shift = shift;
     return window_attention_bwd(a, (const __nv_bfloat16*)dout_bf16, (__nv_bfloat16*)dqkv_bf16, (cudaStream_t)stream);
+}
+
+int ard_window_attention_f32_bwd(const float* qkv_f32, const float* dout_f32, float* dqkv_f32, const float* bias_table, int B, int H, int W,
+                                 int C, int nH, int shift, void* stream) {
+    if (!qkv_f32 || !dout_f32 || !dqkv_f32 || !bias_table) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd: null argument");
+    if (H != W) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd: square token grids only (H=%d W=%d)", H, W);
+    return window_attention_f32_bwd(qkv_f32, dout_f32, dqkv_f32, bias_table, B, H, C, nH, shift, (cudaStream_t)stream);
 }
 
 int ard_layernorm_bwd(const float* x, const float* grad_out, const float* gamma, const float* add, float* grad_in, long long rows, int C,

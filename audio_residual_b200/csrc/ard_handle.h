@@ -51,9 +51,11 @@ struct BlockW {
     int Kp = 0;
     bool bwd_ready = false;
     DevBuf lam, fc1_wT, fc2_wT, qkv_wT, proj_wT, res_wc, res_wcT, res_basis_bf16, res_c0;
-    // activations saved by a save_for_backward forward (views into ard_handle::tape)
+    // activations saved by a save_for_backward forward (views into ard_handle::tape); qkv / ao are bf16 on a bf16 tape
+    // (t_qkv, t_ao) and fp32 on an fp32-grade tape (t_qkvf, t_aof), the other pair is null
     float *t_s = nullptr, *t_x1 = nullptr, *t_x3 = nullptr, *t_out = nullptr;
     __nv_bfloat16 *t_qkv = nullptr, *t_ao = nullptr;
+    float *t_qkvf = nullptr, *t_aof = nullptr;
 };
 struct LayerW {
     std::vector<BlockW> blocks;
@@ -90,7 +92,9 @@ struct ard_handle {
     // training state
     DevBuf tape, p0_wT, p2_wT, t_emb, t_hid, t_proj;
     DevBuf bw_g, bw_gs, bw_t, bw_hpre, bw_dh, bw_gqkv, bw_gb, bw_coef, bw_gcoef, bw_gsc, bw_small;
+    DevBuf bw_g3;            // fp32-grade backward: split form [hi | hi | lo] of the gradient entering a dgrad GEMM
     int tape_B = 0;          // batch of the forward whose activations the tape holds (0: none)
+    int tape_prec = 0;       // ard_forward_args.precision of that forward: the layout of the tape and the backward schedule
     long long tape_gen = 0;  // serial number of that forward (ard_tape_generation): a backward built on an older one is refused
     // CUDA-graph replay of the inference forward (ard_api.cu): the ~110 launches of a forward cost ~1.1 ms of fixed launch /
     // ramp latency whatever the batch; replaying a captured graph removes the host side of that and most of the device side.
@@ -135,7 +139,7 @@ int get(const ard_handle* h, const std::string& key, size_t numel, const std::ve
 int ensure_workspace(ard_handle* h, int B);
 int ensure_fold(ard_handle* h, int l, int b, cudaStream_t s);
 // training (ard_train.cu)
-int ensure_tape(ard_handle* h, int B);
+int ensure_tape(ard_handle* h, int B, int precision);
 int run_block_train(ard_handle* h, int l, int b, int B, float* attn_out, float attn_scale, int attn_acc, float* res_out,
                     long long res_bstride, cudaStream_t s);
 int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s);
@@ -144,7 +148,30 @@ int attn_block_pack(AttnBlockW& w, const std::vector<float>& qkv_w, const std::v
 int attn_block_pad_proj(const __nv_bfloat16* w, const float* bp, const float* bv, __nv_bfloat16* out, float* bp_eff, int C, int nH, cudaStream_t s);
 int attn_block_96(const float* x, float* out, const AttnBlockW& w, const __nv_bfloat16* wp_pad, const float* bp, const float* gamma,
                   const float* beta, int B, int R, int shift, int num_sms, cudaStream_t stream);
-// fp32-grade mode (fp32_mode.cu)
+// fp32-grade mode (fp32_mode.cu). Split weights [W_hi | W_lo | W_hi] ([N, 3K] bf16) of the forward GEMMs and, built on the
+// first fp32-grade backward, of the backward's dgrad GEMMs; all rebuilt when ard_handle::graph_epoch moves.
+struct Fp32BlockW {
+    DevBuf qkv3, proj3, fc13, fc23;
+    DevBuf fc1T3, fc2T3, qkvT3, projT3;                // [C, 3*4C], [4C, 3C], [C, 3*3C] (q rows pre-scaled), [C, 3C]
+    DevBuf wc3, wcT3, basis3;                          // ResiDual: Wc = B Wp [Kp, 3C], Wc^T [C, 3Kp], basis padded to Kp [Kp, 3C]
+};
+struct Fp32Weights {
+    unsigned long long epoch = ~0ULL;            // ard_handle::graph_epoch the split weights were built at (weights / ResiDual changes bump it)
+    unsigned long long bwd_epoch = ~0ULL;        // the same for the backward set (built by the first fp32-grade backward after a change)
+    std::vector<std::vector<Fp32BlockW>> blocks;
+    std::vector<DevBuf> merge3, mergeT3;         // PatchMerging reduction [2C, 3*4C] and its transpose [4C, 3*2C] (backward, lazily)
+    DevBuf tscam3, scratch;
+    DevBuf qkvf, aof, s3;                        // workspace: fp32 [M,4C] (qkv / FFN hidden), fp32 [M,C], split operands [M,12C] bf16
+};
+int fp32_weights(ard_handle* h, Fp32Weights** out, cudaStream_t s);   // the handle's split weights, forward set current
+int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s);
+int split3_weight_host(const std::vector<float>& w, DevBuf& scratch, DevBuf& out, long long N, int K, cudaStream_t s, float scale = 1.0f,
+                       long long scaled_rows = 0);
+int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, int ldo, long long M, int N, const float* bias, int act,
+          const float* r1, const float* r2, float* aux, int aux_T, long long aux_bstride, int num_sms, cudaStream_t s);
+int gelu_bwd_split3(const float* g, const float* hpre, __nv_bfloat16* out3, long long rows, int N, cudaStream_t s);
+int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, const float* bias_table, int B, int R, int C, int nH, int shift,
+                             cudaStream_t s);
 int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, float* Y, float** x_final, cudaStream_t s);
 int tscam_gemm_fp32(ard_handle* h, const float* normed, float* y, int ldy, int B, cudaStream_t s);
 void fp32_release(const ard_handle* h);

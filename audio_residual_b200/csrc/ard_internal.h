@@ -152,9 +152,10 @@ int residual_matrix(const float* basis, const float* lam, int C, int K, float* M
 int tscam_im2col(const float* normed, __nv_bfloat16* A, int B, int C, cudaStream_t s);
 int tscam_finish(const float* y, int ldy, float* framewise, float* clipwise, int B, int NC, cudaStream_t s);
 int fine_grained(const float* normed, float* fine, int B, int C, cudaStream_t s);
-// dlam[k] += sum_t coef[t,k] gcoef[t,k] (k < K; dlam may be NULL), gsc[t,k] = bf16(gcoef[t,k] lam[k]) (k < Kp); rows are Kp wide
+// dlam[k] += sum_t coef[t,k] gcoef[t,k] (k < K; dlam may be NULL), gsc[t,k] = bf16(gcoef[t,k] lam[k]) (k < Kp); rows are Kp wide.
+// split3: gsc rows are 3 Kp wide, [hi | hi | lo] of gcoef * lam (fp32-grade backward)
 int lambda_grad(const float* coef, const float* gcoef, const float* lam, float* dlam, __nv_bfloat16* gsc, long long M, int K, int Kp,
-                cudaStream_t s);
+                cudaStream_t s, bool split3 = false);
 int head_output_tap(const __nv_bfloat16* ao, float* tap, int B, int R, int C, int nH, int shift, cudaStream_t s);   // extras.cu
 int stats_accumulate(const float* x, long long rows, long long ldx, int D, double* sum, double* sumsq, cudaStream_t s);   // stats.cu
 

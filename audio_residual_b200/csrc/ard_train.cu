@@ -10,8 +10,12 @@
 //   s   fp32 [M,C]   block input (= previous block's output buffer, no copy)
 //   x1  fp32 [M,C]   s + r                 (input of the first norm2/FFN)
 //   x3  fp32 [M,C]   s + x1 + mlp(n2(x1))  (input of the second norm2/FFN, patched blocks only)
-//   qkv bf16 [M,3C], ao bf16 [M,C]  attention input / output in token order
+//   qkv bf16 [M,3C], ao bf16 [M,C]  attention input / output in token order (fp32 on the fp32-grade tape, precision = 1)
 // LayerNorm outputs, the FFN hidden pre-activation and the attention probabilities are recomputed in the backward.
+//
+// fp32-grade training (precision = 1): the forward is the fp32-grade mode (fp32_mode.cu) writing the same tape slots, and the
+// backward mirrors the bf16 schedule step for step with every dgrad a 3-term split-bf16 GEMM (gemm3) and everything between
+// the GEMMs fp32: the attention backward on CUDA cores, gelu' and the lambda product writing the split form directly.
 #include <string.h>
 
 #include "ard_handle.h"
@@ -33,8 +37,10 @@ int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bflo
 static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
 
 // Carve the tape: every block's output buffer is the next block's `s`; the last block of a layer writes the PatchMerging input.
-int ensure_tape(ard_handle* h, int B) {
-    if (h->tape_B == B && h->tape.p) return 0;
+// precision 0 keeps qkv / ao in bf16 (20 B per token-channel per block), 1 in fp32 (28 B).
+int ensure_tape(ard_handle* h, int B, int precision) {
+    if (h->tape_B == B && h->tape_prec == precision && h->tape.p) return 0;
+    const size_t act_bytes = precision ? 4 : 2;
     size_t total = 0;
     for (int pass = 0; pass < 2; ++pass) {
         uint8_t* base = h->tape.as<uint8_t>();
@@ -52,8 +58,12 @@ int ensure_tape(ard_handle* h, int B) {
                 bw.t_s = cur_in;
                 bw.t_x1 = (float*)take(MC * 4);
                 bw.t_x3 = (float*)take(MC * 4);
-                bw.t_qkv = (__nv_bfloat16*)take(MC * 3 * 2);
-                bw.t_ao = (__nv_bfloat16*)take(MC * 2);
+                void* qkv = take(MC * 3 * act_bytes);
+                void* ao = take(MC * act_bytes);
+                bw.t_qkv = precision ? nullptr : (__nv_bfloat16*)qkv;
+                bw.t_ao = precision ? nullptr : (__nv_bfloat16*)ao;
+                bw.t_qkvf = precision ? (float*)qkv : nullptr;
+                bw.t_aof = precision ? (float*)ao : nullptr;
                 bw.t_out = (float*)take(MC * 4);
                 cur_in = bw.t_out;
             }
@@ -66,6 +76,7 @@ int ensure_tape(ard_handle* h, int B) {
         }
     }
     h->tape_B = B;
+    h->tape_prec = precision;
     return 0;
 }
 
@@ -77,6 +88,39 @@ static int transpose_upload_bf16(DevBuf& dst, const float* w, int rows, int cols
         for (int c = 0; c < cols; ++c) t[(size_t)c * rows + r] = __float2bfloat16_rn(w[(size_t)r * cols + c] * sc);
     }
     return upload(dst, t.data(), t.size() * 2);
+}
+
+// The ResiDual and the projection fold for the backward too:  with  Wc = B Wp [K,C],  c0 = B (b_p - mu) [K]
+//   coef  = x_proj              = ao Wc^T + c0        (src/residual.py:37-38)
+//   d ao  = (gcoef * lambda) Wc                        (src/residual.py:39-40 then the proj Linear)
+// Host fp32, rows padded to Kp = K rounded up to 16: wc [Kp, C], c0 [Kp], bpad (the basis) [Kp, C].
+static int residual_backward_fold(ard_handle* h, int l, int b, std::vector<float>& wc, std::vector<float>& c0, std::vector<float>& bpad) {
+    BlockW& bw = h->layers[l].blocks[b];
+    const int C = C_of(h, l), K = bw.K, Kp = (K + 15) & ~15;
+    char pfx[64];
+    snprintf(pfx, sizeof(pfx), "layers.%d.blocks.%d.", l, b);
+    const std::string p(pfx);
+    const std::vector<float>* pw = nullptr;
+    const std::vector<float>* pb = nullptr;
+    ARD_TRY(get(h, p + "attn.proj.weight", (size_t)C * C, &pw));
+    ARD_TRY(get(h, p + "attn.proj.bias", C, &pb));
+    wc.assign((size_t)Kp * C, 0.f);
+    c0.assign(Kp, 0.f);
+    bpad.assign((size_t)Kp * C, 0.f);
+    for (int k = 0; k < K; ++k) {
+        const float* bk = bw.h_basis.data() + (size_t)k * C;
+        float* o = wc.data() + (size_t)k * C;
+        double acc0 = 0.0;
+        for (int c = 0; c < C; ++c) {
+            const float bv = bk[c];
+            const float* wr = pw->data() + (size_t)c * C;
+            for (int j = 0; j < C; ++j) o[j] += bv * wr[j];
+            acc0 += (double)bv * ((double)(*pb)[c] - (double)bw.h_mean[c]);
+        }
+        c0[k] = (float)acc0;
+        memcpy(bpad.data() + (size_t)k * C, bk, (size_t)C * 4);
+    }
+    return 0;
 }
 
 static int ensure_backward_weights(ard_handle* h, int l, int b) {
@@ -97,33 +141,69 @@ static int ensure_backward_weights(ard_handle* h, int l, int b) {
     ARD_TRY(get(h, p + "attn.proj.weight", (size_t)C * C, &pw));
     ARD_TRY(transpose_upload_bf16(bw.proj_wT, pw->data(), C, C));
     if (bw.has_res) {
-        // The ResiDual and the projection fold for the backward too:  with  Wc = B Wp [K,C],  c0 = B (b_p - mu) [K]
-        //   coef  = x_proj              = ao Wc^T + c0        (src/residual.py:37-38)
-        //   d ao  = (gcoef * lambda) Wc                        (src/residual.py:39-40 then the proj Linear)
-        const int K = bw.K, Kp = (K + 15) & ~15;
+        const int Kp = (bw.K + 15) & ~15;
         bw.Kp = Kp;
-        const std::vector<float>* pb = nullptr;
-        ARD_TRY(get(h, p + "attn.proj.bias", C, &pb));
-        std::vector<float> wc((size_t)Kp * C, 0.f), c0(Kp, 0.f), bpad((size_t)Kp * C, 0.f);
-        for (int k = 0; k < K; ++k) {
-            const float* bk = bw.h_basis.data() + (size_t)k * C;
-            float* o = wc.data() + (size_t)k * C;
-            double acc0 = 0.0;
-            for (int c = 0; c < C; ++c) {
-                const float bv = bk[c];
-                const float* wr = pw->data() + (size_t)c * C;
-                for (int j = 0; j < C; ++j) o[j] += bv * wr[j];
-                acc0 += (double)bv * ((double)(*pb)[c] - (double)bw.h_mean[c]);
-            }
-            c0[k] = (float)acc0;
-            memcpy(bpad.data() + (size_t)k * C, bk, (size_t)C * 4);
-        }
+        std::vector<float> wc, c0, bpad;
+        ARD_TRY(residual_backward_fold(h, l, b, wc, c0, bpad));
         ARD_TRY(upload_bf16(bw.res_wc, wc));                                   // [Kp, C]
         ARD_TRY(transpose_upload_bf16(bw.res_wcT, wc.data(), Kp, C));          // [C, Kp]
         ARD_TRY(upload_bf16(bw.res_basis_bf16, bpad));                         // [Kp, C]
         ARD_TRY(upload_f32(bw.res_c0, c0));
     }
     bw.bwd_ready = true;
+    return 0;
+}
+
+// w [rows, cols] (the first `scaled_rows` rows times `scale`) -> split form of w^T: dst [cols, 3 rows] = [W_hi^T | W_lo^T | W_hi^T]
+static int transpose_split_upload(DevBuf& dst, DevBuf& scratch, const float* w, int rows, int cols, cudaStream_t s, float scale = 1.0f,
+                                  int scaled_rows = 0) {
+    std::vector<float> t((size_t)rows * cols);
+    for (int r = 0; r < rows; ++r) {
+        const float sc = r < scaled_rows ? scale : 1.0f;
+        for (int c = 0; c < cols; ++c) t[(size_t)c * rows + r] = w[(size_t)r * cols + c] * sc;
+    }
+    return split3_weight_host(t, scratch, dst, cols, rows, s);
+}
+
+// Split forms of every dgrad weight of the fp32-grade backward, next to the forward's split weights (same invalidation).
+static int ensure_backward_weights_fp32(ard_handle* h, Fp32Weights& w, cudaStream_t s) {
+    if (w.bwd_epoch == w.epoch) return 0;
+    const std::vector<float>* v = nullptr;
+    for (int l = 0; l < h->nlayers; ++l) {
+        const int C = C_of(h, l), nH = h->cfg.num_heads[l];
+        for (int b = 0; b < h->cfg.depths[l]; ++b) {
+            BlockW& bw = h->layers[l].blocks[b];
+            Fp32BlockW& fw = w.blocks[l][b];
+            char pfx[64];
+            snprintf(pfx, sizeof(pfx), "layers.%d.blocks.%d.", l, b);
+            const std::string p(pfx);
+            ARD_TRY(get(h, p + "mlp.fc1.weight", (size_t)4 * C * C, &v));
+            ARD_TRY(transpose_split_upload(fw.fc1T3, w.scratch, v->data(), 4 * C, C, s));              // [C, 3*4C]
+            ARD_TRY(get(h, p + "mlp.fc2.weight", (size_t)4 * C * C, &v));
+            ARD_TRY(transpose_split_upload(fw.fc2T3, w.scratch, v->data(), C, 4 * C, s));              // [4C, 3C]
+            ARD_TRY(get(h, p + "attn.qkv.weight", (size_t)3 * C * C, &v));
+            ARD_TRY(transpose_split_upload(fw.qkvT3, w.scratch, v->data(), 3 * C, C, s, 1.0f / sqrtf((float)(C / nH)), C));   // [C, 3*3C]
+            ARD_TRY(get(h, p + "attn.proj.weight", (size_t)C * C, &v));
+            ARD_TRY(transpose_split_upload(fw.projT3, w.scratch, v->data(), C, C, s));                 // [C, 3C]
+            if (bw.has_res) {
+                const int Kp = (bw.K + 15) & ~15;
+                std::vector<float> wc, c0, bpad;
+                ARD_TRY(residual_backward_fold(h, l, b, wc, c0, bpad));
+                ARD_TRY(split3_weight_host(wc, w.scratch, fw.wc3, Kp, C, s));                          // [Kp, 3C]
+                ARD_TRY(transpose_split_upload(fw.wcT3, w.scratch, wc.data(), Kp, C, s));              // [C, 3Kp]
+                ARD_TRY(split3_weight_host(bpad, w.scratch, fw.basis3, Kp, C, s));                     // [Kp, 3C]
+                ARD_TRY(upload_f32(bw.res_c0, c0));
+                bw.Kp = Kp;
+            }
+        }
+        if (l < h->nlayers - 1) {
+            char key[64];
+            snprintf(key, sizeof(key), "layers.%d.downsample.reduction.weight", l);
+            ARD_TRY(get(h, key, (size_t)8 * C * C, &v));
+            ARD_TRY(transpose_split_upload(w.mergeT3[l], w.scratch, v->data(), 2 * C, 4 * C, s));      // [4C, 3*2C]
+        }
+    }
+    w.bwd_epoch = w.epoch;
     return 0;
 }
 
@@ -274,6 +354,58 @@ static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool 
     return layernorm_bwd(bw.t_s, w.T, bw.ln1_g.as<float>(), w.G, w.G, M, C, s, 1.0f, w.GB);  // G += LN1'(dn1), GB = bf16(G)
 }
 
+// ------------------------------------------------------------------------------------------------ fp32-grade backward schedule
+// The same steps as ffn_backward / block_backward with every dgrad a split GEMM; no gemm_dual (its epilogues are bf16 /
+// packed fp16). A3 (split operands, [M, 12C] bf16), HPRE / GQKV (fp32 [M, 4C]) and GAO (fp32 [M, C]) are the fp32-grade
+// forward's workspace, idle once the forward is done.
+struct BwdBufs32 {
+    float *G, *T, *R, *DH, *HPRE, *GQKV, *GAO, *coef, *gcoef;
+    __nv_bfloat16 *A3, *G3;
+};
+
+// gout = out_scale * gin + d/dx [ mlp(norm2(x)) ]^T gin   (gout may alias gin)
+static int ffn_backward_fp32(ard_handle* h, BlockW& bw, Fp32BlockW& fw, int C, long long M, const float* x, const float* gin, float* gout,
+                             float out_scale, const BwdBufs32& w, cudaStream_t s) {
+    ARD_TRY(layernorm_split3(x, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), w.A3, M, C, s));
+    ARD_TRY(gemm3(w.A3, C, fw.fc13, w.HPRE, 4 * C, M, 4 * C, bw.fc1_b.as<float>(), ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));
+    ARD_TRY(split3_act(gin, C, w.G3, M, C, s));                                                       // hpre = fc1(norm2(x)), recomputed
+    ARD_TRY(gemm3(w.G3, C, fw.fc2T3, w.DH, 4 * C, M, 4 * C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));   // g W2
+    ARD_TRY(gelu_bwd_split3(w.DH, w.HPRE, w.A3, M, 4 * C, s));                                         // dh = (g W2) * gelu'(hpre)
+    ARD_TRY(gemm3(w.A3, 4 * C, fw.fc1T3, w.T, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));       // dn2 = dh W1
+    return layernorm_bwd(x, w.T, bw.ln2_g.as<float>(), gin, gout, M, C, s, out_scale, nullptr);       // + LN2'(dn2)
+}
+
+static int block_backward_fp32(ard_handle* h, Fp32Weights& fws, int l, int b, int B, float* dlam, bool stop_after_lambda, const BwdBufs32& w,
+                               cudaStream_t s) {
+    BlockW& bw = h->layers[l].blocks[b];
+    Fp32BlockW& fw = fws.blocks[l][b];
+    const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
+    const long long M = (long long)B * T;
+    if (bw.has_res) {
+        ARD_TRY(ffn_backward_fp32(h, bw, fw, C, M, bw.t_x3, w.G, w.G, 1.0f, w, s));     // G = dL/dx3
+        ARD_TRY(ffn_backward_fp32(h, bw, fw, C, M, bw.t_x1, w.G, w.R, 1.0f, w, s));     // R = dL/dx1 = dL/dr = G + FFN'(G)
+        ARD_TRY(add_f32(w.G, w.R, w.G, nullptr, M * C, s));                             // dL/ds so far = dL/dx3 + dL/dx1
+        const int Kp = bw.Kp;
+        const float* lam = bw.lambda_set && bw.lam.p ? bw.lam.as<float>() : bw.lam_ones.as<float>();
+        ARD_TRY(split3_act(bw.t_aof, C, w.A3, M, C, s));
+        ARD_TRY(gemm3(w.A3, C, fw.wc3, w.coef, Kp, M, Kp, bw.res_c0.as<float>(), ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));   // coef = x_proj
+        ARD_TRY(split3_act(w.R, C, w.G3, M, C, s));
+        ARD_TRY(gemm3(w.G3, C, fw.basis3, w.gcoef, Kp, M, Kp, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));   // gcoef = dL/dr B^T
+        ARD_TRY(lambda_grad(w.coef, w.gcoef, lam, dlam, w.A3, M, bw.K, Kp, s, true));   // dlam += colsum(coef*gcoef); A3 = split(gcoef*lam)
+        if (stop_after_lambda) return 0;
+        ARD_TRY(gemm3(w.A3, Kp, fw.wcT3, w.GAO, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));        // d ao = gsc Wc
+    } else {
+        ARD_TRY(ffn_backward_fp32(h, bw, fw, C, M, bw.t_x1, w.G, w.G, 1.0f, w, s));     // G = dL/dx1 = dL/ds (shortcut) = dL/dr
+        if (stop_after_lambda) return 0;
+        ARD_TRY(split3_act(w.G, C, w.G3, M, C, s));
+        ARD_TRY(gemm3(w.G3, C, fw.projT3, w.GAO, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));       // d ao = dL/dr Wp
+    }
+    ARD_TRY(window_attention_f32_bwd(bw.t_qkvf, w.GAO, w.GQKV, bw.rpb.as<float>(), B, R, C, nH, (b % 2 == 0) ? 0 : 4, s));
+    ARD_TRY(split3_act(w.GQKV, 3 * C, w.A3, M, 3 * C, s));
+    ARD_TRY(gemm3(w.A3, 3 * C, fw.qkvT3, w.T, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));          // dn1 = dqkv Wqkv
+    return layernorm_bwd(bw.t_s, w.T, bw.ln1_g.as<float>(), w.G, w.G, M, C, s, 1.0f, nullptr);           // G += LN1'(dn1)
+}
+
 int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) {
     const int B = a->B;
     if (h->tape_B <= 0 || h->tape_B != B)
@@ -299,9 +431,30 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         if (K) ARD_TRY(fill_f32(a->grad_lambda[l], K, 0.f, s));
     }
     if (stop_l < 0) return 0;
+    const bool fp32 = h->tape_prec == 1;
     const size_t MC = (size_t)B * 4096 * h->cfg.embed_dim;
     ARD_TRY(h->bw_g.ensure(MC * 4));
     ARD_TRY(h->bw_t.ensure(MC * 4));
+    ARD_TRY(h->bw_small.ensure((size_t)B * (2 * J + NF) * 4 + 1024));
+    BwdBufs w;
+    BwdBufs32 w32;
+    Fp32Weights* fws = nullptr;
+    if (fp32) {
+        ARD_TRY(fp32_weights(h, &fws, s));
+        ARD_TRY(ensure_backward_weights_fp32(h, *fws, s));
+        ARD_TRY(fws->qkvf.ensure(MC * 16));
+        ARD_TRY(fws->aof.ensure(MC * 4));
+        ARD_TRY(fws->s3.ensure(MC * 24));
+        ARD_TRY(h->bw_gs.ensure(MC * 4));
+        ARD_TRY(h->bw_dh.ensure(MC * 16));
+        ARD_TRY(h->bw_g3.ensure(MC * 6));
+        ARD_TRY(h->bw_coef.ensure(MC * 4));
+        ARD_TRY(h->bw_gcoef.ensure(MC * 4));
+        w32.G = h->bw_g.as<float>(); w32.T = h->bw_t.as<float>(); w32.R = h->bw_gs.as<float>(); w32.DH = h->bw_dh.as<float>();
+        w32.HPRE = w32.GQKV = fws->qkvf.as<float>(); w32.GAO = fws->aof.as<float>();
+        w32.coef = h->bw_coef.as<float>(); w32.gcoef = h->bw_gcoef.as<float>();
+        w32.A3 = fws->s3.as<__nv_bfloat16>(); w32.G3 = h->bw_g3.as<__nv_bfloat16>();
+    } else {
     ARD_TRY(h->bw_dh.ensure(MC * 4 * 2));
     ARD_TRY(h->bw_gb.ensure(MC * 2));
     if (!h->use_dual_gemm) {   // the fp32 coefficient matrices only exist on the separate-GEMM path
@@ -309,12 +462,11 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         ARD_TRY(h->bw_gcoef.ensure(MC * 4));
     }
     ARD_TRY(h->bw_gsc.ensure(MC * 2));
-    ARD_TRY(h->bw_small.ensure((size_t)B * (2 * J + NF) * 4 + 1024));
-    BwdBufs w;
+    }
     w.G = h->bw_g.as<float>(); w.T = h->bw_t.as<float>();
     w.coef = h->bw_coef.as<float>(); w.gcoef = h->bw_gcoef.as<float>(); w.gsc = h->bw_gsc.as<__nv_bfloat16>();
     w.XN = h->ws_xn.as<__nv_bfloat16>(); w.HPRE = h->ws_h.as<__nv_bfloat16>(); w.DH = h->bw_dh.as<__nv_bfloat16>();
-    w.GB = h->bw_gb.as<__nv_bfloat16>(); w.GQKV = h->ws_qkv.as<__nv_bfloat16>(); w.GAO = h->ws_ao.as<__nv_bfloat16>();
+    w.GB = fp32 ? nullptr : h->bw_gb.as<__nv_bfloat16>(); w.GQKV = h->ws_qkv.as<__nv_bfloat16>(); w.GAO = h->ws_ao.as<__nv_bfloat16>();
 
     // ---- head: audio_embed = normalize(W2 relu(W0 emb + b0) + b2)   (model.py:539-543, :739-741)
     float* g_p = h->bw_small.as<float>();
@@ -352,13 +504,21 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         const int C = C_of(h, l), R = R_of(l);
         for (int b = h->cfg.depths[l] - 1; b >= 0; --b) {
             const bool stop = (l == stop_l && b == stop_b);
-            ARD_TRY(block_backward(h, l, b, B, a->grad_lambda[l], stop, w, s));
+            if (fp32) ARD_TRY(block_backward_fp32(h, *fws, l, b, B, a->grad_lambda[l], stop, w32, s));
+            else ARD_TRY(block_backward(h, l, b, B, a->grad_lambda[l], stop, w, s));
             if (stop) return 0;
         }
         if (l > 0) {   // PatchMerging backward: reduction Linear (no bias) dgrad, then gather + LayerNorm(4C) backward
             const int Cp = C / 2, Rp = R * 2;
             const long long Mm = (long long)B * R * R;
             LayerW& lw = h->layers[l - 1];
+            if (fp32) {
+                ARD_TRY(split3_act(w32.G, C, w32.G3, Mm, C, s));
+                ARD_TRY(gemm3(w32.G3, C, fws->mergeT3[l - 1], w32.T, 4 * Cp, Mm, 4 * Cp, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0,
+                              h->num_sms, s));
+                ARD_TRY(merge_layernorm_bwd(lw.blocks.back().t_out, w32.T, lw.mg_g.as<float>(), w32.G, nullptr, B, Rp, Rp, Cp, s));
+                continue;
+            }
             if (!lw.mg_wT.p) {
                 const std::vector<float>* v = nullptr;
                 char key[64];

@@ -8,7 +8,9 @@
 //
 // Everything between the GEMMs is fp32: LayerNorm, exact-erf GELU in the GEMM epilogue, the window attention core (SIMT fp32:
 // it is 4 % of the flops), residual adds, the ResiDual fold (fp32 SIMT, then split). 3x the tensor work and ~2.5x the
-// traffic of the bf16 path: a verification / high-fidelity mode, not the throughput mode. Inference only.
+// traffic of the bf16 path: a verification / high-fidelity mode, not the throughput mode.
+// Training: with save_for_backward the same forward writes its intermediates to an fp32 tape (ard_train.cu), and the
+// backward runs its dgrads the same way; the pieces only it needs (fp32 attention backward, gelu' into split form) are here.
 #include "ard_common.cuh"
 #include "ard_handle.h"
 
@@ -52,7 +54,7 @@ __global__ void __launch_bounds__(256) split3_weight_kernel(const float* __restr
     }
 }
 
-static int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s) {
+int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s) {
     if (rows <= 0) return 0;
     if (C % 4 || ld_in % 4) return set_error(ARD_ERR_SHAPE, "split3: width must be a multiple of 4");
     long long blocks = (rows * (C / 4) + 255) / 256;
@@ -69,8 +71,8 @@ static int split3_weight_dev(const float* w_dev, DevBuf& out, long long N, int K
     return check_cuda(cudaGetLastError(), "split3_weight launch");
 }
 // host fp32 weight (optionally the first `scaled_rows` rows times `scale`: the q rows of qkv carry head_dim^-0.5) -> split device form
-static int split3_weight_host(const std::vector<float>& w, DevBuf& scratch, DevBuf& out, long long N, int K, cudaStream_t s, float scale = 1.0f,
-                              long long scaled_rows = 0) {
+int split3_weight_host(const std::vector<float>& w, DevBuf& scratch, DevBuf& out, long long N, int K, cudaStream_t s, float scale,
+                       long long scaled_rows) {
     const float* src = w.data();
     std::vector<float> tmp;
     if (scaled_rows > 0) {
@@ -185,6 +187,181 @@ static int window_attention_f32(const float* qkv, float* out, const float* bias_
     return check_cuda(cudaGetLastError(), "window_attention_f32 launch");
 }
 
+// ------------------------------------------------------------------------------------------------ fp32 window attention backward
+// Autograd of the kernel above w.r.t. qkv (loss.backward() through htsat.py:326-352), fp32 on CUDA cores with the same CTA
+// decomposition and addressing. Thread i recomputes probability row i, then
+//   dP = dO V^T,  delta = rowsum(dP . P),  dS = P . (dP - delta),  dQ = dS K          (row i: registers)
+//   dK = dS^T Q,  dV = P^T dO                                                          (key row i: columns of P / dS via smem)
+// qkv fp32 [B*T, 3C] token order (q pre-scaled), dout fp32 [B*T, C] -> dqkv fp32 [B*T, 3C] token order (d of the pre-scaled q).
+template <int HD>
+constexpr int attn_f32_bwd_smem() { return (4 * 64 * (HD + 1) + 2 * 64 * 65 + 225) * 4; }
+
+template <int HD>
+__global__ void __launch_bounds__(64) window_attention_f32_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ dout,
+                                                                      float* __restrict__ dqkv, const float* __restrict__ bias_table, int R,
+                                                                      int C, int nH, int shift) {
+    extern __shared__ float sm[];
+    float (*Qs)[HD + 1] = reinterpret_cast<float (*)[HD + 1]>(sm);
+    float (*Ks)[HD + 1] = Qs + 64;
+    float (*Vs)[HD + 1] = Ks + 64;
+    float (*Os)[HD + 1] = Vs + 64;                                  // dO
+    float (*Ps)[65] = reinterpret_cast<float (*)[65]>(sm + 4 * 64 * (HD + 1));
+    float (*Ds)[65] = Ps + 64;                                      // dS
+    float* bt = sm + 4 * 64 * (HD + 1) + 2 * 64 * 65;
+    const int nWr = R / 8, nW = nWr * nWr;
+    const int h = blockIdx.x % nH;
+    const int win = (blockIdx.x / nH) % nW;
+    const long long b = blockIdx.x / ((long long)nH * nW);
+    const int wy = win / nWr, wx = win % nWr;
+    const int i = threadIdx.x;
+    const int ty = i >> 3, tx = i & 7;
+    const int yr = wy * 8 + ty, xr = wx * 8 + tx;
+    int y = yr + shift, x = xr + shift;
+    if (y >= R) y -= R;
+    if (x >= R) x -= R;
+    const long long tok = (b * R + y) * R + x;
+    const float* row = qkv + tok * 3LL * C + h * HD;
+    const float* grow = dout + tok * (long long)C + h * HD;
+    float q[HD], go[HD];
+#pragma unroll
+    for (int d = 0; d < HD; ++d) {
+        q[d] = row[d];
+        Qs[i][d] = q[d];
+        Ks[i][d] = row[C + d];
+        Vs[i][d] = row[2 * C + d];
+        go[d] = grow[d];
+        Os[i][d] = go[d];
+    }
+    for (int t = i; t < 225; t += 64) bt[t] = bias_table[t * nH + h];
+    __syncthreads();
+    const int ly = shift == 0 ? 0 : (yr < R - 8 ? 0 : (yr < R - shift ? 1 : 2));
+    const int lx = shift == 0 ? 0 : (xr < R - 8 ? 0 : (xr < R - shift ? 1 : 2));
+    const int label = ly * 3 + lx;
+    float sc[64];
+    float m = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < 64; ++j) {                                  // logits exactly as the forward kernel forms them
+        float a = 0.f;
+#pragma unroll
+        for (int d = 0; d < HD; ++d) a = fmaf(q[d], Ks[j][d], a);
+        const int jy = j >> 3, jx = j & 7;
+        a += bt[(ty - jy + 7) * 15 + (tx - jx + 7)];
+        if (shift != 0) {
+            const int yj = wy * 8 + jy, xj = wx * 8 + jx;
+            const int lj = (yj < R - 8 ? 0 : (yj < R - shift ? 1 : 2)) * 3 + (xj < R - 8 ? 0 : (xj < R - shift ? 1 : 2));
+            if (lj != label) a += -100.0f;
+        }
+        sc[j] = a;
+        m = fmaxf(m, a);
+    }
+    float sum = 0.f;
+#pragma unroll
+    for (int j = 0; j < 64; ++j) {
+        sc[j] = expf(sc[j] - m);
+        sum += sc[j];
+    }
+    const float inv = 1.0f / sum;
+    float delta = 0.f;
+#pragma unroll
+    for (int j = 0; j < 64; ++j) {                                  // P to smem, dP into sc
+        const float p = sc[j] * inv;
+        Ps[i][j] = p;
+        float dp = 0.f;
+#pragma unroll
+        for (int d = 0; d < HD; ++d) dp = fmaf(go[d], Vs[j][d], dp);
+        sc[j] = dp;
+        delta = fmaf(dp, p, delta);
+    }
+    float dq[HD];
+#pragma unroll
+    for (int d = 0; d < HD; ++d) dq[d] = 0.f;
+#pragma unroll
+    for (int j = 0; j < 64; ++j) {
+        const float ds = Ps[i][j] * (sc[j] - delta);
+        Ds[i][j] = ds;
+#pragma unroll
+        for (int d = 0; d < HD; ++d) dq[d] = fmaf(ds, Ks[j][d], dq[d]);
+    }
+    float* op = dqkv + tok * 3LL * C + h * HD;
+#pragma unroll
+    for (int d = 0; d < HD; ++d) op[d] = dq[d];
+    __syncthreads();
+    // thread i now owns KEY row i (the same token): column sums over the 64 query rows
+    float dk[HD], dv[HD];
+#pragma unroll
+    for (int d = 0; d < HD; ++d) { dk[d] = 0.f; dv[d] = 0.f; }
+    for (int r = 0; r < 64; ++r) {
+        const float ds = Ds[r][i], p = Ps[r][i];
+#pragma unroll
+        for (int d = 0; d < HD; ++d) {
+            dk[d] = fmaf(ds, Qs[r][d], dk[d]);
+            dv[d] = fmaf(p, Os[r][d], dv[d]);
+        }
+    }
+#pragma unroll
+    for (int d = 0; d < HD; ++d) {
+        op[C + d] = dk[d];
+        op[2 * C + d] = dv[d];
+    }
+}
+
+int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, const float* bias_table, int B, int R, int C, int nH, int shift,
+                             cudaStream_t s) {
+    if (B <= 0 || R <= 0 || R % 8 || nH <= 0 || C % nH)
+        return set_error(ARD_ERR_SHAPE, "window_attention_f32_bwd: unsupported shape B=%d R=%d C=%d nH=%d", B, R, C, nH);
+    const int hd = C / nH;
+    const int nW = (R / 8) * (R / 8);
+    const long long ctas = (long long)B * nW * nH;
+    if (ctas > 0x7fffffffLL) return set_error(ARD_ERR_SHAPE, "window_attention_f32_bwd: batch too large");
+    const int sh = R > 8 ? shift : 0;                               // htsat.py:393-396, as the forward launcher
+    static bool attr_set = false;
+    if (!attr_set) {
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<24>()));
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<32>()));
+        attr_set = true;
+    }
+    ProfScope ps(PROF_ATTN, s, 10.0 * 64 * 64 * hd * ctas, 28.0 * B * R * R * C);
+    if (hd == 24)
+        window_attention_f32_bwd_kernel<24><<<(unsigned)ctas, 64, attn_f32_bwd_smem<24>(), s>>>(qkv, dout, dqkv, bias_table, R, C, nH, sh);
+    else if (hd == 32)
+        window_attention_f32_bwd_kernel<32><<<(unsigned)ctas, 64, attn_f32_bwd_smem<32>(), s>>>(qkv, dout, dqkv, bias_table, R, C, nH, sh);
+    else return set_error(ARD_ERR_SHAPE, "window_attention_f32_bwd: head dim %d unsupported (24 or 32)", hd);
+    return check_cuda(cudaGetLastError(), "window_attention_f32_bwd launch");
+}
+
+// FFN backward through the exact-erf GELU (htsat.py:151): dh = g * gelu'(hpre), g and hpre fp32 [rows, N], written straight
+// into the split activation form [hi | hi | lo] ([rows, 3N] bf16) that the next dgrad GEMM reads
+__global__ void __launch_bounds__(256) gelu_bwd_split3_kernel(const float* __restrict__ g, const float* __restrict__ hpre,
+                                                             __nv_bfloat16* __restrict__ out, long long rows, int N) {
+    const long long total = rows * (N / 4);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const long long r = i / (N / 4);
+        const int c = (int)(i - r * (N / 4)) * 4;
+        const float4 gv = *reinterpret_cast<const float4*>(g + r * N + c);
+        const float4 hv = *reinterpret_cast<const float4*>(hpre + r * N + c);
+        const float x[4] = {gv.x * gelu_erf_grad(hv.x), gv.y * gelu_erf_grad(hv.y), gv.z * gelu_erf_grad(hv.z), gv.w * gelu_erf_grad(hv.w)};
+        float l[4];
+#pragma unroll
+        for (int k = 0; k < 4; ++k) l[k] = x[k] - __bfloat162float(__float2bfloat16_rn(x[k]));
+        uint2 hi, lo;
+        hi.x = pack_bf16x2(x[0], x[1]); hi.y = pack_bf16x2(x[2], x[3]);
+        lo.x = pack_bf16x2(l[0], l[1]); lo.y = pack_bf16x2(l[2], l[3]);
+        __nv_bfloat16* o = out + r * (3LL * N);
+        *reinterpret_cast<uint2*>(o + c) = hi;
+        *reinterpret_cast<uint2*>(o + N + c) = hi;
+        *reinterpret_cast<uint2*>(o + 2 * N + c) = lo;
+    }
+}
+int gelu_bwd_split3(const float* g, const float* hpre, __nv_bfloat16* out3, long long rows, int N, cudaStream_t s) {
+    if (rows <= 0) return 0;
+    if (N % 4) return set_error(ARD_ERR_SHAPE, "gelu_bwd_split3: width must be a multiple of 4");
+    long long blocks = (rows * (N / 4) + 255) / 256;
+    if (blocks > 148 * 16) blocks = 148 * 16;
+    ProfScope ps(PROF_OTHER, s, 30.0 * rows * N, 14.0 * rows * N);
+    gelu_bwd_split3_kernel<<<(unsigned)blocks, 256, 0, s>>>(g, hpre, out3, rows, N);
+    return check_cuda(cudaGetLastError(), "gelu_bwd_split3 launch");
+}
+
 // tscam_conv im2col (heads.cu::tscam_im2col_kernel) straight into the split activation form [hi | hi | lo] of width 3 * 6C
 __global__ void tscam_im2col_split3_kernel(const float* __restrict__ normed, __nv_bfloat16* __restrict__ A3, int B, int C) {
     const long long K6 = 6LL * C;
@@ -213,21 +390,11 @@ __global__ void tscam_im2col_split3_kernel(const float* __restrict__ normed, __n
 }
 
 // ------------------------------------------------------------------------------------------------ weights
-struct Fp32BlockW {
-    DevBuf qkv3, proj3, fc13, fc23;
-};
-struct Fp32Weights {
-    unsigned long long epoch = ~0ULL;            // ard_handle::graph_epoch the split weights were built at (weights / ResiDual changes bump it)
-    std::vector<std::vector<Fp32BlockW>> blocks;
-    std::vector<DevBuf> merge3;
-    DevBuf tscam3, scratch;
-    DevBuf qkvf, aof, s3;                        // workspace: fp32 [M,4C] (qkv / FFN hidden), fp32 [M,C], split operands [M,12C] bf16
-};
-
 static int ensure_fp32_weights(ard_handle* h, Fp32Weights& w, cudaStream_t s) {
     if (w.epoch == h->graph_epoch && !w.blocks.empty()) return 0;
     w.blocks.resize(h->nlayers);
     w.merge3.resize(h->nlayers);
+    w.mergeT3.resize(h->nlayers);
     const std::vector<float>* v = nullptr;
     for (int l = 0; l < h->nlayers; ++l) {
         const int C = C_of(h, l), nH = h->cfg.num_heads[l];
@@ -268,8 +435,15 @@ static std::map<const ard_handle*, Fp32Weights>& fp32_cache() {
 }
 void fp32_release(const ard_handle* h) { fp32_cache().erase(h); }
 
-static int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, int ldo, long long M, int N, const float* bias, int act,
-                 const float* r1, const float* r2, float* aux, int aux_T, long long aux_bstride, int num_sms, cudaStream_t s) {
+int fp32_weights(ard_handle* h, Fp32Weights** out, cudaStream_t s) {
+    Fp32Weights& w = fp32_cache()[h];
+    ARD_TRY(ensure_fp32_weights(h, w, s));
+    *out = &w;
+    return 0;
+}
+
+int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, int ldo, long long M, int N, const float* bias, int act,
+          const float* r1, const float* r2, float* aux, int aux_T, long long aux_bstride, int num_sms, cudaStream_t s) {
     GemmArgs g;
     g.A = A3; g.lda = 3LL * K; g.W = W3.as<__nv_bfloat16>(); g.ldw = 3LL * K; g.out = out; g.ldo = ldo;
     g.M = (int)M; g.N = N; g.K = 3 * K; g.bias = bias; g.act = act;
@@ -279,21 +453,26 @@ static int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, i
     return gemm_bf16(g, num_sms, s);
 }
 
-// One Swin block (plain htsat.py:439-482 or patched src/residual.py:58-98) in the fp32-grade mode. Result ends in X; Y is scratch.
-static int run_block_fp32(ard_handle* h, Fp32Weights& w, int l, int b, int B, float* X, float* Y, float* attn_out, float attn_scale, int attn_acc,
-                          float* res_out, long long res_bstride, float* head_tap, cudaStream_t s) {
+// Where one block of the fp32-grade forward reads and writes. Inference: s = out = X, x1 = x3 = Y (scratch), qkv / ao in the
+// workspace. Training: the block's tape slots (ard_train.cu), so the backward finds every intermediate it needs.
+struct Fp32BlockIO {
+    float *s, *x1, *x3, *out, *qkv, *ao;
+};
+
+// One Swin block (plain htsat.py:439-482 or patched src/residual.py:58-98) in the fp32-grade mode.
+static int run_block_fp32(ard_handle* h, Fp32Weights& w, int l, int b, int B, const Fp32BlockIO& io, float* attn_out, float attn_scale,
+                          int attn_acc, float* res_out, long long res_bstride, float* head_tap, cudaStream_t s) {
     BlockW& bw = h->layers[l].blocks[b];
     Fp32BlockW& fw = w.blocks[l][b];
     const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
     const long long M = (long long)B * T;
-    float* QKVf = w.qkvf.as<float>();
-    float* AOf = w.aof.as<float>();
+    float* Hf = w.qkvf.as<float>();
     __nv_bfloat16* S3 = w.s3.as<__nv_bfloat16>();
     const int shift = (b % 2 == 0) ? 0 : 4;
-    ARD_TRY(layernorm_split3(X, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), S3, M, C, s));
-    ARD_TRY(gemm3(S3, C, fw.qkv3, QKVf, 3 * C, M, 3 * C, bw.qkv_b.as<float>(), ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));
-    ARD_TRY(window_attention_f32(QKVf, AOf, bw.rpb.as<float>(), attn_out, attn_scale, attn_acc, head_tap, B, R, C, nH, shift, s));
-    ARD_TRY(split3_act(AOf, C, S3, M, C, s));
+    ARD_TRY(layernorm_split3(io.s, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), S3, M, C, s));
+    ARD_TRY(gemm3(S3, C, fw.qkv3, io.qkv, 3 * C, M, 3 * C, bw.qkv_b.as<float>(), ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));
+    ARD_TRY(window_attention_f32(io.qkv, io.ao, bw.rpb.as<float>(), attn_out, attn_scale, attn_acc, head_tap, B, R, C, nH, shift, s));
+    ARD_TRY(split3_act(io.ao, C, S3, M, C, s));
     const DevBuf* pw = &fw.proj3;
     const float* pb = bw.proj_b.as<float>();
     static thread_local DevBuf fold3;   // the folded projection depends on the current lambda: re-split per call (C^2 elements)
@@ -303,24 +482,26 @@ static int run_block_fp32(ard_handle* h, Fp32Weights& w, int l, int b, int B, fl
         pw = &fold3;
         pb = bw.proj_b_fold.as<float>();
     }
-    // Y = X + r,  aux = r = residual_x (post-ResiDual for patched blocks)
-    ARD_TRY(gemm3(S3, C, *pw, Y, C, M, C, pb, ARD_ACT_NONE, X, nullptr, res_out, T, res_bstride, h->num_sms, s));
-    auto ffn = [&](float* in, float* out, const float* r2) -> int {   // out = in + mlp(norm2(in)) (+ r2)
+    // x1 = s + r,  aux = r = residual_x (post-ResiDual for patched blocks)
+    ARD_TRY(gemm3(S3, C, *pw, io.x1, C, M, C, pb, ARD_ACT_NONE, io.s, nullptr, res_out, T, res_bstride, h->num_sms, s));
+    auto ffn = [&](const float* in, float* out, const float* r2) -> int {   // out = in + mlp(norm2(in)) (+ r2)
         ARD_TRY(layernorm_split3(in, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), S3, M, C, s));
-        ARD_TRY(gemm3(S3, C, fw.fc13, QKVf, 4 * C, M, 4 * C, bw.fc1_b.as<float>(), ARD_ACT_GELU, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));
-        ARD_TRY(split3_act(QKVf, 4 * C, S3, M, 4 * C, s));
+        ARD_TRY(gemm3(S3, C, fw.fc13, Hf, 4 * C, M, 4 * C, bw.fc1_b.as<float>(), ARD_ACT_GELU, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));
+        ARD_TRY(split3_act(Hf, 4 * C, S3, M, 4 * C, s));
         return gemm3(S3, 4 * C, fw.fc23, out, C, M, C, bw.fc2_b.as<float>(), ARD_ACT_NONE, in, r2, nullptr, 0, 0, h->num_sms, s);
     };
-    if (!bw.has_res) return ffn(Y, X, nullptr);                     // htsat.py:480
-    ARD_TRY(ffn(Y, Y, X));                                           // x3 = shortcut + (x1 + mlp(norm2(x1)))   src/residual.py:93,95
-    return ffn(Y, X, nullptr);                                       // x4 = x3 + mlp(norm2(x3))                src/residual.py:96
+    if (!bw.has_res) return ffn(io.x1, io.out, nullptr);             // htsat.py:480
+    ARD_TRY(ffn(io.x1, io.x3, io.s));                                // x3 = shortcut + (x1 + mlp(norm2(x1)))   src/residual.py:93,95
+    return ffn(io.x3, io.out, nullptr);                              // x4 = x3 + mlp(norm2(x3))                src/residual.py:96
 }
 
-// Swin stages + tail of the forward in the fp32-grade mode; X holds the patch-embed output (front end is fp32 already).
+// Swin stages of the forward in the fp32-grade mode; X holds the patch-embed output (front end is fp32 already). With
+// a->save_for_backward, X is the tape's first slot and every block writes its tape slots (ensure_tape(h, B, 1) ran).
 int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, float* Y, float** x_final, cudaStream_t s) {
     Fp32Weights& w = fp32_cache()[h];
     ARD_TRY(ensure_fp32_weights(h, w, s));
     const int B = a->B;
+    const bool train = a->save_for_backward != 0;
     const size_t MC = (size_t)B * 4096 * h->cfg.embed_dim;
     ARD_TRY(w.qkvf.ensure(MC * 16));
     ARD_TRY(w.aof.ensure(MC * 4));
@@ -330,13 +511,19 @@ int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, floa
         for (int b = 0; b < depth; ++b) {
             float* res = a->layers_residuals[l] ? a->layers_residuals[l] + (long long)b * T * C : nullptr;
             float* tap = a->head_outputs[l] ? a->head_outputs[l] + (long long)b * B * T * C : nullptr;
-            ARD_TRY(run_block_fp32(h, w, l, b, B, X, Y, a->layers_attention[l], 1.0f / depth, b > 0, res, (long long)depth * T, tap, s));
+            const BlockW& bw = h->layers[l].blocks[b];
+            const Fp32BlockIO io = train ? Fp32BlockIO{bw.t_s, bw.t_x1, bw.t_x3, bw.t_out, bw.t_qkvf, bw.t_aof}
+                                         : Fp32BlockIO{X, Y, Y, X, w.qkvf.as<float>(), w.aof.as<float>()};
+            ARD_TRY(run_block_fp32(h, w, l, b, B, io, a->layers_attention[l], 1.0f / depth, b > 0, res, (long long)depth * T, tap, s));
+            if (train) X = bw.t_out;
         }
         if (l < h->nlayers - 1) {   // PatchMerging (htsat.py:505-526)
+            float* mout = train ? h->layers[l + 1].blocks[0].t_s : Y;
             ARD_TRY(merge_layernorm_split3(X, h->layers[l].mg_g.as<float>(), h->layers[l].mg_b.as<float>(), w.s3.as<__nv_bfloat16>(), B, R, R, C, s));
-            ARD_TRY(gemm3(w.s3.as<__nv_bfloat16>(), 4 * C, w.merge3[l], Y, 2 * C, (long long)B * (T / 4), 2 * C, nullptr, ARD_ACT_NONE, nullptr, nullptr,
-                          nullptr, 0, 0, h->num_sms, s));
-            float* t = X; X = Y; Y = t;
+            ARD_TRY(gemm3(w.s3.as<__nv_bfloat16>(), 4 * C, w.merge3[l], mout, 2 * C, (long long)B * (T / 4), 2 * C, nullptr, ARD_ACT_NONE, nullptr,
+                          nullptr, nullptr, 0, 0, h->num_sms, s));
+            if (train) X = mout;
+            else { Y = X; X = mout; }
         }
     }
     *x_final = X;

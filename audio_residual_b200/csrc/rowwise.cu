@@ -503,6 +503,8 @@ int gelu_bwd_mul(__nv_bfloat16* dh, const __nv_bfloat16* hpre, long long n, cuda
 //   dlam[k] += sum_t coef[t,k] * gcoef[t,k]  (k < K);   gsc[t,k] = bf16(gcoef[t,k] * lam[k])  (k < Kp: the gradient flowing on to x_proj)
 // coef, gcoef fp32 [M, Kp]: rows are padded to Kp (a multiple of 16, the GEMMs' K granularity) while dlam holds only the K
 // logical components. Each CTA reduces a slab of rows for 32 columns in registers/smem, one atomicAdd per column per CTA.
+// SPLIT3 (fp32-grade backward): gsc is written in the split activation form [hi | hi | lo], [M, 3 Kp].
+template <bool SPLIT3>
 __global__ void __launch_bounds__(256) lambda_grad_kernel(const float* __restrict__ coef, const float* __restrict__ gcoef,
                                                          const float* __restrict__ lam, float* __restrict__ dlam,
                                                          __nv_bfloat16* __restrict__ gsc, long long M, int K, int Kp, long long rows_per_cta) {
@@ -516,7 +518,16 @@ __global__ void __launch_bounds__(256) lambda_grad_kernel(const float* __restric
         for (long long r = r0 + ty; r < r1; r += 8) {
             const float c = coef[r * Kp + col], gc = gcoef[r * Kp + col];
             acc = fmaf(c, gc, acc);
-            gsc[r * Kp + col] = __float2bfloat16_rn(gc * l);
+            if constexpr (SPLIT3) {
+                const float v = gc * l;
+                const __nv_bfloat16 hi = __float2bfloat16_rn(v);
+                __nv_bfloat16* o = gsc + r * 3LL * Kp + col;
+                o[0] = hi;
+                o[Kp] = hi;
+                o[2 * Kp] = __float2bfloat16_rn(v - __bfloat162float(hi));
+            } else {
+                gsc[r * Kp + col] = __float2bfloat16_rn(gc * l);
+            }
         }
     }
     part[ty][tx] = acc;
@@ -529,15 +540,16 @@ __global__ void __launch_bounds__(256) lambda_grad_kernel(const float* __restric
     }
 }
 int lambda_grad(const float* coef, const float* gcoef, const float* lam, float* dlam, __nv_bfloat16* gsc, long long M, int K, int Kp,
-                cudaStream_t s) {
+                cudaStream_t s, bool split3) {
     if (M <= 0) return 0;
     const int cb = (Kp + 31) / 32;
     long long ysplit = (148 * 8) / cb + 1;
     long long rows_per_cta = (M + ysplit - 1) / ysplit;
     rows_per_cta = ((rows_per_cta + 7) / 8) * 8;
     ysplit = (M + rows_per_cta - 1) / rows_per_cta;
-    ProfScope ps(PROF_OTHER, s, 3.0 * M * Kp, 10.0 * M * Kp);
-    lambda_grad_kernel<<<dim3(cb, (unsigned)ysplit), 256, 0, s>>>(coef, gcoef, lam, dlam, gsc, M, K, Kp, rows_per_cta);
+    ProfScope ps(PROF_OTHER, s, 3.0 * M * Kp, (split3 ? 14.0 : 10.0) * M * Kp);
+    if (split3) lambda_grad_kernel<true><<<dim3(cb, (unsigned)ysplit), 256, 0, s>>>(coef, gcoef, lam, dlam, gsc, M, K, Kp, rows_per_cta);
+    else lambda_grad_kernel<false><<<dim3(cb, (unsigned)ysplit), 256, 0, s>>>(coef, gcoef, lam, dlam, gsc, M, K, Kp, rows_per_cta);
     return check_cuda(cudaGetLastError(), "lambda_grad launch");
 }
 

@@ -210,6 +210,7 @@ class HTSAT_Swin_Transformer(nn.Module):
         self.head = nn.Linear(num_classes, num_classes)   # present (unused) in the reference too, htsat.py:748
         # CLAP-level projection (model.py:539-543) rides on the same handle; set by CLAP.__init__
         object.__setattr__(self, "_projection", None)
+        self.train_precision = "bf16"
         self._hb = _HandleBox()
         self._relink()
         for p in self.parameters():
@@ -231,6 +232,19 @@ class HTSAT_Swin_Transformer(nn.Module):
             new.__dict__[k] = copy.deepcopy(v, memo)
         new._relink()
         return new
+
+    @property
+    def train_precision(self):
+        """Precision of the training step (the autograd route into the ResiDual lambdas): "bf16" (default, the tensor-core
+        path) or "fp32" (3-term split-bf16 GEMMs forward and backward, fp32 attention / LayerNorm / GELU backward; the lambda
+        gradients then match the reference's fp32 loss.backward() to rel. err <= 1e-4)."""
+        return self.__dict__.get("_train_precision", "bf16")
+
+    @train_precision.setter
+    def train_precision(self, value):
+        if value not in ("bf16", "fp32"):
+            raise ValueError(f"train_precision must be 'bf16' or 'fp32' (got {value!r})")
+        object.__setattr__(self, "_train_precision", value)
 
     def _device(self):
         return self.norm.weight.device
@@ -356,17 +370,21 @@ class HTSAT_Swin_Transformer(nn.Module):
         With grad enabled and trainable ResiDual lambdas, `embedding` / `audio_embed` come back attached to the autograd graph
         (backward = ard_encoder_backward, filling `learnable.grad` as loss.backward() does in src/training.py:30-32).
         want_head_outputs: also return `head_outputs`, per layer [depth, B*nW, nH, 64, hd]: every block's per-head `attn @ v`
-        (htsat.py:354). precision: "bf16" (default) or "fp32" (3-term split-bf16 GEMMs + fp32 attention, rel. err <= 1e-4;
-        inference only); None takes the encoder's `precision` attribute."""
+        (htsat.py:354). precision: "bf16" (default) or "fp32" (3-term split-bf16 GEMMs + fp32 attention, rel. err <= 1e-4);
+        None takes the encoder's `precision` attribute. The autograd route runs at the encoder's `train_precision` instead;
+        an encoder set to precision="fp32" trains only with train_precision="fp32" too (never silently in bf16).
+        save_for_backward=True with precision="fp32" saves an fp32-grade forward for an fp32-grade backward."""
         precision = precision or getattr(self, "precision", "bf16")
         if precision not in ("bf16", "fp32"):
             raise ValueError(f"precision must be 'bf16' or 'fp32' (got {precision!r})")
         if not save_for_backward and torch.is_grad_enabled():
             lams = self._lambda_params()
             if any(p is not None and p.requires_grad for p in lams):
-                if precision != "bf16":
-                    raise NotImplementedError("the training step runs on the bf16 tensor-core path; precision='fp32' is inference only")
-                return _encode_with_grad(self, lams, waveform, mel_fusion, quantize, want_dict, want_audio_embed, want_capture)
+                if precision != "bf16" and self.train_precision != "fp32":
+                    raise NotImplementedError(f"precision={precision!r} with train_precision={self.train_precision!r}: the training step "
+                                              "runs at train_precision; set train_precision='fp32' to train at fp32 grade")
+                return _encode_with_grad(self, lams, waveform, mel_fusion, quantize, want_dict, want_audio_embed, want_capture,
+                                         self.train_precision)
         h = self._handle()
         lib = L.load()
         dev = self._device()
@@ -499,9 +517,9 @@ class _EncodeFn(torch.autograd.Function):
         return (None, None, None) + tuple(outs[l].to(d) for l, d in zip(ctx.layers, ctx.devs))
 
 
-def _encode_with_grad(enc, lams, waveform, mel_fusion, quantize, want_dict, want_audio_embed, want_capture):
+def _encode_with_grad(enc, lams, waveform, mel_fusion, quantize, want_dict, want_audio_embed, want_capture, precision):
     kw = dict(waveform=waveform, mel_fusion=mel_fusion, quantize=quantize, want_dict=want_dict, want_audio_embed=want_audio_embed,
-              want_capture=want_capture)
+              want_capture=want_capture, precision=precision)
     holder = {}
     live = [p for p in lams if p is not None]
     res = _EncodeFn.apply(enc, kw, holder, *live)

@@ -82,6 +82,7 @@ def load(check_symbols=False):
         lib.ard_ln_qkv_96.argtypes = [vp, vp, vp, vp, vp, vp, ll, vp]
         lib.ard_window_attention.argtypes = [vp, vp, vp, vp, f, i, i, i, i, i, i, i, vp]
         lib.ard_window_attention_bwd.argtypes = [vp, vp, vp, vp, i, i, i, i, i, i, vp]
+        lib.ard_window_attention_f32_bwd.argtypes = [vp, vp, vp, vp, i, i, i, i, i, i, vp]
         lib.ard_layernorm_bwd.argtypes = [vp, vp, vp, vp, vp, ll, i, vp]
         lib.ard_f32_to_bf16.argtypes = [vp, vp, ll, f, vp]
         lib.ard_quantize_waveform.argtypes = [vp, vp, ll, vp]

@@ -101,7 +101,8 @@ typedef struct ard_forward_args {
                                               * WindowAttention.forward (htsat.py:354) of every block, window order of that block
                                               * (shifted blocks: windows of the rolled image), before transpose / proj */
     int precision;           /* 0: bf16/fp16 tensor-core operands (rel. err <= 1e-2); 1: fp32-grade (3-term split-bf16 GEMMs, fp32
-                              * attention; rel. err <= 1e-4 vs the reference's fp32 arithmetic, hook.py:40). Inference only. */
+                              * attention; rel. err <= 1e-4 vs the reference's fp32 arithmetic, hook.py:40). With save_for_backward,
+                              * the precision of the training step: ard_encoder_backward runs at the precision of the saved forward. */
 } ard_forward_args;
 
 /* HTSAT_Swin_Transformer.forward (htsat.py:881-994) in eval mode + optional audio_projection/normalize. */
@@ -110,6 +111,8 @@ int ard_encoder_forward(ard_handle* h, const ard_forward_args* args, void* strea
 /* Backward of the last ard_encoder_forward(save_for_backward=1) on this handle: what loss.backward() (src/training.py:30-32)
  * computes for the only trainable tensors of setup_residual_htsat (src/residual.py:199-201): the ResiDual `learnable`
  * vectors. The encoder is frozen and in eval mode (src/training.py:105-108), so no weight gradients exist.
+ * It runs at the precision of that forward: bf16 tensor-core dgrads (precision 0), or fp32-grade (precision 1: 3-term
+ * split-bf16 dgrads, fp32 attention backward / gelu' / LayerNorm backward; rel. err <= 1e-4 vs the reference's fp32 autograd).
  * Inputs are dL/d(audio_embed) and/or dL/d(embedding); grad_lambda[l] (device [K_l] fp32, required for every layer that
  * carries a ResiDual) is OVERWRITTEN with the gradient summed over the layer's patched blocks, which share one
  * ResiDual module in the reference (src/residual.py:186-197). */
@@ -191,6 +194,10 @@ int ard_window_attention(const void* qkv_bf16, void* out_bf16, const float* bias
  * dout [B*H*W, C] bf16; the probabilities are recomputed from qkv. */
 int ard_window_attention_bwd(const void* qkv_bf16, const void* dout_bf16, void* dqkv_bf16, const float* bias_table, int B, int H, int W, int C,
                              int nH, int shift, void* stream);
+/* The same backward in fp32 (fp32 CUDA cores; backward of the fp32-grade mode's attention core): qkv [B*H*W, 3C] fp32 token
+ * order (q pre-scaled), dout [B*H*W, C] fp32 -> dqkv [B*H*W, 3C] fp32. H == W, head dim C/nH of 24 or 32; no shift when H == 8. */
+int ard_window_attention_f32_bwd(const float* qkv_f32, const float* dout_f32, float* dqkv_f32, const float* bias_table, int B, int H, int W,
+                                 int C, int nH, int shift, void* stream);
 /* Backward of nn.LayerNorm over the last dim: grad_in = (add ? add : 0) + dLN(x)^T grad_out; all fp32 [rows, C]. */
 int ard_layernorm_bwd(const float* x, const float* grad_out, const float* gamma, const float* add, float* grad_in, long long rows, int C,
                       void* stream);
