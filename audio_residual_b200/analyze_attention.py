@@ -17,6 +17,7 @@ import numpy as np
 import torch
 
 from .clap import batch_features
+from .linalg import sym_eigvals
 from .residual import MomentAccumulator, quantize_tensor, pad_or_truncate  # noqa: F401  (re-exported like the reference)
 
 
@@ -39,6 +40,56 @@ def _gram_spectrum(rows, n_total, D):
     return out
 
 
+# Smallest group (number of matrices of one size) from which one ard_sym_eigvals call beats the per-head torch.linalg.eigvalsh loop,
+# per matrix size: the first winning batch of the crossover sweep in profiles/eig_bench.json (B200, 1000 W; batches 1, 2, 4, 8, 16).
+# The library pays its D column steps once per call, so a lone matrix is slower there (4096^2: 0.33 s against 0.08 s) while a batch
+# shares them (28 x 4096^2: 1.0 s against 2.2 s). A size between two measured ones takes the larger one's entry.
+_LIB_MIN_BATCH = ((64, 8), (256, 4), (1152, 4), (2000, 8), (4096, 8))
+
+
+def _library_wins(batch, D):
+    need = next((b for d, b in _LIB_MIN_BATCH if D <= d), _LIB_MIN_BATCH[-1][1])
+    return batch >= need
+
+
+def _solve_owned_batched(owned, accs, spectra, D):
+    """The owned heads' spectra into `spectra` rows, grouped by route and size: the D x D covariances form one group, the Gram
+    matrices one group per sample count. A group at or above the measured crossover (_LIB_MIN_BATCH) is solved by one
+    ard_sym_eigvals call on matrices assembled exactly as _spectrum / _gram_spectrum assemble them; a smaller group goes head by
+    head through _spectrum / _gram_spectrum (also the route for CPU accumulators). A batched group holds all its matrices at once:
+    28 x 128 MB = 3.8 GB for the covariance heads of one GPU at D = 4096, where the per-head route holds one."""
+    cov = [(i, n_i) for i, n_i, r in owned if r is None]
+    if cov and _library_wins(len(cov), D):
+        M = torch.empty((len(cov), D, D), device=spectra.device, dtype=torch.float64)
+        for k, (i, n_i) in enumerate(cov):
+            mean = accs[i].s1 / n_i
+            c = (accs[i].s2 - n_i * torch.outer(mean, mean)) / (n_i - 1)
+            M[k] = 0.5 * (c + c.t())
+        w = sym_eigvals(M, overwrite=True).flip(-1).clamp_min(0)
+        spectra[[i for i, _ in cov]] = w
+        del M
+    else:
+        for i, n_i in cov:
+            spectra[i] = _spectrum(n_i, accs[i].s1, accs[i].s2)
+    grams = defaultdict(list)
+    for i, n_i, r in owned:
+        if r is not None:
+            grams[r.shape[0]].append((i, n_i, r))
+    for n, group in grams.items():
+        if not _library_wins(len(group), n):
+            for i, n_i, r in group:
+                spectra[i] = _gram_spectrum(r, n_i, D)
+            continue
+        G = torch.empty((len(group), n, n), device=spectra.device, dtype=torch.float64)
+        for k, (i, n_i, r) in enumerate(group):
+            X = r.double()
+            Xc = X - X.mean(0, keepdim=True)
+            G[k] = Xc @ Xc.t() / (n_i - 1)
+        w = sym_eigvals(G, overwrite=True).flip(-1).clamp_min(0)
+        m = min(n, D)
+        spectra[[i for i, _, _ in group], :m] = w[:, :m]
+
+
 def finalize_head_spectra(accs, n_components=None):
     """Spectra of a list of MomentAccumulators (one per (layer, head)), as numpy arrays.
     Under torch.distributed (clip-sharded pass, SURVEY 8e) the moments are summed over ranks with the heads dealt round-robin
@@ -47,7 +98,10 @@ def finalize_head_spectra(accs, n_components=None):
     single GPU become ceil(60 / N) per GPU. After the call every accumulator's `n` is the global sample count.
     Heads that saw fewer samples than dimensions and still hold them all (MomentAccumulator.parked_rows: the last HTSAT layer
     has ONE window per clip, so a 2000-clip pass gives its 32 heads 2000 samples of 4096 dimensions) take the Gram route: the
-    rows (not the D x D matrix) go to the owner and the eigen-solve is n x n (9 instead of 79 ms at n = 2000)."""
+    rows (not the D x D matrix) go to the owner and the eigen-solve is n x n (9 instead of 79 ms at n = 2000).
+    On CUDA accumulators each rank solves a group of same-size heads with one ard_sym_eigvals call instead of one
+    torch.linalg.eigvalsh per head, when the group is large enough for that to be faster (_solve_owned_batched); CPU accumulators
+    keep _spectrum / _gram_spectrum."""
     import torch.distributed as dist
     world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     rank = dist.get_rank() if world > 1 else 0
@@ -106,8 +160,11 @@ def finalize_head_spectra(accs, n_components=None):
                 owned.append((i, n_i, None))
         a.n = n_i
         a.mean_global = s1[i] / max(n_i, 1)
-    for i, n_i, r in owned:
-        spectra[i] = _gram_spectrum(r, n_i, D) if r is not None else _spectrum(n_i, accs[i].s1, accs[i].s2)
+    if dev.type == "cuda":
+        _solve_owned_batched(owned, accs, spectra, D)
+    else:
+        for i, n_i, r in owned:
+            spectra[i] = _gram_spectrum(r, n_i, D) if r is not None else _spectrum(n_i, accs[i].s1, accs[i].s2)
     if world > 1:
         dist.all_reduce(spectra)
     out = spectra.cpu().numpy()

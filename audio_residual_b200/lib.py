@@ -91,6 +91,9 @@ def load(check_symbols=False):
         lib.ard_patch_embed.argtypes = [vp, vp, i, vp, vp]
         lib.ard_stats_accumulate.argtypes = [vp, ll, i, vp, vp, vp]
         lib.ard_stats_accumulate_strided.argtypes = [vp, ll, ll, i, vp, vp, vp]
+        lib.ard_sym_eigvals_workspace.restype = C.c_longlong
+        lib.ard_sym_eigvals_workspace.argtypes = [i, i]
+        lib.ard_sym_eigvals.argtypes = [vp, ll, i, i, vp, vp, ll, vp]
         lib.ard_tape_generation.argtypes = [vp]
         lib.ard_residual_forward.argtypes = [vp, vp, vp, vp, vp, ll, i, i, vp]
         lib.ard_residual_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, ll, i, i, vp]

@@ -272,6 +272,17 @@ int ard_stats_accumulate(const float* x, long long rows, int D, double* sum, dou
 int ard_stats_accumulate_strided(const float* x, long long rows, long long ldx, int D, double* sum, double* sumsq, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * Eigenvalues of `batch` symmetric matrices A[b] (fp64 device, D x D row-major, matrix b at A + b*stride; the lower triangle
+ * is read, A is overwritten). w [batch, D] fp64 device, ascending per matrix. work: device scratch of at least
+ * ard_sym_eigvals_workspace(D, batch) bytes. Replaces the eigen-solve behind run_PCA's per-head spectra, src/analyze_attention.py:13-59.
+ * Blocked Householder tridiagonalisation (dsytrd) + Sturm bisection (dstebz), every launch covering the whole batch; asynchronous
+ * on `stream`. ARD_ERR_SHAPE (before any device work): D < 1, batch < 1 or > 65535, stride < D*D, a NULL pointer, a workspace
+ * that is too small.
+ * ------------------------------------------------------------------------------------------------------------------ */
+long long ard_sym_eigvals_workspace(int D, int batch);
+int ard_sym_eigvals(double* A, long long stride, int D, int batch, double* w, void* work, long long work_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * Measurement support (bench.py): per-kernel-class device time. Classes: 0 tcgen05 GEMM, 1 window attention,
  * 2 LayerNorm/merge, 3 front end (STFT/log-mel/patch-embed), 4 heads, 5 other, 6 fused FFN. While enabled every launch is bracketed
  * by CUDA events on its stream; ard_profile_read synchronises, sums elapsed ms / algorithmic flops / algorithmic bytes /
