@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from .clap import batch_features
-from .linalg import sym_eigvals
+from .linalg import eigh_batch, eigh_library_wins, sign_fix, sym_eigvals
 from .residual import MomentAccumulator, quantize_tensor, pad_or_truncate  # noqa: F401  (re-exported like the reference)
 
 
@@ -40,6 +40,36 @@ def _gram_spectrum(rows, n_total, D):
     return out
 
 
+def _desc(w, Q):
+    """Ascending (w, Q with eigenvectors as columns) -> descending clamped spectrum and eigenvector rows."""
+    return w.flip(-1).clamp_min(0), Q.mT.flip(-2)
+
+
+def _gram_components(Xc, U, D):
+    """Principal axes [D, D] (rows, descending variance) of the centred rows Xc [n, D], n < D, from the Gram eigenvectors U [n, n]
+    (rows, descending): the orthonormalised columns of Xc^T U^T, completed to an orthonormal basis of R^D by the complete QR."""
+    Q, _ = torch.linalg.qr(Xc.mT @ U.mT, mode="complete")
+    return Q.mT
+
+
+def _components(n, s1, s2):
+    """_spectrum with the principal axes: (descending spectrum, eigenvector rows [D, D]) of the ddof=1 covariance."""
+    mean = s1 / n
+    cov = (s2 - n * torch.outer(mean, mean)) / (n - 1)
+    cov = 0.5 * (cov + cov.t())
+    return _desc(*torch.linalg.eigh(cov))
+
+
+def _gram_route_components(rows, n_total, D):
+    """_gram_spectrum with the principal axes: (descending spectrum of length D, axes [D, D])."""
+    X = rows.double()
+    Xc = X - X.mean(0, keepdim=True)
+    w, U = _desc(*torch.linalg.eigh(Xc @ Xc.t() / (n_total - 1)))
+    out = torch.zeros(D, device=rows.device, dtype=torch.float64)
+    out[:w.numel()] = w[:D]
+    return out, _gram_components(Xc, U, D)
+
+
 # Smallest group (number of matrices of one size) from which one ard_sym_eigvals call beats the per-head torch.linalg.eigvalsh loop,
 # per matrix size: the first winning batch of the crossover sweep in profiles/eig_bench.json (B200, 1000 W; batches 1, 2, 4, 8, 16).
 # The library pays its D column steps once per call, so a lone matrix is slower there (4096^2: 0.33 s against 0.08 s) while a batch
@@ -52,45 +82,65 @@ def _library_wins(batch, D):
     return batch >= need
 
 
-def _solve_owned_batched(owned, accs, spectra, D):
+def _solve_owned_batched(owned, accs, spectra, D, comps=None):
     """The owned heads' spectra into `spectra` rows, grouped by route and size: the D x D covariances form one group, the Gram
     matrices one group per sample count. A group at or above the measured crossover (_LIB_MIN_BATCH) is solved by one
     ard_sym_eigvals call on matrices assembled exactly as _spectrum / _gram_spectrum assemble them; a smaller group goes head by
     head through _spectrum / _gram_spectrum (also the route for CPU accumulators). A batched group holds all its matrices at once:
-    28 x 128 MB = 3.8 GB for the covariance heads of one GPU at D = 4096, where the per-head route holds one."""
+    28 x 128 MB = 3.8 GB for the covariance heads of one GPU at D = 4096, where the per-head route holds one.
+    With `comps` (a dict) comps[i] receives head i's principal axes [D, D] (rows, descending variance, not yet sign-fixed), and
+    each group, assembled the same way, goes through linalg.eigh_batch instead: one ard_sym_eigh call where that was measured
+    faster than torch.linalg.eigh per head (its spectra are then bitwise those of ard_sym_eigvals), else torch.linalg.eigh per head."""
     cov = [(i, n_i) for i, n_i, r in owned if r is None]
-    if cov and _library_wins(len(cov), D):
+    if cov and (eigh_library_wins(len(cov), D) if comps is not None else _library_wins(len(cov), D)):
         M = torch.empty((len(cov), D, D), device=spectra.device, dtype=torch.float64)
         for k, (i, n_i) in enumerate(cov):
             mean = accs[i].s1 / n_i
             c = (accs[i].s2 - n_i * torch.outer(mean, mean)) / (n_i - 1)
             M[k] = 0.5 * (c + c.t())
-        w = sym_eigvals(M, overwrite=True).flip(-1).clamp_min(0)
+        if comps is None:
+            w = sym_eigvals(M, overwrite=True).flip(-1).clamp_min(0)
+        else:
+            w, V = _desc(*eigh_batch(M))
+            for k, (i, _) in enumerate(cov):
+                comps[i] = V[k]
         spectra[[i for i, _ in cov]] = w
         del M
     else:
         for i, n_i in cov:
-            spectra[i] = _spectrum(n_i, accs[i].s1, accs[i].s2)
+            if comps is None:
+                spectra[i] = _spectrum(n_i, accs[i].s1, accs[i].s2)
+            else:
+                spectra[i], comps[i] = _components(n_i, accs[i].s1, accs[i].s2)
     grams = defaultdict(list)
     for i, n_i, r in owned:
         if r is not None:
             grams[r.shape[0]].append((i, n_i, r))
     for n, group in grams.items():
-        if not _library_wins(len(group), n):
+        if not (eigh_library_wins(len(group), n) if comps is not None else _library_wins(len(group), n)):
             for i, n_i, r in group:
-                spectra[i] = _gram_spectrum(r, n_i, D)
+                if comps is None:
+                    spectra[i] = _gram_spectrum(r, n_i, D)
+                else:
+                    spectra[i], comps[i] = _gram_route_components(r, n_i, D)
             continue
         G = torch.empty((len(group), n, n), device=spectra.device, dtype=torch.float64)
         for k, (i, n_i, r) in enumerate(group):
             X = r.double()
             Xc = X - X.mean(0, keepdim=True)
             G[k] = Xc @ Xc.t() / (n_i - 1)
-        w = sym_eigvals(G, overwrite=True).flip(-1).clamp_min(0)
+        if comps is None:
+            w = sym_eigvals(G, overwrite=True).flip(-1).clamp_min(0)
+        else:
+            w, U = _desc(*eigh_batch(G))
+            for k, (i, _, r) in enumerate(group):
+                X = r.double()
+                comps[i] = _gram_components(X - X.mean(0, keepdim=True), U[k], D)
         m = min(n, D)
         spectra[[i for i, _, _ in group], :m] = w[:, :m]
 
 
-def finalize_head_spectra(accs, n_components=None):
+def finalize_head_spectra(accs, n_components=None, with_components=False):
     """Spectra of a list of MomentAccumulators (one per (layer, head)), as numpy arrays.
     Under torch.distributed (clip-sharded pass, SURVEY 8e) the moments are summed over ranks with the heads dealt round-robin
     to owners (`reduce` to the owner instead of an allreduce: each 4096^2 float64 matrix crosses NVLink once), every rank
@@ -101,12 +151,18 @@ def finalize_head_spectra(accs, n_components=None):
     rows (not the D x D matrix) go to the owner and the eigen-solve is n x n (9 instead of 79 ms at n = 2000).
     On CUDA accumulators each rank solves a group of same-size heads with one ard_sym_eigvals call instead of one
     torch.linalg.eigvalsh per head, when the group is large enough for that to be faster (_solve_owned_batched); CPU accumulators
-    keep _spectrum / _gram_spectrum."""
+    keep _spectrum / _gram_spectrum.
+    with_components=True returns (spectra, components) instead: components[i] is head i's principal axes, numpy float64
+    [k, D] (k = n_components or D), rows in descending variance, sign-fixed like residual.pca_from_moments. The owner of a head
+    solves it with eigenvectors (ard_sym_eigh where measured faster, spectra then bitwise as without the flag; torch.linalg.eigh
+    per head otherwise, spectra within rounding, see linalg._EIGH_LIB_MIN_BATCH); Gram-route heads take the orthonormalised Xc^T U, completed to a basis of R^D. Under torch.distributed every
+    rank then holds every head's components (one allreduce of a buffer that is zero outside the owner's slots): 60 heads at
+    k = D = 4096 are 8 GB per rank, which is why this is opt-in."""
     import torch.distributed as dist
     world = dist.get_world_size() if dist.is_available() and dist.is_initialized() else 1
     rank = dist.get_rank() if world > 1 else 0
     if not accs:
-        return []
+        return ([], []) if with_components else []
     def local_s1(a):       # first moment without disturbing parked rows (plain accumulators - the gloo tests use them - have only s1)
         if hasattr(a, "_s1"):
             return a._s1 + (a._buf[:a._fill].double().sum(0) if a._fill else 0.0)
@@ -160,16 +216,29 @@ def finalize_head_spectra(accs, n_components=None):
                 owned.append((i, n_i, None))
         a.n = n_i
         a.mean_global = s1[i] / max(n_i, 1)
+    comps = {} if with_components else None
     if dev.type == "cuda":
-        _solve_owned_batched(owned, accs, spectra, D)
+        _solve_owned_batched(owned, accs, spectra, D, comps)
     else:
         for i, n_i, r in owned:
-            spectra[i] = _gram_spectrum(r, n_i, D) if r is not None else _spectrum(n_i, accs[i].s1, accs[i].s2)
+            if comps is not None:
+                spectra[i], comps[i] = _gram_route_components(r, n_i, D) if r is not None else _components(n_i, accs[i].s1, accs[i].s2)
+            else:
+                spectra[i] = _gram_spectrum(r, n_i, D) if r is not None else _spectrum(n_i, accs[i].s1, accs[i].s2)
     if world > 1:
         dist.all_reduce(spectra)
     out = spectra.cpu().numpy()
     k = n_components or D
-    return [out[i, :k] for i in range(len(accs))]
+    spec = [out[i, :k] for i in range(len(accs))]
+    if comps is None:
+        return spec
+    allc = torch.zeros((len(accs), k, D), device=dev, dtype=torch.float64)
+    for i, c in comps.items():
+        allc[i] = sign_fix(c[:k])
+    if world > 1:
+        dist.all_reduce(allc)
+    allc = allc.cpu().numpy()
+    return spec, [allc[i] for i in range(len(accs))]
 
 
 class HeadPCA:
@@ -185,10 +254,13 @@ class HeadPCA:
         self.acc.update(X)
         return self
 
-    def _set(self, w, n_components=None):
+    def _set(self, w, n_components=None, components=None):
         """w: full descending spectrum (numpy). n_components defaults to what IncrementalPCA(n_components=None) settles on at
-        its first partial_fit: min(samples of the first batch, features) (sklearn _incremental_pca.py)."""
+        its first partial_fit: min(samples of the first batch, features) (sklearn _incremental_pca.py). components: the
+        principal axes (numpy rows, descending variance, at least k of them), kept as components_ when given."""
         k = n_components or min(self.first_batch or len(w), len(w))
+        if components is not None:
+            self.components_ = components[:k]
         mean = getattr(self.acc, "mean_global", None)
         self.mean_ = (mean if mean is not None else self.acc.s1 / self.acc.n).cpu().numpy()
         self.explained_variance_ = w[:k]
@@ -197,8 +269,20 @@ class HeadPCA:
         self.n_samples_seen_ = self.acc.n
         return self
 
-    def finalize(self, n_components=None):
-        return self._set(finalize_head_spectra([self.acc])[0], n_components)
+    def finalize(self, n_components=None, with_components=False):
+        """with_components=True also sets components_ [n_components_, D] and enables transform()."""
+        if not with_components:
+            return self._set(finalize_head_spectra([self.acc])[0], n_components)
+        spectra, comps = finalize_head_spectra([self.acc], with_components=True)
+        return self._set(spectra[0], n_components, comps[0])
+
+    def transform(self, X):
+        """(X - mean_) @ components_.T: sklearn IncrementalPCA.transform with whiten=False (numpy float64)."""
+        if not hasattr(self, "components_"):
+            raise AttributeError("HeadPCA.transform needs components_: finalize (or run_PCA) with with_components=True")
+        if isinstance(X, torch.Tensor):
+            X = X.detach().cpu().numpy()
+        return (np.asarray(X, dtype=np.float64) - self.mean_) @ self.components_.T
 
 
 def extract_attention(clap, X, max_len=480000, data_filling="repeatpad", pad_or_truncate=False):
@@ -213,8 +297,10 @@ def extract_attention(clap, X, max_len=480000, data_filling="repeatpad", pad_or_
     return out["layers_attention"]
 
 
-def run_PCA(clap, dataloader, num_layers, num_heads, components=None, data_filling="repeatpad", pad_or_truncate=False):
-    """src/analyze_attention.py:13-59. Returns {layer: {head: fitted HeadPCA}}."""
+def run_PCA(clap, dataloader, num_layers, num_heads, components=None, data_filling="repeatpad", pad_or_truncate=False,
+            with_components=False):
+    """src/analyze_attention.py:13-59. Returns {layer: {head: fitted HeadPCA}}. with_components=True also gives every HeadPCA its
+    components_ and transform() (finalize_head_spectra: up to 8 GB of float64 axes on every rank for 60 heads)."""
     pca_models = defaultdict(dict)
     dev = clap.device
     for l in range(num_layers):
@@ -226,8 +312,14 @@ def run_PCA(clap, dataloader, num_layers, num_heads, components=None, data_filli
             for h in range(layer_attn.shape[1]):
                 pca_models[l][h].partial_fit(layer_attn[:, h].reshape(layer_attn.shape[0], 4096))
     models = [pca_models[l][h] for l in pca_models for h in pca_models[l]]
-    for m, w in zip(models, finalize_head_spectra([m.acc for m in models])):   # heads sharded over ranks when distributed
-        m._set(w, components)
+    accs = [m.acc for m in models]
+    if with_components:
+        spectra, comps = finalize_head_spectra(accs, with_components=True)   # heads sharded over ranks when distributed
+        for m, w, c in zip(models, spectra, comps):
+            m._set(w, components, c)
+    else:
+        for m, w in zip(models, finalize_head_spectra(accs)):
+            m._set(w, components)
     return pca_models
 
 

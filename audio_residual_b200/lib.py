@@ -94,6 +94,9 @@ def load(check_symbols=False):
         lib.ard_sym_eigvals_workspace.restype = C.c_longlong
         lib.ard_sym_eigvals_workspace.argtypes = [i, i]
         lib.ard_sym_eigvals.argtypes = [vp, ll, i, i, vp, vp, ll, vp]
+        lib.ard_sym_eigh_workspace.restype = C.c_longlong
+        lib.ard_sym_eigh_workspace.argtypes = [i, i]
+        lib.ard_sym_eigh.argtypes = [vp, ll, i, i, vp, vp, ll, vp, vp, ll, vp]
         lib.ard_tape_generation.argtypes = [vp]
         lib.ard_residual_forward.argtypes = [vp, vp, vp, vp, vp, ll, i, i, vp]
         lib.ard_residual_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, ll, i, i, vp]

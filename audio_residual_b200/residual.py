@@ -252,8 +252,12 @@ class MomentAccumulator:
             self.n = int(n.item())
         return self
 
-    def pca(self):
-        return pca_from_moments(self.n, self.s1.cpu().numpy(), self.s2.cpu().numpy())
+    def pca(self, n_components=None):
+        """PCA dict (pca_from_moments' schema) of the moments. On a CUDA accumulator the covariance is assembled and solved on the
+        device (pca_on_device); on the CPU it goes through pca_from_moments."""
+        if self._s1.device.type == "cuda":
+            return pca_on_device(self.n, self.s1, self.s2, n_components)
+        return pca_from_moments(self.n, self.s1.cpu().numpy(), self.s2.cpu().numpy(), n_components)
 
 
 def pca_from_moments(n, s1, s2, n_components=None):
@@ -279,6 +283,25 @@ def pca_from_moments(n, s1, s2, n_components=None):
             "n_components": k, "input_dim": comps.shape[1], "num_samples": int(n)}
 
 
+def pca_on_device(n, s1, s2, n_components=None):
+    """pca_from_moments for float64 moments on a CUDA device: the ddof=1 covariance is assembled there and solved there, by
+    ard_sym_eigh or torch.linalg.eigh, whichever was measured faster at this width (linalg.eigh_batch); ordering, clamping, the
+    sign rule and the truncation to n_components (from the one solve) are pca_from_moments'. Returns the same dict of numpy float64
+    arrays."""
+    from .linalg import eigh_batch, sign_fix
+    mean = s1 / n
+    cov = (s2 - n * torch.outer(mean, mean)) / (n - 1)
+    cov = 0.5 * (cov + cov.t())
+    w, Q = eigh_batch(cov[None])
+    w, Q = w[0], Q[0]
+    k = n_components or cov.shape[0]
+    comps = sign_fix(Q.mT.flip(0)[:k])
+    w = w.flip(0).clamp_min(0).cpu().numpy()
+    total = w.sum()
+    return {"components": comps.cpu().numpy(), "mean": mean.cpu().numpy(), "explained_variance": w[:k],
+            "explained_variance_ratio": w[:k] / total, "n_components": k, "input_dim": cov.shape[0], "num_samples": int(n)}
+
+
 def compute_pca_components(model, dataloader, target_layer, n_components=None, max_batches=None, save_path=None, max_len=480000,
                            data_filling="repeatpad", pad_or_truncate=False):
     """src/residual.py:103-159. `model` is the CLAP_Module wrapper; batches are (waveform[B,1,T], ...)."""
@@ -302,9 +325,7 @@ def compute_pca_components(model, dataloader, target_layer, n_components=None, m
             acc.update(res)
     if acc is None:
         raise ValueError("compute_pca_components: the dataloader produced no batch")
-    pca_results = acc.allreduce().pca()
-    if n_components:
-        pca_results = pca_from_moments(acc.n, acc.s1.cpu().numpy(), acc.s2.cpu().numpy(), n_components)
+    pca_results = acc.allreduce().pca(n_components)
     if save_path:
         os.makedirs(os.path.dirname(save_path), exist_ok=True)
         with open(save_path, "wb") as f:

@@ -283,6 +283,21 @@ long long ard_sym_eigvals_workspace(int D, int batch);
 int ard_sym_eigvals(double* A, long long stride, int D, int batch, double* w, void* work, long long work_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------
+ * Eigenvalues and eigenvectors of `batch` symmetric matrices A[b], laid out as for ard_sym_eigvals (lower triangle read, A
+ * overwritten). w [batch, D] fp64 device, ascending, bitwise identical to ard_sym_eigvals on the same input (same reduction and
+ * bisection). Z[b] at Z + b*zstride: row-major D x D, row m the unit eigenvector of w[b][m]. info [batch] device int: 0, or the
+ * number of off-diagonals the tridiagonal QL iteration left unconverged after 30 D sweeps (then Z[b] is not to be used). work:
+ * device scratch of at least ard_sym_eigh_workspace(D, batch) bytes (it holds a D x D matrix per batch entry). The eigen-solve
+ * behind compute_pca_components (src/residual.py:103-159) and run_PCA's per-head components (src/analyze_attention.py:13-59).
+ * Householder tridiagonalisation keeping its reflectors (dsytrd), Sturm bisection (dstebz), implicit QL with the rotations
+ * accumulated on the device (tql2), blocked back-transformation (dlarft / dlarfb); asynchronous on `stream`. ARD_ERR_SHAPE
+ * (before any device work): every case of ard_sym_eigvals, a NULL Z or info, zstride < D*D, D > 12288.
+ * ------------------------------------------------------------------------------------------------------------------ */
+long long ard_sym_eigh_workspace(int D, int batch);
+int ard_sym_eigh(double* A, long long stride, int D, int batch, double* w, double* Z, long long zstride, int* info,
+                 void* work, long long work_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------
  * Measurement support (bench.py): per-kernel-class device time. Classes: 0 tcgen05 GEMM, 1 window attention,
  * 2 LayerNorm/merge, 3 front end (STFT/log-mel/patch-embed), 4 heads, 5 other, 6 fused FFN. While enabled every launch is bracketed
  * by CUDA events on its stream; ard_profile_read synchronises, sums elapsed ms / algorithmic flops / algorithmic bytes /
