@@ -283,54 +283,60 @@ int ensure_fold(ard_handle* h, int l, int b, cudaStream_t s) {
     return 0;
 }
 
-// One Swin block on the residual stream held in X (fp32 [B*T, C]); Y is scratch. Result ends in X.
-//   plain  : htsat.py:439-482            patched: src/residual.py:58-98 (doubled shortcut + FFN, SURVEY Q2)
-static int run_block(ard_handle* h, int l, int b, int B, float* X, float* Y, float* attn_out, float attn_scale, int attn_acc,
-                     float* res_out, long long res_bstride, int res_T, float* head_tap, cudaStream_t s) {
+// Where one block reads and writes. Inference: s = out = X (the residual stream), x1 = x3 = Y (scratch), qkv / ao in the
+// workspace. Training (tape): the block's tape slots (ard_train.cu), so the backward finds every intermediate it needs and the
+// training forward computes bit for bit what inference does.
+struct BlockIO {
+    float *s, *x1, *x3, *out;
+    __nv_bfloat16 *qkv, *ao;
+    bool tape;   // qkv / ao must be materialised (the fused attention block keeps them on chip)
+};
+
+// One Swin block: plain htsat.py:439-482, patched src/residual.py:58-98 (doubled shortcut + FFN, SURVEY Q2).
+static int run_block(ard_handle* h, int l, int b, int B, const BlockIO& io, float* attn_out, float attn_scale, int attn_acc,
+                     float* res_out, long long res_bstride, float* head_tap, cudaStream_t s) {
     BlockW& bw = h->layers[l].blocks[b];
     const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
     const long long M = (long long)B * T;
     __nv_bfloat16* XN = h->ws_xn.as<__nv_bfloat16>();
-    __nv_bfloat16* AO = h->ws_ao.as<__nv_bfloat16>();
-    __nv_bfloat16* QKV = h->ws_qkv.as<__nv_bfloat16>();
     __nv_bfloat16* Hb = h->ws_h.as<__nv_bfloat16>();
     const int shift = (b % 2 == 0) ? 0 : 4;   // htsat.py:563
 
     GemmArgs g;
-    const bool fused_attn = h->use_attn_block && bw.ab.ready && !attn_out && !res_out && !head_tap && (R % 16) == 0;
+    const bool fused_attn = h->use_attn_block && bw.ab.ready && !io.tape && !attn_out && !res_out && !head_tap && (R % 16) == 0;
     if (fused_attn) {
-        // norm1 + qkv + window attention + (folded) projection + shortcut in ONE kernel: Y = X + r. q/k/v, the attention
-        // probabilities and the attention output never reach HBM (capture outputs need them: those calls take the path below)
+        // norm1 + qkv + window attention + (folded) projection + shortcut in ONE kernel: x1 = s + r. q/k/v, the attention
+        // probabilities and the attention output never reach HBM (capture outputs and the tape need them: those calls take the path below)
         ARD_TRY(ensure_fold(h, l, b, s));
-        ARD_TRY(attn_block_96(X, Y, bw.ab, (bw.has_res ? bw.ab.wp_fold : bw.ab.wp_plain).as<__nv_bfloat16>(),
+        ARD_TRY(attn_block_96(io.s, io.x1, bw.ab, (bw.has_res ? bw.ab.wp_fold : bw.ab.wp_plain).as<__nv_bfloat16>(),
                               (bw.has_res ? bw.ab.bp_fold : bw.ab.bp_plain).as<float>(), bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), B, R, shift,
                               h->num_sms, s));
     } else {
     if (C == 96 && h->use_ln_qkv) {   // norm1 + qkv in one kernel: the bf16 LayerNorm output never reaches HBM
-        ARD_TRY(ln_qkv_96(X, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), bw.qkv_w.as<__nv_bfloat16>(), bw.qkv_b.as<float>(), QKV, M, h->num_sms, s));
+        ARD_TRY(ln_qkv_96(io.s, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), bw.qkv_w.as<__nv_bfloat16>(), bw.qkv_b.as<float>(), io.qkv, M,
+                          h->num_sms, s));
     } else {
-        ARD_TRY(layernorm_bf16(X, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), XN, M, C, s));
-        g.A = XN; g.lda = C; g.W = bw.qkv_w.as<__nv_bfloat16>(); g.ldw = C; g.out = QKV; g.ldo = 3 * C; g.out_bf16 = 1;
+        ARD_TRY(layernorm_bf16(io.s, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), XN, M, C, s));
+        g.A = XN; g.lda = C; g.W = bw.qkv_w.as<__nv_bfloat16>(); g.ldw = C; g.out = io.qkv; g.ldo = 3 * C; g.out_bf16 = 1;
         g.M = (int)M; g.N = 3 * C; g.K = C; g.bias = bw.qkv_b.as<float>();
         ARD_TRY(gemm_bf16(g, h->num_sms, s));
     }
     AttnArgs a;
-    a.qkv = QKV; a.out = AO; a.bias_table = bw.rpb.as<float>(); a.attn_mean = attn_out; a.attn_scale = attn_scale; a.attn_accumulate = attn_acc;
+    a.qkv = io.qkv; a.out = io.ao; a.bias_table = bw.rpb.as<float>(); a.attn_mean = attn_out; a.attn_scale = attn_scale; a.attn_accumulate = attn_acc;
     a.B = B; a.H = R; a.W = R; a.C = C; a.nH = nH; a.shift = shift;
     ARD_TRY(window_attention(a, s));
-    if (head_tap) ARD_TRY(head_output_tap(AO, head_tap, B, R, C, nH, shift, s));   // per-head attn @ v (htsat.py:354)
-    // proj (+ folded ResiDual) + shortcut:  Y = X + r,  aux = r = residual_x
+    if (head_tap) ARD_TRY(head_output_tap(io.ao, head_tap, B, R, C, nH, shift, s));   // per-head attn @ v (htsat.py:354)
+    // proj (+ folded ResiDual) + shortcut:  x1 = s + r,  aux = r = residual_x
     ARD_TRY(ensure_fold(h, l, b, s));
     g = GemmArgs();
-    g.A = AO; g.lda = C; g.ldw = C; g.out = Y; g.ldo = C; g.M = (int)M; g.N = C; g.K = C;
+    g.A = io.ao; g.lda = C; g.ldw = C; g.out = io.x1; g.ldo = C; g.M = (int)M; g.N = C; g.K = C;
     if (bw.has_res) { g.W = bw.proj_w_fold.as<__nv_bfloat16>(); g.bias = bw.proj_b_fold.as<float>(); }
     else { g.W = bw.proj_w.as<__nv_bfloat16>(); g.bias = bw.proj_b.as<float>(); }
-    g.resid1 = X; g.ldr1 = C;
-    if (res_out) { g.aux = res_out; g.ld_aux = C; g.aux_T = T; g.aux_bstride = res_bstride; (void)res_T; }
+    g.resid1 = io.s; g.ldr1 = C;
+    if (res_out) { g.aux = res_out; g.ld_aux = C; g.aux_T = T; g.aux_bstride = res_bstride; }
     ARD_TRY(gemm_bf16(g, h->num_sms, s));
     }
-    // FFN: (Y) -> LN2 -> fc1+GELU -> fc2
-    // one FFN: out = in + mlp(norm2(in)) (+ r2 inside the fused kernel). `pre_add`: the LayerNorm input is in + pre_add, written back to `in`.
+    // one FFN: out = in + mlp(norm2(in)) (+ r2), the second residual inside the fused kernel or the fc2 epilogue.
     // HTSAT-base widths (C = 128 / 256) are opt-in (ARD_FUSED_FFN_WIDE=3): the kernel passes its parity tests there and is 6 % faster
     // on the base model (24.0 -> 22.6 ms per 256 clips), but with it the FIRST graph executions of a fresh handle faulted
     // ("unspecified launch failure") 6 times in ~260 tries against 0 in ~280 without it; the cause is not found, so the default keeps
@@ -339,18 +345,16 @@ static int run_block(ard_handle* h, int l, int b, int B, float* X, float* Y, flo
     // 192-channel stage (217 / 255 us plain / with second residual vs 341 / 339 us at B = 256). At C = 384 (254 vs 200 us: three
     // ring slots cannot cover the L2 latency) the unfused chain stays. ARD_FUSED_FFN_WIDE=2 forces it for C = 384 too (A/B
     // measurements), =0 disables it.
-    const bool wide = (((C == 192 && h->use_fused_ffn_wide >= 1) || ((C == 128 || C == 256) && h->use_fused_ffn_wide >= 3)) || (C == 384 && h->use_fused_ffn_wide >= 2)) && C != h->wide_skip;
-    auto ffn = [&](float* in, float* out, const float* r2, const float* pre_add) -> int {
-        if (C == 96 && h->use_fused_ffn && pre_add == nullptr)   // whole FFN in one kernel, hidden activation never leaves the SM
+    const bool wide = (C == 192 && h->use_fused_ffn_wide >= 1) || ((C == 128 || C == 256) && h->use_fused_ffn_wide >= 3) ||
+                      (C == 384 && h->use_fused_ffn_wide >= 2);
+    auto ffn = [&](const float* in, float* out, const float* r2) -> int {
+        if (C == 96 && h->use_fused_ffn)   // whole FFN in one kernel, hidden activation never leaves the SM
             return ffn_fused_96(in, r2, out, M, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), bw.fc1_w.as<__nv_bfloat16>(), bw.fc1_b.as<float>(),
                                 bw.fc2_w.as<__half>(), bw.fc2_b.as<float>(), h->num_sms, s);
-        if (wide && pre_add == nullptr)                          // same, weights streamed from L2
+        if (wide)                          // same, weights streamed from L2
             return ffn_fused_wide(in, r2, out, M, C, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), bw.fc1_w.as<__nv_bfloat16>(),
                                   bw.fc1_b_half.as<float>(), bw.fc2_w.as<__half>(), bw.fc2_b.as<float>(), h->num_sms, s);
-        if (pre_add)
-            ARD_TRY(add_layernorm_bf16(in, pre_add, in, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), XN, M, C, s));
-        else
-            ARD_TRY(layernorm_bf16(in, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), XN, M, C, s));
+        ARD_TRY(layernorm_bf16(in, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), XN, M, C, s));
         GemmArgs f;
         f.A = XN; f.lda = C; f.W = bw.fc1_w.as<__nv_bfloat16>(); f.ldw = C; f.out = Hb; f.ldo = 4 * C; f.out_bf16 = 1;
         f.M = (int)M; f.N = 4 * C; f.K = C; f.bias = bw.fc1_b.as<float>(); f.act = ARD_ACT_GELU; f.out_f16 = 1;
@@ -358,19 +362,12 @@ static int run_block(ard_handle* h, int l, int b, int B, float* X, float* Y, flo
         f = GemmArgs();
         f.A = Hb; f.lda = 4 * C; f.W = bw.fc2_w.as<__nv_bfloat16>(); f.ldw = 4 * C; f.out = out; f.ldo = C; f.ab_f16 = 1;
         f.M = (int)M; f.N = C; f.K = 4 * C; f.bias = bw.fc2_b.as<float>();
-        f.resid1 = in; f.ldr1 = C; f.resid2 = r2; f.ldr2 = C;
+        f.resid1 = in; f.ldr1 = C; f.resid2 = r2; f.ldr2 = C;   // ((acc + b) + in) + r2
         return gemm_bf16(f, h->num_sms, s);
     };
-    if (!bw.has_res) {
-        ARD_TRY(ffn(Y, X, nullptr, nullptr));          // x = x1 + mlp(norm2(x1))                       htsat.py:480
-    } else if ((C == 96 && h->use_fused_ffn) || wide) {
-        ARD_TRY(ffn(Y, Y, X, nullptr));                // x3 = shortcut + (x1 + mlp(norm2(x1)))         src/residual.py:93,95
-        ARD_TRY(ffn(Y, X, nullptr, nullptr));          // x4 = x3 + mlp(norm2(x3))                      src/residual.py:96
-    } else {
-        ARD_TRY(ffn(Y, Y, nullptr, nullptr));          // x2 = x1 + mlp(norm2(x1))                      src/residual.py:93
-        ARD_TRY(ffn(Y, X, nullptr, X));                // x3 = shortcut + x2 (fused into the norm2 pass), x4 = x3 + mlp(norm2(x3))   :95-96
-    }
-    return 0;
+    if (!bw.has_res) return ffn(io.x1, io.out, nullptr);     // htsat.py:480
+    ARD_TRY(ffn(io.x1, io.x3, io.s));                        // x3 = shortcut + (x1 + mlp(norm2(x1)))   src/residual.py:93,95
+    return ffn(io.x3, io.out, nullptr);                      // x4 = x3 + mlp(norm2(x3))                src/residual.py:96
 }
 
 static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_t s) {
@@ -414,13 +411,11 @@ static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_
             float* res = a->layers_residuals[l] ? a->layers_residuals[l] + (long long)b * T * C : nullptr;
             // BasicLayer.forward (htsat.py:589-596): mean of the blocks' maps; residuals concatenated along tokens
             float* tap = a->head_outputs[l] ? a->head_outputs[l] + (long long)b * B * T * C : nullptr;
-            if (train) {
-                ARD_TRY(run_block_train(h, l, b, B, a->layers_attention[l], 1.0f / depth, b > 0, res, (long long)depth * T, s));
-                if (tap) ARD_TRY(head_output_tap(h->layers[l].blocks[b].t_ao, tap, B, R, C, h->cfg.num_heads[l], (b % 2 == 0) ? 0 : 4, s));
-                X = h->layers[l].blocks[b].t_out;
-            } else {
-                ARD_TRY(run_block(h, l, b, B, X, Y, a->layers_attention[l], 1.0f / depth, b > 0, res, (long long)depth * T, T, tap, s));
-            }
+            const BlockW& bw = h->layers[l].blocks[b];
+            const BlockIO io = train ? BlockIO{bw.t_s, bw.t_x1, bw.t_x3, bw.t_out, bw.t_qkv, bw.t_ao, true}
+                                     : BlockIO{X, Y, Y, X, h->ws_qkv.as<__nv_bfloat16>(), h->ws_ao.as<__nv_bfloat16>(), false};
+            ARD_TRY(run_block(h, l, b, B, io, a->layers_attention[l], 1.0f / depth, b > 0, res, (long long)depth * T, tap, s));
+            if (train) X = bw.t_out;
         }
         if (l < h->nlayers - 1) {   // PatchMerging (htsat.py:505-526)
             __nv_bfloat16* Hb = h->ws_h.as<__nv_bfloat16>();
@@ -505,13 +500,11 @@ int ard_create(const ard_config* cfg, ard_handle** out) {
     if (const char* e = getenv("ARD_LN_QKV")) h->use_ln_qkv = atoi(e) != 0;
     if (const char* e = getenv("ARD_ATTN_BLOCK")) h->use_attn_block = atoi(e) != 0;
     if (const char* e = getenv("ARD_DUAL_GEMM")) h->use_dual_gemm = atoi(e);
-    if (const char* e = getenv("ARD_FFN_WIDE_SKIP")) h->wide_skip = atoi(e);   // development: one width back on the unfused chain
     *out = h;
     return 0;
 }
 
 int ard_destroy(ard_handle* h) {
-    if (h) fp32_release(h);
     delete h;
     return 0;
 }
@@ -727,8 +720,10 @@ int ard_block_forward(ard_handle* h, int layer, int block, const float* x_in, in
     const int C = C_of(h, layer), T = R_of(layer) * R_of(layer);
     const size_t bytes = (size_t)B * T * C * 4;
     float* X = h->ws_x.as<float>();
+    float* Y = h->ws_y.as<float>();
     ARD_CUDA(cudaMemcpyAsync(X, x_in, bytes, cudaMemcpyDeviceToDevice, s));
-    ARD_TRY(run_block(h, layer, block, B, X, h->ws_y.as<float>(), attn, 1.0f, 0, residual_x, T, T, nullptr, s));
+    const BlockIO io{X, Y, Y, X, h->ws_qkv.as<__nv_bfloat16>(), h->ws_ao.as<__nv_bfloat16>(), false};
+    ARD_TRY(run_block(h, layer, block, B, io, attn, 1.0f, 0, residual_x, T, nullptr, s));
     ARD_CUDA(cudaMemcpyAsync(x_out, X, bytes, cudaMemcpyDeviceToDevice, s));
     h->last_launches = g_launches;
     return 0;
@@ -766,8 +761,8 @@ long long ard_tape_generation(const ard_handle* h) { return h && h->tape_B > 0 ?
 long long ard_workspace_bytes(const ard_handle* h) {
     if (!h) return 0;
     const DevBuf* bufs[] = {&h->ws_logmel, &h->ws_x, &h->ws_y, &h->ws_xn, &h->ws_ao, &h->ws_qkv, &h->ws_h, &h->ws_normed,
-                            &h->ws_emb, &h->ws_hid, &h->ws_proj, &h->ws_tscam_a, &h->ws_tscam_y, &h->ws_wave, &h->tape, &h->bw_g,
-                            &h->bw_gs, &h->bw_t, &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small, &h->bw_g3};
+                            &h->ws_hid, &h->ws_proj, &h->ws_tscam_a, &h->ws_tscam_y, &h->tape, &h->bw_g, &h->bw_gs, &h->bw_t,
+                            &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small, &h->bw_g3};
     long long t = 0;
     for (const DevBuf* b : bufs) t += (long long)b->bytes;
     return t;

@@ -1,4 +1,5 @@
-// Handle layout shared by ard_api.cu (forward schedule, C ABI) and ard_train.cu (saved activations + backward schedule).
+// Handle layout shared by ard_api.cu (forward schedule, C ABI), ard_train.cu (tape layout + backward schedule) and
+// fp32_mode.cu (fp32-grade forward).
 #pragma once
 #include <map>
 #include <string>
@@ -51,8 +52,8 @@ struct BlockW {
     int Kp = 0;
     bool bwd_ready = false;
     DevBuf lam, fc1_wT, fc2_wT, qkv_wT, proj_wT, res_wc, res_wcT, res_basis_bf16, res_c0;
-    // activations saved by a save_for_backward forward (views into ard_handle::tape); qkv / ao are bf16 on a bf16 tape
-    // (t_qkv, t_ao) and fp32 on an fp32-grade tape (t_qkvf, t_aof), the other pair is null
+    // activations saved by a save_for_backward forward (views into ard_handle::tape, the block's BlockIO / Fp32BlockIO in that
+    // forward); qkv / ao are bf16 on a bf16 tape (t_qkv, t_ao) and fp32 on an fp32-grade tape (t_qkvf, t_aof), the other pair is null
     float *t_s = nullptr, *t_x1 = nullptr, *t_x3 = nullptr, *t_out = nullptr;
     __nv_bfloat16 *t_qkv = nullptr, *t_ao = nullptr;
     float *t_qkvf = nullptr, *t_aof = nullptr;
@@ -62,11 +63,29 @@ struct LayerW {
     DevBuf mg_g, mg_b, mg_w, mg_wT;
 };
 
+// fp32-grade mode (fp32_mode.cu). Split weights [W_hi | W_lo | W_hi] ([N, 3K] bf16) of the forward GEMMs and, built on the
+// first fp32-grade backward, of the backward's dgrad GEMMs; all rebuilt when ard_handle::graph_epoch moves.
+struct Fp32BlockW {
+    DevBuf qkv3, proj3, fc13, fc23;
+    DevBuf fc1T3, fc2T3, qkvT3, projT3;                // [C, 3*4C], [4C, 3C], [C, 3*3C] (q rows pre-scaled), [C, 3C]
+    DevBuf wc3, wcT3, basis3;                          // ResiDual: Wc = B Wp [Kp, 3C], Wc^T [C, 3Kp], basis padded to Kp [Kp, 3C]
+};
+struct Fp32Weights {
+    unsigned long long epoch = ~0ULL;            // ard_handle::graph_epoch the split weights were built at (weights / ResiDual changes bump it)
+    unsigned long long bwd_epoch = ~0ULL;        // the same for the backward set (built by the first fp32-grade backward after a change)
+    std::vector<std::vector<Fp32BlockW>> blocks;
+    std::vector<DevBuf> merge3, mergeT3;         // PatchMerging reduction [2C, 3*4C] and its transpose [4C, 3*2C] (backward, lazily)
+    DevBuf tscam3, scratch;
+    DevBuf fold3;                                // folded projection of the block being run: depends on the current lambda, re-split per call
+    DevBuf qkvf, aof, s3;                        // workspace: fp32 [M,4C] (qkv / FFN hidden), fp32 [M,C], split operands [M,12C] bf16
+};
+
 }  // namespace ard
 
 struct ard_handle {
     using DevBuf = ard::DevBuf;
     using LayerW = ard::LayerW;
+    using Fp32Weights = ard::Fp32Weights;
     ard_config cfg;
     int nlayers = 4;
     int num_sms = 148;
@@ -81,18 +100,18 @@ struct ard_handle {
     std::vector<LayerW> layers;
     DevBuf norm_g, norm_b, tscam_w, tscam_b, p0_w, p0_b, p2_w, p2_b;
     // workspace
-    DevBuf ws_logmel, ws_x, ws_y, ws_xn, ws_ao, ws_qkv, ws_h, ws_normed, ws_emb, ws_hid, ws_proj, ws_tscam_a, ws_tscam_y, ws_wave;
+    DevBuf ws_logmel, ws_x, ws_y, ws_xn, ws_ao, ws_qkv, ws_h, ws_normed, ws_hid, ws_proj, ws_tscam_a, ws_tscam_y;
     int last_launches = 0;
     bool use_fused_ffn = true;   // ARD_FUSED_FFN=0 disables the fused 96-channel FFN kernel (A/B measurements)
     bool use_ln_qkv = true;      // ARD_LN_QKV=0: LayerNorm kernel + qkv GEMM instead of ln_qkv_96 (A/B measurements)
     bool use_attn_block = true;  // ARD_ATTN_BLOCK=0: ln_qkv + window_attention + proj GEMM instead of attn_block_96 (A/B measurements)
     int use_dual_gemm = 1;       // ARD_DUAL_GEMM: backward with gemm_dual (1, default) or the separate GEMMs + lambda_grad kernel (0; A/B measurements)
-    int wide_skip = 0;           // ARD_FFN_WIDE_SKIP=<C>: that width takes the unfused FFN chain (development)
     int use_fused_ffn_wide = 1;    // ARD_FUSED_FFN_WIDE: 0 never, 1 C = 192 (default), 2 also C = 384, 3 also the HTSAT-base widths 128 / 256 (opt-in, see ard_api.cu)
     // training state
-    DevBuf tape, p0_wT, p2_wT, t_emb, t_hid, t_proj;
-    DevBuf bw_g, bw_gs, bw_t, bw_hpre, bw_dh, bw_gqkv, bw_gb, bw_coef, bw_gcoef, bw_gsc, bw_small;
+    DevBuf tape, p0_wT, p2_wT;
+    DevBuf bw_g, bw_gs, bw_t, bw_dh, bw_gb, bw_coef, bw_gcoef, bw_gsc, bw_small;
     DevBuf bw_g3;            // fp32-grade backward: split form [hi | hi | lo] of the gradient entering a dgrad GEMM
+    Fp32Weights fp32;        // fp32-grade split weights and workspace (ensure_fp32_weights)
     int tape_B = 0;          // batch of the forward whose activations the tape holds (0: none)
     int tape_prec = 0;       // ard_forward_args.precision of that forward: the layout of the tape and the backward schedule
     long long tape_gen = 0;  // serial number of that forward (ard_tape_generation): a backward built on an older one is refused
@@ -140,30 +159,14 @@ int ensure_workspace(ard_handle* h, int B);
 int ensure_fold(ard_handle* h, int l, int b, cudaStream_t s);
 // training (ard_train.cu)
 int ensure_tape(ard_handle* h, int B, int precision);
-int run_block_train(ard_handle* h, int l, int b, int B, float* attn_out, float attn_scale, int attn_acc, float* res_out,
-                    long long res_bstride, cudaStream_t s);
 int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s);
 // window-resident attention block (attn_block.cu)
 int attn_block_pack(AttnBlockW& w, const std::vector<float>& qkv_w, const std::vector<float>& qkv_b, const std::vector<float>& rpb, int C, int nH);
 int attn_block_pad_proj(const __nv_bfloat16* w, const float* bp, const float* bv, __nv_bfloat16* out, float* bp_eff, int C, int nH, cudaStream_t s);
 int attn_block_96(const float* x, float* out, const AttnBlockW& w, const __nv_bfloat16* wp_pad, const float* bp, const float* gamma,
                   const float* beta, int B, int R, int shift, int num_sms, cudaStream_t stream);
-// fp32-grade mode (fp32_mode.cu). Split weights [W_hi | W_lo | W_hi] ([N, 3K] bf16) of the forward GEMMs and, built on the
-// first fp32-grade backward, of the backward's dgrad GEMMs; all rebuilt when ard_handle::graph_epoch moves.
-struct Fp32BlockW {
-    DevBuf qkv3, proj3, fc13, fc23;
-    DevBuf fc1T3, fc2T3, qkvT3, projT3;                // [C, 3*4C], [4C, 3C], [C, 3*3C] (q rows pre-scaled), [C, 3C]
-    DevBuf wc3, wcT3, basis3;                          // ResiDual: Wc = B Wp [Kp, 3C], Wc^T [C, 3Kp], basis padded to Kp [Kp, 3C]
-};
-struct Fp32Weights {
-    unsigned long long epoch = ~0ULL;            // ard_handle::graph_epoch the split weights were built at (weights / ResiDual changes bump it)
-    unsigned long long bwd_epoch = ~0ULL;        // the same for the backward set (built by the first fp32-grade backward after a change)
-    std::vector<std::vector<Fp32BlockW>> blocks;
-    std::vector<DevBuf> merge3, mergeT3;         // PatchMerging reduction [2C, 3*4C] and its transpose [4C, 3*2C] (backward, lazily)
-    DevBuf tscam3, scratch;
-    DevBuf qkvf, aof, s3;                        // workspace: fp32 [M,4C] (qkv / FFN hidden), fp32 [M,C], split operands [M,12C] bf16
-};
-int fp32_weights(ard_handle* h, Fp32Weights** out, cudaStream_t s);   // the handle's split weights, forward set current
+// fp32-grade mode (fp32_mode.cu)
+int ensure_fp32_weights(ard_handle* h, cudaStream_t s);   // h->fp32: forward split weights current
 int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s);
 int split3_weight_host(const std::vector<float>& w, DevBuf& scratch, DevBuf& out, long long N, int K, cudaStream_t s, float scale = 1.0f,
                        long long scaled_rows = 0);
@@ -174,5 +177,4 @@ int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, c
                              cudaStream_t s);
 int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, float* Y, float** x_final, cudaStream_t s);
 int tscam_gemm_fp32(ard_handle* h, const float* normed, float* y, int ldy, int B, cudaStream_t s);
-void fp32_release(const ard_handle* h);
 }  // namespace ard

@@ -95,9 +95,6 @@ int ln_qkv_96(const float* x, const float* gamma, const float* beta, const __nv_
 // ---------------------------------------------------------------- row-wise kernels (rowwise.cu)
 // LayerNorm over the last dim C of x[rows, C] (fp32) -> bf16; two-pass variance like at::native layer_norm.
 int layernorm_bf16(const float* x, const float* gamma, const float* beta, __nv_bfloat16* out, long long rows, int C, cudaStream_t s);
-// sum_out = x + add (fp32), out = LayerNorm(sum_out) (bf16); sum_out may alias x.
-int add_layernorm_bf16(const float* x, const float* add, float* sum_out, const float* gamma, const float* beta, __nv_bfloat16* out,
-                       long long rows, int C, cudaStream_t s);
 // PatchMerging gather (htsat.py:516-521) + LayerNorm(4C) -> bf16 [B*(H/2)*(W/2), 4C]
 int merge_layernorm_bf16(const float* x, const float* gamma, const float* beta, __nv_bfloat16* out, int B, int H, int W, int C,
                          cudaStream_t s);

@@ -1,5 +1,7 @@
-// Training path of libard_b200.so: the forward that keeps what the backward needs, and the backward schedule that
-// produces the gradient of a loss on audio_embed / embedding w.r.t. every ResiDual `learnable` vector (lambda).
+// Training path of libard_b200.so: the layout of what the forward keeps for the backward, and the backward schedule that
+// produces the gradient of a loss on audio_embed / embedding w.r.t. every ResiDual `learnable` vector (lambda). The training
+// forward is the inference block schedule itself (run_block in ard_api.cu, run_block_fp32 in fp32_mode.cu) pointed at the
+// block's tape slots instead of the workspace, so it computes bit for bit what inference computes.
 //
 // Reference: train_one_epoch  src/training.py:18-37 (loss.backward() through the frozen, eval-mode encoder into
 // ResiDual.learnable, src/residual.py:26-27,39) with the patched block forward src/residual.py:58-98.
@@ -13,9 +15,9 @@
 //   qkv bf16 [M,3C], ao bf16 [M,C]  attention input / output in token order (fp32 on the fp32-grade tape, precision = 1)
 // LayerNorm outputs, the FFN hidden pre-activation and the attention probabilities are recomputed in the backward.
 //
-// fp32-grade training (precision = 1): the forward is the fp32-grade mode (fp32_mode.cu) writing the same tape slots, and the
-// backward mirrors the bf16 schedule step for step with every dgrad a 3-term split-bf16 GEMM (gemm3) and everything between
-// the GEMMs fp32: the attention backward on CUDA cores, gelu' and the lambda product writing the split form directly.
+// fp32-grade training (precision = 1): the forward writes the same tape slots with qkv / ao in fp32, and the backward mirrors
+// the bf16 schedule step for step with every dgrad a 3-term split-bf16 GEMM (gemm3) and everything between the GEMMs fp32:
+// the attention backward on CUDA cores, gelu' and the lambda product writing the split form directly.
 #include <string.h>
 
 #include "ard_handle.h"
@@ -207,60 +209,6 @@ static int ensure_backward_weights_fp32(ard_handle* h, Fp32Weights& w, cudaStrea
     return 0;
 }
 
-// ------------------------------------------------------------------------------------------------ forward with tape
-// Same arithmetic as run_block (ard_api.cu) with every intermediate the backward needs written to its tape slot.
-int run_block_train(ard_handle* h, int l, int b, int B, float* attn_out, float attn_scale, int attn_acc, float* res_out,
-                    long long res_bstride, cudaStream_t s) {
-    BlockW& bw = h->layers[l].blocks[b];
-    const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
-    const long long M = (long long)B * T;
-    __nv_bfloat16* XN = h->ws_xn.as<__nv_bfloat16>();
-    __nv_bfloat16* Hb = h->ws_h.as<__nv_bfloat16>();
-    GemmArgs g;
-    if (C == 96 && h->use_ln_qkv) {
-        ARD_TRY(ln_qkv_96(bw.t_s, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), bw.qkv_w.as<__nv_bfloat16>(), bw.qkv_b.as<float>(), bw.t_qkv, M,
-                          h->num_sms, s));
-    } else {
-        ARD_TRY(layernorm_bf16(bw.t_s, bw.ln1_g.as<float>(), bw.ln1_b.as<float>(), XN, M, C, s));
-        g.A = XN; g.lda = C; g.W = bw.qkv_w.as<__nv_bfloat16>(); g.ldw = C; g.out = bw.t_qkv; g.ldo = 3 * C; g.out_bf16 = 1;
-        g.M = (int)M; g.N = 3 * C; g.K = C; g.bias = bw.qkv_b.as<float>();
-        ARD_TRY(gemm_bf16(g, h->num_sms, s));
-    }
-    AttnArgs a;
-    a.qkv = bw.t_qkv; a.out = bw.t_ao; a.bias_table = bw.rpb.as<float>(); a.attn_mean = attn_out; a.attn_scale = attn_scale;
-    a.attn_accumulate = attn_acc; a.B = B; a.H = R; a.W = R; a.C = C; a.nH = nH; a.shift = (b % 2 == 0) ? 0 : 4;
-    ARD_TRY(window_attention(a, s));
-    ARD_TRY(ensure_fold(h, l, b, s));
-    g = GemmArgs();
-    g.A = bw.t_ao; g.lda = C; g.ldw = C; g.out = bw.t_x1; g.ldo = C; g.M = (int)M; g.N = C; g.K = C;
-    if (bw.has_res) { g.W = bw.proj_w_fold.as<__nv_bfloat16>(); g.bias = bw.proj_b_fold.as<float>(); }
-    else { g.W = bw.proj_w.as<__nv_bfloat16>(); g.bias = bw.proj_b.as<float>(); }
-    g.resid1 = bw.t_s; g.ldr1 = C;
-    if (res_out) { g.aux = res_out; g.ld_aux = C; g.aux_T = T; g.aux_bstride = res_bstride; }
-    ARD_TRY(gemm_bf16(g, h->num_sms, s));
-    auto ffn = [&](const float* in, float* out, const float* r2) -> int {
-        if (C == 96 && h->use_fused_ffn)
-            return ffn_fused_96(in, r2, out, M, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), bw.fc1_w.as<__nv_bfloat16>(), bw.fc1_b.as<float>(),
-                                bw.fc2_w.as<__half>(), bw.fc2_b.as<float>(), h->num_sms, s);
-        if (((C == 192 && h->use_fused_ffn_wide >= 1) || ((C == 128 || C == 256) && h->use_fused_ffn_wide >= 3)) || (C == 384 && h->use_fused_ffn_wide >= 2))
-            return ffn_fused_wide(in, r2, out, M, C, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), bw.fc1_w.as<__nv_bfloat16>(),
-                                  bw.fc1_b_half.as<float>(), bw.fc2_w.as<__half>(), bw.fc2_b.as<float>(), h->num_sms, s);
-        ARD_TRY(layernorm_bf16(in, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), XN, M, C, s));
-        GemmArgs f;
-        f.A = XN; f.lda = C; f.W = bw.fc1_w.as<__nv_bfloat16>(); f.ldw = C; f.out = Hb; f.ldo = 4 * C; f.out_bf16 = 1;
-        f.M = (int)M; f.N = 4 * C; f.K = C; f.bias = bw.fc1_b.as<float>(); f.act = ARD_ACT_GELU; f.out_f16 = 1;
-        ARD_TRY(gemm_bf16(f, h->num_sms, s));
-        f = GemmArgs();
-        f.A = Hb; f.lda = 4 * C; f.W = bw.fc2_w.as<__nv_bfloat16>(); f.ldw = 4 * C; f.out = out; f.ldo = C; f.ab_f16 = 1;
-        f.M = (int)M; f.N = C; f.K = 4 * C; f.bias = bw.fc2_b.as<float>();
-        f.resid1 = in; f.ldr1 = C; f.resid2 = r2; f.ldr2 = C;
-        return gemm_bf16(f, h->num_sms, s);
-    };
-    if (!bw.has_res) return ffn(bw.t_x1, bw.t_out, nullptr);     // htsat.py:480
-    ARD_TRY(ffn(bw.t_x1, bw.t_x3, bw.t_s));                      // x3 = shortcut + (x1 + mlp(norm2(x1)))   src/residual.py:93,95
-    return ffn(bw.t_x3, bw.t_out, nullptr);                      // x4 = x3 + mlp(norm2(x3))                src/residual.py:96
-}
-
 // ------------------------------------------------------------------------------------------------ backward schedule
 struct BwdBufs {
     float *G, *T, *coef, *gcoef;
@@ -438,22 +386,22 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
     ARD_TRY(h->bw_small.ensure((size_t)B * (2 * J + NF) * 4 + 1024));
     BwdBufs w;
     BwdBufs32 w32;
-    Fp32Weights* fws = nullptr;
+    Fp32Weights& fws = h->fp32;
     if (fp32) {
-        ARD_TRY(fp32_weights(h, &fws, s));
-        ARD_TRY(ensure_backward_weights_fp32(h, *fws, s));
-        ARD_TRY(fws->qkvf.ensure(MC * 16));
-        ARD_TRY(fws->aof.ensure(MC * 4));
-        ARD_TRY(fws->s3.ensure(MC * 24));
+        ARD_TRY(ensure_fp32_weights(h, s));
+        ARD_TRY(ensure_backward_weights_fp32(h, fws, s));
+        ARD_TRY(fws.qkvf.ensure(MC * 16));
+        ARD_TRY(fws.aof.ensure(MC * 4));
+        ARD_TRY(fws.s3.ensure(MC * 24));
         ARD_TRY(h->bw_gs.ensure(MC * 4));
         ARD_TRY(h->bw_dh.ensure(MC * 16));
         ARD_TRY(h->bw_g3.ensure(MC * 6));
         ARD_TRY(h->bw_coef.ensure(MC * 4));
         ARD_TRY(h->bw_gcoef.ensure(MC * 4));
         w32.G = h->bw_g.as<float>(); w32.T = h->bw_t.as<float>(); w32.R = h->bw_gs.as<float>(); w32.DH = h->bw_dh.as<float>();
-        w32.HPRE = w32.GQKV = fws->qkvf.as<float>(); w32.GAO = fws->aof.as<float>();
+        w32.HPRE = w32.GQKV = fws.qkvf.as<float>(); w32.GAO = fws.aof.as<float>();
         w32.coef = h->bw_coef.as<float>(); w32.gcoef = h->bw_gcoef.as<float>();
-        w32.A3 = fws->s3.as<__nv_bfloat16>(); w32.G3 = h->bw_g3.as<__nv_bfloat16>();
+        w32.A3 = fws.s3.as<__nv_bfloat16>(); w32.G3 = h->bw_g3.as<__nv_bfloat16>();
     } else {
     ARD_TRY(h->bw_dh.ensure(MC * 4 * 2));
     ARD_TRY(h->bw_gb.ensure(MC * 2));
@@ -504,7 +452,7 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         const int C = C_of(h, l), R = R_of(l);
         for (int b = h->cfg.depths[l] - 1; b >= 0; --b) {
             const bool stop = (l == stop_l && b == stop_b);
-            if (fp32) ARD_TRY(block_backward_fp32(h, *fws, l, b, B, a->grad_lambda[l], stop, w32, s));
+            if (fp32) ARD_TRY(block_backward_fp32(h, fws, l, b, B, a->grad_lambda[l], stop, w32, s));
             else ARD_TRY(block_backward(h, l, b, B, a->grad_lambda[l], stop, w, s));
             if (stop) return 0;
         }
@@ -514,7 +462,7 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
             LayerW& lw = h->layers[l - 1];
             if (fp32) {
                 ARD_TRY(split3_act(w32.G, C, w32.G3, Mm, C, s));
-                ARD_TRY(gemm3(w32.G3, C, fws->mergeT3[l - 1], w32.T, 4 * Cp, Mm, 4 * Cp, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0,
+                ARD_TRY(gemm3(w32.G3, C, fws.mergeT3[l - 1], w32.T, 4 * Cp, Mm, 4 * Cp, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0,
                               h->num_sms, s));
                 ARD_TRY(merge_layernorm_bwd(lw.blocks.back().t_out, w32.T, lw.mg_g.as<float>(), w32.G, nullptr, B, Rp, Rp, Cp, s));
                 continue;

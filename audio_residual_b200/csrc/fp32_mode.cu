@@ -390,7 +390,8 @@ __global__ void tscam_im2col_split3_kernel(const float* __restrict__ normed, __n
 }
 
 // ------------------------------------------------------------------------------------------------ weights
-static int ensure_fp32_weights(ard_handle* h, Fp32Weights& w, cudaStream_t s) {
+int ensure_fp32_weights(ard_handle* h, cudaStream_t s) {
+    Fp32Weights& w = h->fp32;
     if (w.epoch == h->graph_epoch && !w.blocks.empty()) return 0;
     w.blocks.resize(h->nlayers);
     w.merge3.resize(h->nlayers);
@@ -429,19 +430,6 @@ static int ensure_fp32_weights(ard_handle* h, Fp32Weights& w, cudaStream_t s) {
     return 0;
 }
 
-static std::map<const ard_handle*, Fp32Weights>& fp32_cache() {
-    static std::map<const ard_handle*, Fp32Weights> m;
-    return m;
-}
-void fp32_release(const ard_handle* h) { fp32_cache().erase(h); }
-
-int fp32_weights(ard_handle* h, Fp32Weights** out, cudaStream_t s) {
-    Fp32Weights& w = fp32_cache()[h];
-    ARD_TRY(ensure_fp32_weights(h, w, s));
-    *out = &w;
-    return 0;
-}
-
 int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, int ldo, long long M, int N, const float* bias, int act,
           const float* r1, const float* r2, float* aux, int aux_T, long long aux_bstride, int num_sms, cudaStream_t s) {
     GemmArgs g;
@@ -475,11 +463,10 @@ static int run_block_fp32(ard_handle* h, Fp32Weights& w, int l, int b, int B, co
     ARD_TRY(split3_act(io.ao, C, S3, M, C, s));
     const DevBuf* pw = &fw.proj3;
     const float* pb = bw.proj_b.as<float>();
-    static thread_local DevBuf fold3;   // the folded projection depends on the current lambda: re-split per call (C^2 elements)
-    if (bw.has_res) {
+    if (bw.has_res) {   // the folded projection depends on the current lambda: re-split per call (C^2 elements)
         ARD_TRY(ensure_fold(h, l, b, s));
-        ARD_TRY(split3_weight_dev(bw.proj_w_fold_f32.as<float>(), fold3, C, C, s));
-        pw = &fold3;
+        ARD_TRY(split3_weight_dev(bw.proj_w_fold_f32.as<float>(), w.fold3, C, C, s));
+        pw = &w.fold3;
         pb = bw.proj_b_fold.as<float>();
     }
     // x1 = s + r,  aux = r = residual_x (post-ResiDual for patched blocks)
@@ -498,8 +485,8 @@ static int run_block_fp32(ard_handle* h, Fp32Weights& w, int l, int b, int B, co
 // Swin stages of the forward in the fp32-grade mode; X holds the patch-embed output (front end is fp32 already). With
 // a->save_for_backward, X is the tape's first slot and every block writes its tape slots (ensure_tape(h, B, 1) ran).
 int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, float* Y, float** x_final, cudaStream_t s) {
-    Fp32Weights& w = fp32_cache()[h];
-    ARD_TRY(ensure_fp32_weights(h, w, s));
+    ARD_TRY(ensure_fp32_weights(h, s));
+    Fp32Weights& w = h->fp32;
     const int B = a->B;
     const bool train = a->save_for_backward != 0;
     const size_t MC = (size_t)B * 4096 * h->cfg.embed_dim;
@@ -532,7 +519,7 @@ int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, floa
 
 // tscam_conv (htsat.py:813-816) as a split GEMM: y [B*32, ldy] fp32
 int tscam_gemm_fp32(ard_handle* h, const float* normed, float* y, int ldy, int B, cudaStream_t s) {
-    Fp32Weights& w = fp32_cache()[h];
+    Fp32Weights& w = h->fp32;
     const int NF = C_of(h, h->nlayers - 1);
     if (!w.tscam3.p) return set_error(ARD_ERR_STATE, "tscam_conv weights were never set");
     ARD_TRY(w.s3.ensure((size_t)B * 32 * 18 * NF * 2));

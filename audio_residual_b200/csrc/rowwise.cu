@@ -114,82 +114,6 @@ __global__ void __launch_bounds__(256) layernorm_rows_kernel(Rows rows, const fl
     }
 }
 
-// x3 = x + add (fp32, written to sum_out) followed by LayerNorm(x3) -> bf16: the "x = shortcut + drop_path(x)" step of the
-// ResiDual-patched block (src/residual.py:95) fused with the norm2 that follows it (src/residual.py:96).
-template <int VEC, int NV>
-__global__ void __launch_bounds__(256) add_layernorm_rows_kernel(const float* __restrict__ x, const float* __restrict__ add,
-                                                                float* __restrict__ sum_out, const float* __restrict__ gamma,
-                                                                const float* __restrict__ beta, __nv_bfloat16* __restrict__ out,
-                                                                long long nrows) {
-    pdl_launch_dependents();
-    pdl_wait();
-    constexpr int C = 32 * VEC * NV;
-    const int lane = threadIdx.x & 31;
-    const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (row >= nrows) return;
-    float v[NV][VEC];
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        const long long off = row * C + (i * 32 + lane) * VEC;
-        float a[VEC];
-        load_vec<VEC>(x + off, v[i]);
-        load_vec<VEC>(add + off, a);
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) v[i][k] += a[k];
-        if constexpr (VEC == 4) *reinterpret_cast<float4*>(sum_out + off) = make_float4(v[i][0], v[i][1], v[i][2], v[i][3]);
-        else if constexpr (VEC == 2) *reinterpret_cast<float2*>(sum_out + off) = make_float2(v[i][0], v[i][1]);
-        else sum_out[off] = v[i][0];
-    }
-    float s = 0.f;
-#pragma unroll
-    for (int i = 0; i < NV; ++i)
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) s += v[i][k];
-    const float mean = warp_sum(s) * (1.0f / C);
-    float q = 0.f;
-#pragma unroll
-    for (int i = 0; i < NV; ++i)
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) {
-            const float d = v[i][k] - mean;
-            q = fmaf(d, d, q);
-        }
-    const float rstd = rsqrtf(warp_sum(q) * (1.0f / C) + LN_EPS);
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        const int e = (i * 32 + lane) * VEC;
-        float g[VEC], b[VEC], o[VEC];
-        load_vec<VEC>(gamma + e, g);
-        load_vec<VEC>(beta + e, b);
-#pragma unroll
-        for (int k = 0; k < VEC; ++k) o[k] = fmaf((v[i][k] - mean) * rstd, g[k], b[k]);
-        store_bf16_vec<VEC>(out + row * C + e, o);
-    }
-}
-
-int add_layernorm_bf16(const float* x, const float* add, float* sum_out, const float* gamma, const float* beta, __nv_bfloat16* out,
-                       long long rows, int C, cudaStream_t s) {
-    if (rows <= 0) return 0;
-    const int wpb = 8;
-    const unsigned grid = (unsigned)((rows + wpb - 1) / wpb);
-    ProfScope ps(PROF_LN, s, 9.0 * rows * C, 14.0 * rows * C);
-#define ARD_ALN_CASE(c, vec, nv) \
-    case c: ARD_CUDA(enqueue_pdl(add_layernorm_rows_kernel<vec, nv>, dim3(grid), dim3(wpb * 32), 0, s, x, add, sum_out, gamma, beta, out, rows)); break;
-    switch (C) {
-        ARD_ALN_CASE(96, 1, 3)
-        ARD_ALN_CASE(128, 4, 1)
-        ARD_ALN_CASE(192, 2, 3)
-        ARD_ALN_CASE(256, 4, 2)
-        ARD_ALN_CASE(384, 4, 3)
-        ARD_ALN_CASE(512, 4, 4)
-        ARD_ALN_CASE(768, 4, 6)
-        ARD_ALN_CASE(1024, 4, 8)
-        default: return set_error(ARD_ERR_SHAPE, "add_layernorm: unsupported width C=%d", C);
-    }
-#undef ARD_ALN_CASE
-    return check_cuda(cudaGetLastError(), "add_layernorm launch");
-}
-
 template <class Rows, bool SPLIT3 = false>
 static int launch_ln(Rows rows, const float* gamma, const float* beta, __nv_bfloat16* out, long long nrows, int C, cudaStream_t s) {
     const int wpb = 8;

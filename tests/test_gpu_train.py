@@ -64,6 +64,27 @@ def test_zero_shot_step_subset_of_layers_vs_oracle():
     assert m["lambda_cos1"] > 0.999 and abs(m["lambda_norm_ratio1"] - 1) < 0.01 and m["lambda_grad1"] < 2e-2, m
 
 
+@pytest.mark.parametrize("model,env", [("tiny", {}), ("tiny", {"ARD_FUSED_FFN": "0", "ARD_FUSED_FFN_WIDE": "0"}), ("base", {})])
+def test_training_forward_equals_bf16_inference(model, env, monkeypatch):
+    """The bf16 training forward (tape slots instead of the workspace) computes exactly what bf16 inference does. Inference is
+    kept off the fused attention block, which training cannot take (it keeps qkv / ao on chip). The unfused-FFN tiny case and
+    HTSAT-base run the patched block's FFN pair on the LayerNorm + GEMM chain at every width."""
+    monkeypatch.setenv("ARD_ATTN_BLOCK", "0")
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)
+    clap, _, _ = G.make_encoder(model, residual=True)
+    enc = clap.model.audio_branch
+    wave = G.W.make_clips(2, seed=1234).cuda()
+    with torch.no_grad():
+        ref = enc.encode(waveform=wave, want_audio_embed=True)
+        got = enc.encode(waveform=wave, want_audio_embed=True, save_for_backward=True)
+        again = enc.encode(waveform=wave, want_audio_embed=True)
+    torch.cuda.synchronize()
+    for k in ("embedding", "audio_embed"):
+        assert torch.equal(got[k], ref[k]), (k, G.rel(got[k], ref[k]))
+        assert torch.equal(again[k], ref[k]), k
+
+
 def test_backward_requires_saved_forward():
     clap, sd, _ = G.make_encoder("tiny", residual=True)
     enc = clap.model.audio_branch
