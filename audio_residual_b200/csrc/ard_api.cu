@@ -247,7 +247,7 @@ static int finalize(ard_handle* h, cudaStream_t) {
     }
     // transposed copies the backward builds lazily from the host tensors (ard_train.cu) are stale now
     auto drop = [](DevBuf& b) { if (b.p) { cudaFree(b.p); b.p = nullptr; b.bytes = 0; ++alloc_epoch(); } };
-    drop(h->p0_wT); drop(h->p2_wT);
+    drop(h->p0_wT); drop(h->p2_wT); drop(h->tscam_wT);
     for (LayerW& lw : h->layers) drop(lw.mg_wT);
     h->tape_B = 0;   // activations of a forward run with the old weights must not be back-propagated through the new ones
     h->finalized = true;
@@ -386,6 +386,9 @@ static int encoder_forward(ard_handle* h, const ard_forward_args* a, cudaStream_
     if (train) {
         ARD_TRY(ensure_tape(h, B, a->precision));
         ++h->tape_gen;
+        // the tail backward reads this forward's tscam pre-activation (ws_tscam_y), which the next inference forward overwrites
+        h->tape_tail = (a->framewise_output ? TAPE_FRAMEWISE : 0) | (a->clipwise_output ? TAPE_CLIPWISE : 0) |
+                       (a->fine_grained_embedding ? TAPE_FINE : 0);
         X = h->layers[0].blocks[0].t_s;
     }
     // ---- front end
@@ -747,11 +750,29 @@ int ard_attention_block(ard_handle* h, int layer, int block, const float* x_in, 
     return rc;
 }
 
-int ard_encoder_backward(ard_handle* h, const ard_backward_args* args, void* stream) {
+int ard_encoder_backward_outputs(ard_handle* h, const ard_backward_args* args, const ard_output_grads* outs, void* stream) {
     if (!h || !args) return set_error(ARD_ERR_SHAPE, "null argument");
     if (!h->finalized) return set_error(ARD_ERR_STATE, "ard_finalize_weights has not been called");
     g_launches = 0;
-    const int rc = encoder_backward(h, args, (cudaStream_t)stream);
+    const int rc = encoder_backward(h, args, outs, (cudaStream_t)stream);
+    h->last_launches = g_launches;
+    return rc;
+}
+
+int ard_encoder_backward(ard_handle* h, const ard_backward_args* args, void* stream) {
+    return ard_encoder_backward_outputs(h, args, nullptr, stream);
+}
+
+int ard_tail_backward(ard_handle* h, const float* y, int ldy, const float* grad_framewise, const float* grad_clipwise, const float* grad_fine,
+                      const float* grad_embedding, int B, int precision, float* grad_normed, void* stream) {
+    if (!h || !grad_normed) return set_error(ARD_ERR_SHAPE, "null argument");
+    if (!h->finalized) return set_error(ARD_ERR_STATE, "ard_finalize_weights has not been called");
+    if (B <= 0 || (precision != 0 && precision != 1)) return set_error(ARD_ERR_SHAPE, "ard_tail_backward: B = %d, precision = %d", B, precision);
+    if ((grad_framewise || grad_clipwise) && (!y || ldy < ARD_CLASS_NUM))
+        return set_error(ARD_ERR_SHAPE, "ard_tail_backward: the framewise / clipwise terms need y [B*32, ldy >= 527]");
+    g_launches = 0;
+    const int rc = tail_backward(h, y, ldy, grad_framewise, grad_clipwise, grad_fine, grad_embedding, B, precision == 1, grad_normed,
+                                 (cudaStream_t)stream);
     h->last_launches = g_launches;
     return rc;
 }
@@ -762,7 +783,8 @@ long long ard_workspace_bytes(const ard_handle* h) {
     if (!h) return 0;
     const DevBuf* bufs[] = {&h->ws_logmel, &h->ws_x, &h->ws_y, &h->ws_xn, &h->ws_ao, &h->ws_qkv, &h->ws_h, &h->ws_normed,
                             &h->ws_hid, &h->ws_proj, &h->ws_tscam_a, &h->ws_tscam_y, &h->tape, &h->bw_g, &h->bw_gs, &h->bw_t,
-                            &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small, &h->bw_g3};
+                            &h->bw_dh, &h->bw_gb, &h->bw_coef, &h->bw_gcoef, &h->bw_gsc, &h->bw_small, &h->bw_g3,
+                            &h->bw_tail_dy, &h->bw_tail_da};
     long long t = 0;
     for (const DevBuf* b : bufs) t += (long long)b->bytes;
     return t;
@@ -862,6 +884,21 @@ int ard_window_attention_f32_bwd(const float* qkv_f32, const float* dout_f32, fl
     if (!qkv_f32 || !dout_f32 || !dqkv_f32 || !bias_table) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd: null argument");
     if (H != W) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd: square token grids only (H=%d W=%d)", H, W);
     return window_attention_f32_bwd(qkv_f32, dout_f32, dqkv_f32, bias_table, B, H, C, nH, shift, (cudaStream_t)stream);
+}
+
+int ard_window_attention_bwd_pgrad(const void* qkv_bf16, const void* dout_bf16, const float* pgrad, float pscale, void* dqkv_bf16,
+                                   const float* bias_table, int B, int H, int W, int C, int nH, int shift, void* stream) {
+    if (!pgrad) return set_error(ARD_ERR_SHAPE, "ard_window_attention_bwd_pgrad: null probability gradient");
+    AttnArgs a;
+    a.qkv = (const __nv_bfloat16*)qkv_bf16; a.bias_table = bias_table; a.B = B; a.H = H; a.W = W; a.C = C; a.nH = nH; a.shift = shift;
+    return window_attention_bwd(a, (const __nv_bfloat16*)dout_bf16, (__nv_bfloat16*)dqkv_bf16, (cudaStream_t)stream, pgrad, pscale);
+}
+
+int ard_window_attention_f32_bwd_pgrad(const float* qkv_f32, const float* dout_f32, const float* pgrad, float pscale, float* dqkv_f32,
+                                       const float* bias_table, int B, int H, int W, int C, int nH, int shift, void* stream) {
+    if (!qkv_f32 || !dout_f32 || !pgrad || !dqkv_f32 || !bias_table) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd_pgrad: null argument");
+    if (H != W) return set_error(ARD_ERR_SHAPE, "ard_window_attention_f32_bwd_pgrad: square token grids only (H=%d W=%d)", H, W);
+    return window_attention_f32_bwd(qkv_f32, dout_f32, dqkv_f32, bias_table, B, H, C, nH, shift, (cudaStream_t)stream, pgrad, pscale);
 }
 
 int ard_layernorm_bwd(const float* x, const float* grad_out, const float* gamma, const float* add, float* grad_in, long long rows, int C,

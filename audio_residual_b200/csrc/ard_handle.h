@@ -73,9 +73,10 @@ struct Fp32BlockW {
 struct Fp32Weights {
     unsigned long long epoch = ~0ULL;            // ard_handle::graph_epoch the split weights were built at (weights / ResiDual changes bump it)
     unsigned long long bwd_epoch = ~0ULL;        // the same for the backward set (built by the first fp32-grade backward after a change)
+    unsigned long long tscam_epoch = ~0ULL;      // the same for tscamT3 (built by the first fp32-grade tail backward after a change)
     std::vector<std::vector<Fp32BlockW>> blocks;
     std::vector<DevBuf> merge3, mergeT3;         // PatchMerging reduction [2C, 3*4C] and its transpose [4C, 3*2C] (backward, lazily)
-    DevBuf tscam3, scratch;
+    DevBuf tscam3, tscamT3, scratch;                   // tscam_conv [527, 3*6C] and, for the tail backward, its transpose [6C, 3*528]
     DevBuf fold3;                                // folded projection of the block being run: depends on the current lambda, re-split per call
     DevBuf qkvf, aof, s3;                        // workspace: fp32 [M,4C] (qkv / FFN hidden), fp32 [M,C], split operands [M,12C] bf16
 };
@@ -111,10 +112,13 @@ struct ard_handle {
     DevBuf tape, p0_wT, p2_wT;
     DevBuf bw_g, bw_gs, bw_t, bw_dh, bw_gb, bw_coef, bw_gcoef, bw_gsc, bw_small;
     DevBuf bw_g3;            // fp32-grade backward: split form [hi | hi | lo] of the gradient entering a dgrad GEMM
+    DevBuf tscam_wT;         // tail backward: tscam_conv weight transposed, K = 527 zero-padded to 528 [6C, 528] bf16 (built lazily)
+    DevBuf bw_tail_dy, bw_tail_da;   // tail backward: dL/dy [B*32, 528] (bf16, or split [B*32, 3*528]) and dL/d im2col [B*32, 6C] fp32
     Fp32Weights fp32;        // fp32-grade split weights and workspace (ensure_fp32_weights)
     int tape_B = 0;          // batch of the forward whose activations the tape holds (0: none)
     int tape_prec = 0;       // ard_forward_args.precision of that forward: the layout of the tape and the backward schedule
     long long tape_gen = 0;  // serial number of that forward (ard_tape_generation): a backward built on an older one is refused
+    int tape_tail = 0;       // tail outputs that forward computed (TAPE_* bits): a gradient for one it did not compute is refused
     // CUDA-graph replay of the inference forward (ard_api.cu): the ~110 launches of a forward cost ~1.1 ms of fixed launch /
     // ramp latency whatever the batch; replaying a captured graph removes the host side of that and most of the device side.
     struct GraphEntry {
@@ -148,6 +152,8 @@ struct ard_handle {
 
 
 namespace ard {
+enum { TAPE_FRAMEWISE = 1, TAPE_CLIPWISE = 2, TAPE_FINE = 4 };
+constexpr int TSCAM_KP = 528;   // the 527 classes padded to the GEMM's K granularity
 inline int C_of(const ard_handle* h, int l) { return h->cfg.embed_dim << l; }
 inline int R_of(int l) { return 64 >> l; }   // tokens per side
 int upload(DevBuf& b, const void* src, size_t bytes);
@@ -159,7 +165,9 @@ int ensure_workspace(ard_handle* h, int B);
 int ensure_fold(ard_handle* h, int l, int b, cudaStream_t s);
 // training (ard_train.cu)
 int ensure_tape(ard_handle* h, int B, int precision);
-int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s);
+int encoder_backward(ard_handle* h, const ard_backward_args* a, const ard_output_grads* o, cudaStream_t s);
+int tail_backward(ard_handle* h, const float* y, int ldy, const float* g_frame, const float* g_clip, const float* g_fine, const float* g_emb, int B,
+                  bool fp32, float* out, cudaStream_t s);
 // window-resident attention block (attn_block.cu)
 int attn_block_pack(AttnBlockW& w, const std::vector<float>& qkv_w, const std::vector<float>& qkv_b, const std::vector<float>& rpb, int C, int nH);
 int attn_block_pad_proj(const __nv_bfloat16* w, const float* bp, const float* bv, __nv_bfloat16* out, float* bp_eff, int C, int nH, cudaStream_t s);
@@ -167,14 +175,14 @@ int attn_block_96(const float* x, float* out, const AttnBlockW& w, const __nv_bf
                   const float* beta, int B, int R, int shift, int num_sms, cudaStream_t stream);
 // fp32-grade mode (fp32_mode.cu)
 int ensure_fp32_weights(ard_handle* h, cudaStream_t s);   // h->fp32: forward split weights current
-int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s);
+int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s, RowAddend ext = RowAddend());
 int split3_weight_host(const std::vector<float>& w, DevBuf& scratch, DevBuf& out, long long N, int K, cudaStream_t s, float scale = 1.0f,
                        long long scaled_rows = 0);
 int gemm3(const __nv_bfloat16* A3, int K, const DevBuf& W3, float* out, int ldo, long long M, int N, const float* bias, int act,
           const float* r1, const float* r2, float* aux, int aux_T, long long aux_bstride, int num_sms, cudaStream_t s);
 int gelu_bwd_split3(const float* g, const float* hpre, __nv_bfloat16* out3, long long rows, int N, cudaStream_t s);
 int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, const float* bias_table, int B, int R, int C, int nH, int shift,
-                             cudaStream_t s);
+                             cudaStream_t s, const float* pgrad = nullptr, float pscale = 1.0f);   // pgrad: ProbGrad (ard_internal.h)
 int encoder_stages_fp32(ard_handle* h, const ard_forward_args* a, float* X, float* Y, float** x_final, cudaStream_t s);
 int tscam_gemm_fp32(ard_handle* h, const float* normed, float* y, int ldy, int B, cudaStream_t s);
 }  // namespace ard

@@ -106,9 +106,16 @@ int final_norm_mean(const float* x, const float* gamma, const float* beta, float
 int f32_to_bf16(const float* in, __nv_bfloat16* out, long long n, float scale, cudaStream_t s);
 int fill_f32(float* p, long long n, float v, cudaStream_t s);
 // backward kernels (training path)
-// out = add_scale*add + dLN(x)^T g (fp32); optional out_bf = bf16(add + dLN(x)^T g)
+// An fp32 addend to rows [B*T, C] stored per clip `bstride` floats apart (one block's rows b*T.. of a layers_residuals gradient
+// [B, depth*T, C]: p = grad + b*T*C, bstride = depth*T*C). p == nullptr: none.
+struct RowAddend {
+    const float* p = nullptr;
+    int T = 1;
+    long long bstride = 0;
+};
+// out = add_scale*add + dLN(x)^T g (fp32); optional out_bf = bf16(add + dLN(x)^T g (+ ext))
 int layernorm_bwd(const float* x, const float* g, const float* gamma, const float* add, float* out, long long rows, int C, cudaStream_t s,
-                  float add_scale = 1.0f, __nv_bfloat16* out_bf = nullptr);
+                  float add_scale = 1.0f, __nv_bfloat16* out_bf = nullptr, RowAddend ext = RowAddend());
 
 // ---------------------------------------------------------------- window attention (attn_window.cu)
 struct AttnArgs {
@@ -121,7 +128,17 @@ struct AttnArgs {
     int B = 0, H = 0, W = 0, C = 0, nH = 0, shift = 0;
 };
 int window_attention(const AttnArgs& a, cudaStream_t s);
-int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, cudaStream_t s);
+// A gradient w.r.t. the attention probabilities (a loss on layers_attention, the block mean of BasicLayer.forward
+// htsat.py:589-595): dP += scale * p[window, head, query, key] ([B*nW, nH, 64, 64] fp32, window order of the block). Empty when
+// the kernel is instantiated without it, so those instantiations compile to the kernels without the injection.
+template <bool ON> struct ProbGrad {
+    const float* p;
+    float scale;
+};
+template <> struct ProbGrad<false> {};
+// pgrad (or nullptr): the probability gradient above, weighted by pscale
+int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, cudaStream_t s, const float* pgrad = nullptr,
+                         float pscale = 1.0f);
 
 // ---------------------------------------------------------------- front end (frontend.cu)
 struct MelBands {            // banded view of logmel_extractor.melW [513,64]
@@ -149,6 +166,10 @@ int residual_matrix(const float* basis, const float* lam, int C, int K, float* M
 int tscam_im2col(const float* normed, __nv_bfloat16* A, int B, int C, cudaStream_t s);
 int tscam_finish(const float* y, int ldy, float* framewise, float* clipwise, int B, int NC, cudaStream_t s);
 int fine_grained(const float* normed, float* fine, int B, int C, cudaStream_t s);
+// tail backward (training path): dY of the tscam conv from the pre-sigmoid y, and the token gradient in front of the final norm
+int tscam_bwd_dy(const float* y, int ldy, const float* g_frame, const float* g_clip, __nv_bfloat16* dY, int Kp, int B, bool split3,
+                 cudaStream_t s);
+int tail_token_grad(const float* g_emb, const float* dA, const float* g_fine, float* out, int B, int C, cudaStream_t s);
 // dlam[k] += sum_t coef[t,k] gcoef[t,k] (k < K; dlam may be NULL), gsc[t,k] = bf16(gcoef[t,k] lam[k]) (k < Kp); rows are Kp wide.
 // split3: gsc rows are 3 Kp wide, [hi | hi | lo] of gcoef * lam (fp32-grade backward)
 int lambda_grad(const float* coef, const float* gcoef, const float* lam, float* dlam, __nv_bfloat16* gsc, long long M, int K, int Kp,

@@ -1,5 +1,6 @@
 // Training path of libard_b200.so: the layout of what the forward keeps for the backward, and the backward schedule that
-// produces the gradient of a loss on audio_embed / embedding w.r.t. every ResiDual `learnable` vector (lambda). The training
+// produces the gradient of a loss on audio_embed / embedding / the tail keys (framewise, clipwise, fine-grained) / layers_residuals
+// w.r.t. every ResiDual `learnable` vector (lambda). The training
 // forward is the inference block schedule itself (run_block in ard_api.cu, run_block_fp32 in fp32_mode.cu) pointed at the
 // block's tape slots instead of the workspace, so it computes bit for bit what inference computes.
 //
@@ -33,8 +34,6 @@ int merge_layernorm_bwd(const float* x, const float* g, const float* gamma, floa
 int gelu_bwd_mul(__nv_bfloat16* dh, const __nv_bfloat16* hpre, long long n, cudaStream_t s);
 int bcast_rows(const float* g, float* out, int B, int T, int C, float scale, cudaStream_t s);
 int add_f32(const float* a, const float* b, float* y, __nv_bfloat16* ybf, long long n, cudaStream_t s);
-// attn_window.cu
-int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, cudaStream_t s);
 
 static size_t align256(size_t n) { return (n + 255) & ~(size_t)255; }
 
@@ -217,8 +216,9 @@ struct BwdBufs {
 
 // gout = out_scale * gin + d/dx [ mlp(norm2(x)) ]^T gin   (one FFN residual branch; gout may alias gin).
 // w.GB must hold bf16(gin) on entry; on exit it holds bf16(gin + branch gradient), the bf16 copy of the un-scaled result.
+// ext: a layers_residuals gradient added to that bf16 copy only (the operand of the next dgrad, not the shortcut gradient gout).
 static int ffn_backward(ard_handle* h, BlockW& bw, int C, long long M, const float* x, const float* gin, float* gout, float out_scale,
-                        const BwdBufs& w, cudaStream_t s) {
+                        const BwdBufs& w, cudaStream_t s, RowAddend ext = RowAddend()) {
     ARD_TRY(layernorm_bf16(x, bw.ln2_g.as<float>(), bw.ln2_b.as<float>(), w.XN, M, C, s));
     GemmArgs f;
     if (h->use_dual_gemm && C <= 192) {
@@ -243,12 +243,15 @@ static int ffn_backward(ard_handle* h, BlockW& bw, int C, long long M, const flo
     f.A = w.DH; f.lda = 4 * C; f.W = bw.fc1_wT.as<__nv_bfloat16>(); f.ldw = 4 * C; f.out = w.T; f.ldo = C;
     f.M = (int)M; f.N = C; f.K = 4 * C;
     ARD_TRY(gemm_bf16(f, h->num_sms, s));                                       // dn2 = dh W1
-    return layernorm_bwd(x, w.T, bw.ln2_g.as<float>(), gin, gout, M, C, s, out_scale, w.GB);   // + LN2'(dn2), and its bf16 copy
+    return layernorm_bwd(x, w.T, bw.ln2_g.as<float>(), gin, gout, M, C, s, out_scale, w.GB, ext);   // + LN2'(dn2), and its bf16 copy
 }
 
 // G holds dL/d(block output) on entry and dL/d(block input) on exit. `stop_after_lambda`: nothing below this block needs
-// a gradient, so the attention / norm1 backward of this block is skipped.
-static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool stop_after_lambda, const BwdBufs& w, cudaStream_t s) {
+// a gradient, so the attention / norm1 backward of this block is skipped. `ext`: dL/d residual_x from a loss on layers_residuals
+// (src/residual.py:88-92, htsat.py:476-479): it adds to dL/dr only, never to the shortcut gradient dL/ds. `pgrad`: dL/d layers_attention
+// (or nullptr), whose mean over the layer's blocks (htsat.py:589-595) gives each block's probabilities pgrad / depth.
+static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool stop_after_lambda, const BwdBufs& w, cudaStream_t s,
+                          RowAddend ext, const float* pgrad) {
     BlockW& bw = h->layers[l].blocks[b];
     const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
     const long long M = (long long)B * T;
@@ -258,7 +261,7 @@ static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool 
         ARD_TRY(ffn_backward(h, bw, C, M, bw.t_x3, w.G, w.G, 1.0f, w, s));       // G  = dL/dx3, GB = bf16(G)
         // dL/dx1 = dL/dr = G + FFN'(G)   (x3 = s + x2, x2 = x1 + mlp): only its bf16 copy (GB) is needed below, and the
         // shortcut sum dL/ds so far = dL/dx3 + dL/dx1 = 2 G + FFN'(G) is written straight into G
-        ARD_TRY(ffn_backward(h, bw, C, M, bw.t_x1, w.G, w.G, 2.0f, w, s));
+        ARD_TRY(ffn_backward(h, bw, C, M, bw.t_x1, w.G, w.G, 2.0f, w, s, ext));   // GB = bf16(dL/dr + ext)
         const int Kp = bw.Kp;
         const float* lam = bw.lambda_set && bw.lam.p ? bw.lam.as<float>() : bw.lam_ones.as<float>();
         if (h->use_dual_gemm) {
@@ -286,7 +289,7 @@ static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool 
         g.M = (int)M; g.N = C; g.K = Kp;
         ARD_TRY(gemm_bf16(g, h->num_sms, s));                                    // d ao = gsc Wc
     } else {
-        ARD_TRY(ffn_backward(h, bw, C, M, bw.t_x1, w.G, w.G, 1.0f, w, s));       // G = dL/dx1 = dL/ds (shortcut) = dL/dr, GB = bf16(G)
+        ARD_TRY(ffn_backward(h, bw, C, M, bw.t_x1, w.G, w.G, 1.0f, w, s, ext));  // G = dL/dx1 = dL/ds (shortcut), GB = bf16(dL/dr = G + ext)
         if (stop_after_lambda) return 0;
         g.A = w.GB; g.lda = C; g.W = bw.proj_wT.as<__nv_bfloat16>(); g.ldw = C; g.out = w.GAO; g.ldo = C; g.out_bf16 = 1;
         g.M = (int)M; g.N = C; g.K = C;
@@ -294,7 +297,7 @@ static int block_backward(ard_handle* h, int l, int b, int B, float* dlam, bool 
     }
     AttnArgs a;
     a.qkv = bw.t_qkv; a.bias_table = bw.rpb.as<float>(); a.B = B; a.H = R; a.W = R; a.C = C; a.nH = nH; a.shift = (b % 2 == 0) ? 0 : 4;
-    ARD_TRY(window_attention_bwd(a, w.GAO, w.GQKV, s));
+    ARD_TRY(window_attention_bwd(a, w.GAO, w.GQKV, s, pgrad, 1.0f / h->cfg.depths[l]));
     g = GemmArgs();
     g.A = w.GQKV; g.lda = 3 * C; g.W = bw.qkv_wT.as<__nv_bfloat16>(); g.ldw = 3 * C; g.out = w.T; g.ldo = C;
     g.M = (int)M; g.N = C; g.K = 3 * C;
@@ -324,7 +327,7 @@ static int ffn_backward_fp32(ard_handle* h, BlockW& bw, Fp32BlockW& fw, int C, l
 }
 
 static int block_backward_fp32(ard_handle* h, Fp32Weights& fws, int l, int b, int B, float* dlam, bool stop_after_lambda, const BwdBufs32& w,
-                               cudaStream_t s) {
+                               cudaStream_t s, RowAddend ext, const float* pgrad) {
     BlockW& bw = h->layers[l].blocks[b];
     Fp32BlockW& fw = fws.blocks[l][b];
     const int C = C_of(h, l), R = R_of(l), T = R * R, nH = h->cfg.num_heads[l];
@@ -337,7 +340,7 @@ static int block_backward_fp32(ard_handle* h, Fp32Weights& fws, int l, int b, in
         const float* lam = bw.lambda_set && bw.lam.p ? bw.lam.as<float>() : bw.lam_ones.as<float>();
         ARD_TRY(split3_act(bw.t_aof, C, w.A3, M, C, s));
         ARD_TRY(gemm3(w.A3, C, fw.wc3, w.coef, Kp, M, Kp, bw.res_c0.as<float>(), ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));   // coef = x_proj
-        ARD_TRY(split3_act(w.R, C, w.G3, M, C, s));
+        ARD_TRY(split3_act(w.R, C, w.G3, M, C, s, ext));                                // split(dL/dr + ext)
         ARD_TRY(gemm3(w.G3, C, fw.basis3, w.gcoef, Kp, M, Kp, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));   // gcoef = dL/dr B^T
         ARD_TRY(lambda_grad(w.coef, w.gcoef, lam, dlam, w.A3, M, bw.K, Kp, s, true));   // dlam += colsum(coef*gcoef); A3 = split(gcoef*lam)
         if (stop_after_lambda) return 0;
@@ -345,23 +348,82 @@ static int block_backward_fp32(ard_handle* h, Fp32Weights& fws, int l, int b, in
     } else {
         ARD_TRY(ffn_backward_fp32(h, bw, fw, C, M, bw.t_x1, w.G, w.G, 1.0f, w, s));     // G = dL/dx1 = dL/ds (shortcut) = dL/dr
         if (stop_after_lambda) return 0;
-        ARD_TRY(split3_act(w.G, C, w.G3, M, C, s));
+        ARD_TRY(split3_act(w.G, C, w.G3, M, C, s, ext));                                // split(dL/dr = G + ext)
         ARD_TRY(gemm3(w.G3, C, fw.projT3, w.GAO, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));       // d ao = dL/dr Wp
     }
-    ARD_TRY(window_attention_f32_bwd(bw.t_qkvf, w.GAO, w.GQKV, bw.rpb.as<float>(), B, R, C, nH, (b % 2 == 0) ? 0 : 4, s));
+    ARD_TRY(window_attention_f32_bwd(bw.t_qkvf, w.GAO, w.GQKV, bw.rpb.as<float>(), B, R, C, nH, (b % 2 == 0) ? 0 : 4, s, pgrad,
+                                     1.0f / h->cfg.depths[l]));
     ARD_TRY(split3_act(w.GQKV, 3 * C, w.A3, M, 3 * C, s));
     ARD_TRY(gemm3(w.A3, 3 * C, fw.qkvT3, w.T, C, M, C, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0, h->num_sms, s));          // dn1 = dqkv Wqkv
     return layernorm_bwd(bw.t_s, w.T, bw.ln1_g.as<float>(), w.G, w.G, M, C, s, 1.0f, nullptr);           // G += LN1'(dn1)
 }
 
-int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) {
+// ------------------------------------------------------------------------------------------------ tail backward
+// Backward of htsat.py:798-821 (restated at heads.cu tscam_im2col_kernel): the per-token gradient in front of the final LayerNorm,
+// out [B, 64, NF] = dL/d normed, from the framewise / clipwise terms (through sigma' of the saved pre-sigmoid y and the tscam conv
+// dgrad dA = dY W), the fine-grained term and the token mean of g_emb. Everything but the dgrad is fp32; the dgrad is a bf16
+// tcgen05 GEMM, or at fp32 grade (fp32) a split gemm3 against [W_hi^T | W_lo^T | W_hi^T].
+int tail_backward(ard_handle* h, const float* y, int ldy, const float* g_frame, const float* g_clip, const float* g_fine, const float* g_emb, int B,
+                  bool fp32, float* out, cudaStream_t s) {
+    const int NF = C_of(h, h->nlayers - 1);
+    float* dA = nullptr;
+    if (g_frame || g_clip) {
+        if (!h->host.count("tscam_conv.weight")) return set_error(ARD_ERR_STATE, "tscam_conv weights were never set");
+        const long long rows = (long long)B * 32;
+        ARD_TRY(h->bw_tail_da.ensure((size_t)rows * 6 * NF * 4));
+        ARD_TRY(h->bw_tail_dy.ensure((size_t)rows * TSCAM_KP * 2 * (fp32 ? 3 : 1)));
+        dA = h->bw_tail_da.as<float>();
+        __nv_bfloat16* dY = h->bw_tail_dy.as<__nv_bfloat16>();
+        ARD_TRY(tscam_bwd_dy(y, ldy, g_frame, g_clip, dY, TSCAM_KP, B, fp32, s));
+        if (fp32) {
+            Fp32Weights& fw = h->fp32;
+            ARD_TRY(ensure_fp32_weights(h, s));
+            if (fw.tscam_epoch != fw.epoch) {   // tscam_conv.weight.view(527, 6C) transposed, K = 527 padded to 528, split: built lazily
+                const std::vector<float>* v = nullptr;
+                ARD_TRY(get(h, "tscam_conv.weight", (size_t)ARD_CLASS_NUM * NF * 6, &v));
+                std::vector<float> wp((size_t)TSCAM_KP * 6 * NF, 0.f);
+                memcpy(wp.data(), v->data(), (size_t)ARD_CLASS_NUM * 6 * NF * 4);
+                ARD_TRY(transpose_split_upload(fw.tscamT3, fw.scratch, wp.data(), TSCAM_KP, 6 * NF, s));   // [6C, 3*528]
+                fw.tscam_epoch = fw.epoch;
+            }
+            ARD_TRY(gemm3(dY, TSCAM_KP, h->fp32.tscamT3, dA, 6 * NF, rows, 6 * NF, nullptr, ARD_ACT_NONE, nullptr, nullptr, nullptr, 0, 0,
+                          h->num_sms, s));
+        } else {
+            if (!h->tscam_wT.p) {
+                const std::vector<float>* v = nullptr;
+                ARD_TRY(get(h, "tscam_conv.weight", (size_t)ARD_CLASS_NUM * NF * 6, &v));
+                std::vector<float> wp((size_t)TSCAM_KP * 6 * NF, 0.f);
+                memcpy(wp.data(), v->data(), (size_t)ARD_CLASS_NUM * 6 * NF * 4);
+                ARD_TRY(transpose_upload_bf16(h->tscam_wT, wp.data(), TSCAM_KP, 6 * NF));   // [6NF, 528]
+            }
+            GemmArgs g;
+            g.A = dY; g.lda = TSCAM_KP; g.W = h->tscam_wT.as<__nv_bfloat16>(); g.ldw = TSCAM_KP; g.out = dA; g.ldo = 6LL * NF;
+            g.M = (int)rows; g.N = 6 * NF; g.K = TSCAM_KP;
+            ARD_TRY(gemm_bf16(g, h->num_sms, s));                                      // dA = dY W
+        }
+    }
+    return tail_token_grad(g_emb, dA, g_fine, out, B, NF, s);
+}
+
+int encoder_backward(ard_handle* h, const ard_backward_args* a, const ard_output_grads* o, cudaStream_t s) {
     const int B = a->B;
     if (h->tape_B <= 0 || h->tape_B != B)
         return set_error(ARD_ERR_STATE, "ard_encoder_backward: no saved forward for batch %d (run ard_encoder_forward with save_for_backward=1)", B);
     if (a->generation != 0 && a->generation != h->tape_gen)
         return set_error(ARD_ERR_STATE, "ard_encoder_backward: the saved activations belong to training forward #%lld, this backward to #%lld "
                                         "(the handle keeps one tape: run forward and backward of a step back to back)", h->tape_gen, a->generation);
-    if (!a->grad_audio_embed && !a->grad_embedding) return set_error(ARD_ERR_SHAPE, "ard_encoder_backward: no output gradient given");
+    const ard_output_grads none = {};
+    if (!o) o = &none;
+    const int tail = (o->grad_framewise_output ? TAPE_FRAMEWISE : 0) | (o->grad_clipwise_output ? TAPE_CLIPWISE : 0) |
+                     (o->grad_fine_grained_embedding ? TAPE_FINE : 0);
+    bool any_cap = false;   // a gradient of a per-layer capture (layers_residuals / layers_attention)
+    for (int l = 0; l < h->nlayers; ++l) any_cap = any_cap || o->grad_layers_residuals[l] || o->grad_layers_attention[l];
+    const bool head = a->grad_audio_embed || a->grad_embedding || tail;
+    if (!head && !any_cap) return set_error(ARD_ERR_SHAPE, "ard_encoder_backward: no output gradient given");
+    if (tail & ~h->tape_tail)
+        return set_error(ARD_ERR_STATE, "ard_encoder_backward_outputs: a gradient for %s, which the saved forward did not compute (request it "
+                                        "in the save_for_backward forward)", (tail & ~h->tape_tail & TAPE_FRAMEWISE) ? "framewise_output" :
+                                        (tail & ~h->tape_tail & TAPE_CLIPWISE) ? "clipwise_output" : "fine_grained_embedding");
     const int NF = C_of(h, h->nlayers - 1), J = h->cfg.joint_dim;
     // lowest patched block: nothing below it needs a gradient
     int stop_l = -1, stop_b = -1;
@@ -378,7 +440,11 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         if (K && !a->grad_lambda[l]) return set_error(ARD_ERR_SHAPE, "grad_lambda[%d] is required (layer has ResiDual)", l);
         if (K) ARD_TRY(fill_f32(a->grad_lambda[l], K, 0.f, s));
     }
-    if (stop_l < 0) return 0;
+    // the walk starts at the top of the highest layer a given gradient reaches, with G = 0 above it
+    int top_l = h->nlayers - 1;
+    if (!head)
+        while (!o->grad_layers_residuals[top_l] && !o->grad_layers_attention[top_l]) --top_l;
+    if (stop_l < 0 || top_l < stop_l) return 0;
     const bool fp32 = h->tape_prec == 1;
     const size_t MC = (size_t)B * 4096 * h->cfg.embed_dim;
     ARD_TRY(h->bw_g.ensure(MC * 4));
@@ -416,6 +482,7 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
     w.XN = h->ws_xn.as<__nv_bfloat16>(); w.HPRE = h->ws_h.as<__nv_bfloat16>(); w.DH = h->bw_dh.as<__nv_bfloat16>();
     w.GB = fp32 ? nullptr : h->bw_gb.as<__nv_bfloat16>(); w.GQKV = h->ws_qkv.as<__nv_bfloat16>(); w.GAO = h->ws_ao.as<__nv_bfloat16>();
 
+    if (head) {
     // ---- head: audio_embed = normalize(W2 relu(W0 emb + b0) + b2)   (model.py:539-543, :739-741)
     float* g_p = h->bw_small.as<float>();
     float* g_h = g_p + (size_t)B * J;
@@ -440,20 +507,32 @@ int encoder_backward(ard_handle* h, const ard_backward_args* a, cudaStream_t s) 
         ARD_TRY(relu_bwd_mul(g_h, h->ws_hid.as<float>(), (long long)B * J, s));
         ARD_TRY(linear_small(g_h, J, h->p0_wT.as<float>(), nullptr, g_emb, NF, B, NF, J, ARD_ACT_NONE, s));
         if (a->grad_embedding) ARD_TRY(add_f32(g_emb, a->grad_embedding, g_emb, nullptr, (long long)B * NF, s));
-    } else {
+    } else if (!tail) {
         ARD_CUDA(cudaMemcpyAsync(g_emb, a->grad_embedding, (size_t)B * NF * 4, cudaMemcpyDeviceToDevice, s));
     }
-    // ---- token mean + final norm (htsat.py:797, :810-811)
+    // ---- token mean (+ the tail: tscam head and fine-grained embedding, htsat.py:798-821) + final norm (htsat.py:797, :810-811)
     const LayerW& last = h->layers[h->nlayers - 1];
-    ARD_TRY(bcast_rows(g_emb, w.T, B, 64, NF, 1.0f / 64.0f, s));
+    if (tail)
+        ARD_TRY(tail_backward(h, h->ws_tscam_y.as<float>(), TSCAM_KP, o->grad_framewise_output, o->grad_clipwise_output,
+                              o->grad_fine_grained_embedding, a->grad_audio_embed ? g_emb : a->grad_embedding, B, fp32, w.T, s));
+    else
+        ARD_TRY(bcast_rows(g_emb, w.T, B, 64, NF, 1.0f / 64.0f, s));
     ARD_TRY(layernorm_bwd(last.blocks.back().t_out, w.T, h->norm_g.as<float>(), nullptr, w.G, (long long)B * 64, NF, s, 1.0f, w.GB));
+    } else {   // only capture gradients: G = 0 (and its bf16 copy) above the highest of them
+        const long long Mt = (long long)B * R_of(top_l) * R_of(top_l) * C_of(h, top_l);
+        ARD_TRY(fill_f32(h->bw_g.as<float>(), Mt, 0.f, s));
+        if (!fp32) ARD_CUDA(cudaMemsetAsync(w.GB, 0, (size_t)Mt * 2, s));
+    }
     // ---- swin stages, top down
-    for (int l = h->nlayers - 1; l >= stop_l; --l) {
-        const int C = C_of(h, l), R = R_of(l);
-        for (int b = h->cfg.depths[l] - 1; b >= 0; --b) {
+    for (int l = top_l; l >= stop_l; --l) {
+        const int C = C_of(h, l), R = R_of(l), T = R * R, depth = h->cfg.depths[l];
+        for (int b = depth - 1; b >= 0; --b) {
             const bool stop = (l == stop_l && b == stop_b);
-            if (fp32) ARD_TRY(block_backward_fp32(h, fws, l, b, B, a->grad_lambda[l], stop, w32, s));
-            else ARD_TRY(block_backward(h, l, b, B, a->grad_lambda[l], stop, w, s));
+            const float* gr = o->grad_layers_residuals[l];
+            const RowAddend ext{gr ? gr + (long long)b * T * C : nullptr, T, (long long)depth * T * C};
+            const float* pg = o->grad_layers_attention[l];
+            if (fp32) ARD_TRY(block_backward_fp32(h, fws, l, b, B, a->grad_lambda[l], stop, w32, s, ext, pg));
+            else ARD_TRY(block_backward(h, l, b, B, a->grad_lambda[l], stop, w, s, ext, pg));
             if (stop) return 0;
         }
         if (l > 0) {   // PatchMerging backward: reduction Linear (no bias) dgrad, then gather + LayerNorm(4C) backward

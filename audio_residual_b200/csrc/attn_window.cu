@@ -281,16 +281,17 @@ __global__ void __launch_bounds__(128) window_attention_kernel(const __nv_bfloat
 // probabilities are recomputed from the saved qkv (no S/P in HBM), and with P, dS in registers
 //   dP = dO V^T,  delta = rowsum(dP . P),  dS = P . (dP - delta),  dQ = dS K        (per warp: its 16 query rows)
 //   dV = P^T dO,  dK = dS^T Q                                                        (per warp: 16 KEY rows, P/dS via smem + ldmatrix.trans)
+// GP: a probability gradient (ProbGrad) is added to dP before delta, read in the m16n8k16 accumulator layout of dp.
 constexpr int ATB_TILE_BYTES = 4 * AT_HEADS * 64 * 64;            // q, k, v, dO
 constexpr int ATB_PS_BYTES = 2 * 64 * 128;                        // P and dS of the head in flight (bf16 [64 q][64 keys])
 constexpr int ATB_SMEM_BYTES = ATB_TILE_BYTES + ATB_PS_BYTES + AT_HEADS * 232 * 4 + 2 * 64 * 4;
 
 ARD_DEVINL uint32_t ptile_off(int row, int unit) { return (uint32_t)(row * 128 + ((unit ^ (row & 7)) << 4)); }
 
-template <int HD>
+template <int HD, bool GP = false>
 __global__ void __launch_bounds__(128) window_attention_bwd_kernel(const __nv_bfloat16* __restrict__ qkv, const __nv_bfloat16* __restrict__ dout,
                                                                    __nv_bfloat16* __restrict__ dqkv, const float* __restrict__ bias_table,
-                                                                   int H, int W, int C, int nH, int shift) {
+                                                                   int H, int W, int C, int nH, int shift, ProbGrad<GP> pg = {}) {
     constexpr int UPH = HD / 8;
     constexpr int UPR = AT_HEADS * UPH;
     constexpr int NT_O = HD / 8;
@@ -431,6 +432,18 @@ __global__ void __launch_bounds__(128) window_attention_bwd_kernel(const __nv_bf
         sum1 += __shfl_xor_sync(0xffffffffu, sum1, 1);
         sum1 += __shfl_xor_sync(0xffffffffu, sum1, 2);
         const float inv0 = 1.0f / sum0, inv1 = 1.0f / sum1;
+        if constexpr (GP) {   // dp[nt][e]: query row r0, key nt*8 + (lane&3)*2 + e; dp[nt][2+e]: row r0 + 8
+            const float* gp = pg.p + ((long long)wflat * nH + g * AT_HEADS + hh) * 4096 + r0 * 64 + (lane & 3) * 2;
+#pragma unroll
+            for (int nt = 0; nt < 8; ++nt) {
+                const float2 a = __ldg(reinterpret_cast<const float2*>(gp + nt * 8));
+                const float2 c = __ldg(reinterpret_cast<const float2*>(gp + 8 * 64 + nt * 8));
+                dp[nt][0] = fmaf(pg.scale, a.x, dp[nt][0]);
+                dp[nt][1] = fmaf(pg.scale, a.y, dp[nt][1]);
+                dp[nt][2] = fmaf(pg.scale, c.x, dp[nt][2]);
+                dp[nt][3] = fmaf(pg.scale, c.y, dp[nt][3]);
+            }
+        }
         float d0 = 0.f, d1 = 0.f;
 #pragma unroll
         for (int nt = 0; nt < 8; ++nt)
@@ -528,7 +541,7 @@ __global__ void __launch_bounds__(128) window_attention_bwd_kernel(const __nv_bf
     }
 }
 
-int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, cudaStream_t s) {
+int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bfloat16* dqkv, cudaStream_t s, const float* pgrad, float pscale) {
     if (a.B <= 0) return 0;
     if (a.nH <= 0 || a.C % a.nH != 0) return set_error(ARD_ERR_SHAPE, "window_attention_bwd: C=%d not divisible by heads=%d", a.C, a.nH);
     const int hd = a.C / a.nH;
@@ -541,10 +554,22 @@ int window_attention_bwd(const AttnArgs& a, const __nv_bfloat16* dout, __nv_bflo
     if (!attr_set) {
         ARD_CUDA(cudaFuncSetAttribute(window_attention_bwd_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATB_SMEM_BYTES));
         ARD_CUDA(cudaFuncSetAttribute(window_attention_bwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATB_SMEM_BYTES));
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_bwd_kernel<24, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATB_SMEM_BYTES));
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_bwd_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ATB_SMEM_BYTES));
         attr_set = true;
     }
     const double tokens = (double)a.B * a.H * a.W;
-    ProfScope ps(PROF_ATTN, s, 10.0 * tokens * 64 * a.C, tokens * a.C * 2.0 * 7.0);
+    ProfScope ps(PROF_ATTN, s, 10.0 * tokens * 64 * a.C, tokens * a.C * 2.0 * 7.0 + (pgrad ? tokens * a.nH * 64 * 4.0 : 0.0));
+    if (pgrad) {
+        const ProbGrad<true> pg{pgrad, pscale};
+        if (hd == 24)
+            window_attention_bwd_kernel<24, true><<<(unsigned)blocks, 128, ATB_SMEM_BYTES, s>>>(a.qkv, dout, dqkv, a.bias_table, a.H, a.W, a.C, a.nH, shift, pg);
+        else if (hd == 32)
+            window_attention_bwd_kernel<32, true><<<(unsigned)blocks, 128, ATB_SMEM_BYTES, s>>>(a.qkv, dout, dqkv, a.bias_table, a.H, a.W, a.C, a.nH, shift, pg);
+        else
+            return set_error(ARD_ERR_SHAPE, "window_attention_bwd: head_dim %d unsupported (24 or 32)", hd);
+        return check_cuda(cudaGetLastError(), "window_attention_bwd launch");
+    }
     if (hd == 24)
         window_attention_bwd_kernel<24><<<(unsigned)blocks, 128, ATB_SMEM_BYTES, s>>>(a.qkv, dout, dqkv, a.bias_table, a.H, a.W, a.C, a.nH, shift);
     else if (hd == 32)

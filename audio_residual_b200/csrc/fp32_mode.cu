@@ -18,13 +18,19 @@ namespace ard {
 
 // ------------------------------------------------------------------------------------------------ splitting
 // in [rows, C] fp32 (row stride ld_in) -> out [rows, 3C] bf16 = [hi | hi | lo]   (activation form)
+// EXT: the split of in + ext (RowAddend: a layers_residuals gradient entering the dgrad operand only)
+template <bool EXT = false>
 __global__ void __launch_bounds__(256) split3_act_kernel(const float* __restrict__ in, long long ld_in, __nv_bfloat16* __restrict__ out,
-                                                        long long rows, int C) {
+                                                        long long rows, int C, RowAddend ext = RowAddend()) {
     const long long total = rows * (C / 4);
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long r = i / (C / 4);
         const int c = (int)(i - r * (C / 4)) * 4;
-        const float4 v = *reinterpret_cast<const float4*>(in + r * ld_in + c);
+        float4 v = *reinterpret_cast<const float4*>(in + r * ld_in + c);
+        if constexpr (EXT) {
+            const float4 e = *reinterpret_cast<const float4*>(ext.p + (r / ext.T) * ext.bstride + (r % ext.T) * C + c);
+            v.x += e.x; v.y += e.y; v.z += e.z; v.w += e.w;
+        }
         const float x[4] = {v.x, v.y, v.z, v.w};
         float l[4];
 #pragma unroll
@@ -54,13 +60,14 @@ __global__ void __launch_bounds__(256) split3_weight_kernel(const float* __restr
     }
 }
 
-int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s) {
+int split3_act(const float* in, long long ld_in, __nv_bfloat16* out, long long rows, int C, cudaStream_t s, RowAddend ext) {
     if (rows <= 0) return 0;
     if (C % 4 || ld_in % 4) return set_error(ARD_ERR_SHAPE, "split3: width must be a multiple of 4");
     long long blocks = (rows * (C / 4) + 255) / 256;
     if (blocks > 148 * 16) blocks = 148 * 16;
-    ProfScope ps(PROF_OTHER, s, 0.0, 10.0 * rows * C);
-    split3_act_kernel<<<(unsigned)blocks, 256, 0, s>>>(in, ld_in, out, rows, C);
+    ProfScope ps(PROF_OTHER, s, 0.0, (ext.p ? 14.0 : 10.0) * rows * C);
+    if (ext.p) split3_act_kernel<true><<<(unsigned)blocks, 256, 0, s>>>(in, ld_in, out, rows, C, ext);
+    else split3_act_kernel<<<(unsigned)blocks, 256, 0, s>>>(in, ld_in, out, rows, C);
     return check_cuda(cudaGetLastError(), "split3_act launch");
 }
 static int split3_weight_dev(const float* w_dev, DevBuf& out, long long N, int K, cudaStream_t s) {
@@ -196,10 +203,11 @@ static int window_attention_f32(const float* qkv, float* out, const float* bias_
 template <int HD>
 constexpr int attn_f32_bwd_smem() { return (4 * 64 * (HD + 1) + 2 * 64 * 65 + 225) * 4; }
 
-template <int HD>
+// GP: a probability gradient (ProbGrad) is added to dP before delta.
+template <int HD, bool GP = false>
 __global__ void __launch_bounds__(64) window_attention_f32_bwd_kernel(const float* __restrict__ qkv, const float* __restrict__ dout,
                                                                       float* __restrict__ dqkv, const float* __restrict__ bias_table, int R,
-                                                                      int C, int nH, int shift) {
+                                                                      int C, int nH, int shift, ProbGrad<GP> pg = {}) {
     extern __shared__ float sm[];
     float (*Qs)[HD + 1] = reinterpret_cast<float (*)[HD + 1]>(sm);
     float (*Ks)[HD + 1] = Qs + 64;
@@ -262,6 +270,8 @@ __global__ void __launch_bounds__(64) window_attention_f32_bwd_kernel(const floa
     }
     const float inv = 1.0f / sum;
     float delta = 0.f;
+    const float* gp = nullptr;
+    if constexpr (GP) gp = pg.p + ((b * nW + win) * nH + h) * 4096 + i * 64;   // (window, head, query row i)
 #pragma unroll
     for (int j = 0; j < 64; ++j) {                                  // P to smem, dP into sc
         const float p = sc[j] * inv;
@@ -269,6 +279,7 @@ __global__ void __launch_bounds__(64) window_attention_f32_bwd_kernel(const floa
         float dp = 0.f;
 #pragma unroll
         for (int d = 0; d < HD; ++d) dp = fmaf(go[d], Vs[j][d], dp);
+        if constexpr (GP) dp = fmaf(pg.scale, __ldg(gp + j), dp);
         sc[j] = dp;
         delta = fmaf(dp, p, delta);
     }
@@ -306,7 +317,7 @@ __global__ void __launch_bounds__(64) window_attention_f32_bwd_kernel(const floa
 }
 
 int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, const float* bias_table, int B, int R, int C, int nH, int shift,
-                             cudaStream_t s) {
+                             cudaStream_t s, const float* pgrad, float pscale) {
     if (B <= 0 || R <= 0 || R % 8 || nH <= 0 || C % nH)
         return set_error(ARD_ERR_SHAPE, "window_attention_f32_bwd: unsupported shape B=%d R=%d C=%d nH=%d", B, R, C, nH);
     const int hd = C / nH;
@@ -318,9 +329,20 @@ int window_attention_f32_bwd(const float* qkv, const float* dout, float* dqkv, c
     if (!attr_set) {
         ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<24>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<24>()));
         ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<32>()));
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<24, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<24>()));
+        ARD_CUDA(cudaFuncSetAttribute(window_attention_f32_bwd_kernel<32, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, attn_f32_bwd_smem<32>()));
         attr_set = true;
     }
-    ProfScope ps(PROF_ATTN, s, 10.0 * 64 * 64 * hd * ctas, 28.0 * B * R * R * C);
+    ProfScope ps(PROF_ATTN, s, 10.0 * 64 * 64 * hd * ctas, 28.0 * B * R * R * C + (pgrad ? 16384.0 * ctas : 0.0));
+    if (pgrad) {
+        const ProbGrad<true> pg{pgrad, pscale};
+        if (hd == 24)
+            window_attention_f32_bwd_kernel<24, true><<<(unsigned)ctas, 64, attn_f32_bwd_smem<24>(), s>>>(qkv, dout, dqkv, bias_table, R, C, nH, sh, pg);
+        else if (hd == 32)
+            window_attention_f32_bwd_kernel<32, true><<<(unsigned)ctas, 64, attn_f32_bwd_smem<32>(), s>>>(qkv, dout, dqkv, bias_table, R, C, nH, sh, pg);
+        else return set_error(ARD_ERR_SHAPE, "window_attention_f32_bwd: head dim %d unsupported (24 or 32)", hd);
+        return check_cuda(cudaGetLastError(), "window_attention_f32_bwd launch");
+    }
     if (hd == 24)
         window_attention_f32_bwd_kernel<24><<<(unsigned)ctas, 64, attn_f32_bwd_smem<24>(), s>>>(qkv, dout, dqkv, bias_table, R, C, nH, sh);
     else if (hd == 32)

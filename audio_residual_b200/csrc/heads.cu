@@ -337,6 +337,85 @@ __global__ void fine_grained_kernel(const float* __restrict__ normed, float* __r
     }
 }
 
+// Backward of tscam_finish: dY[b*32 + T', o] = dL/dy[o][T'] from the pre-sigmoid y, for o < Kp (columns 527.. are zero, the
+// K padding of the dgrad GEMM). Clipwise: g_clip * sigma'(mean y) / 32 (mean over the 32 steps); framewise: sigma'(y) times the
+// sum of its 32 repeats (interpolate x32, utils.py:209-224). One CTA per (clip, T'), threads over classes. Output bf16 [rows, Kp]
+// or, split3, the split activation form [hi | hi | lo] [rows, 3 Kp] of the fp32-grade dgrad.
+__global__ void __launch_bounds__(256) tscam_bwd_dy_kernel(const float* __restrict__ y, int ldy, const float* __restrict__ g_frame,
+                                                          const float* __restrict__ g_clip, __nv_bfloat16* __restrict__ dY, int Kp, int NC,
+                                                          bool split3) {
+    const long long row = blockIdx.x;
+    const long long b = row / 32;
+    const int Tp = (int)(row % 32);
+    for (int o = threadIdx.x; o < Kp; o += blockDim.x) {
+        float d = 0.f;
+        if (o < NC) {
+            if (g_clip) {
+                float s = 0.f;
+                for (int t = 0; t < 32; ++t) s += y[(b * 32 + t) * ldy + o];
+                const float sg = 1.0f / (1.0f + expf(-s * (1.0f / 32.0f)));
+                d = g_clip[b * NC + o] * sg * (1.0f - sg) * (1.0f / 32.0f);
+            }
+            if (g_frame) {
+                const float sg = 1.0f / (1.0f + expf(-y[row * ldy + o]));
+                float gs = 0.f;
+                for (int r = 0; r < 32; ++r) gs += g_frame[(b * 1024 + Tp * 32 + r) * NC + o];
+                d = fmaf(gs, sg * (1.0f - sg), d);
+            }
+        }
+        const __nv_bfloat16 hi = __float2bfloat16_rn(d);
+        if (split3) {
+            __nv_bfloat16* r3 = dY + row * 3 * Kp;
+            r3[o] = hi;
+            r3[Kp + o] = hi;
+            r3[2 * Kp + o] = __float2bfloat16_rn(d - __bfloat162float(hi));
+        } else {
+            dY[row * Kp + o] = hi;
+        }
+    }
+}
+
+// dL/d normed [B, 64, C] (token f*8 + t) = g_emb / 64 (token mean, htsat.py:810-811)
+//   + col2im of dA [B*32, 6C] (the inverse of tscam_im2col_kernel: tokens (g*2 + fb)*8 + t feed column (c, fb, kw) of row T' = g*8+t-kw+1)
+//   + g_fine summed over its 32 repeats / 2 (mean over the 2 frequency bins, htsat.py:807-808)
+__global__ void tail_token_grad_kernel(const float* __restrict__ g_emb, const float* __restrict__ dA, const float* __restrict__ g_fine,
+                                       float* __restrict__ out, int B, int C) {
+    const long long total = (long long)B * 64 * C;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int c = (int)(i % C);
+        const int tok = (int)((i / C) % 64);
+        const long long b = i / (64LL * C);
+        const int f = tok >> 3, t = tok & 7, fb = f & 1;
+        const int tt = (f >> 1) * 8 + t;
+        float v = g_emb ? g_emb[b * C + c] * (1.0f / 64.0f) : 0.f;
+        if (dA) {
+#pragma unroll
+            for (int kw = 0; kw < 3; ++kw) {
+                const int Tp = tt - kw + 1;
+                if (Tp >= 0 && Tp < 32) v += dA[(b * 32 + Tp) * 6LL * C + c * 6 + fb * 3 + kw];
+            }
+        }
+        if (g_fine) {
+            float s = 0.f;
+            for (int r = 0; r < 32; ++r) s += g_fine[(b * 1024 + tt * 32 + r) * C + c];
+            v = fmaf(0.5f, s, v);
+        }
+        out[i] = v;
+    }
+}
+
+int tscam_bwd_dy(const float* y, int ldy, const float* g_frame, const float* g_clip, __nv_bfloat16* dY, int Kp, int B, bool split3,
+                 cudaStream_t s) {
+    ProfScope ps(PROF_HEAD, s, 0.0, 4.0 * B * 32 * ARD_CLASS_NUM * (1 + (g_clip ? 1 : 0) + (g_frame ? 33 : 0)));
+    tscam_bwd_dy_kernel<<<B * 32, 256, 0, s>>>(y, ldy, g_frame, g_clip, dY, Kp, ARD_CLASS_NUM, split3);
+    return check_cuda(cudaGetLastError(), "tscam_bwd_dy launch");
+}
+int tail_token_grad(const float* g_emb, const float* dA, const float* g_fine, float* out, int B, int C, cudaStream_t s) {
+    ProfScope ps(PROF_HEAD, s, 0.0, 4.0 * B * 64 * C * (1 + (dA ? 3 : 0) + (g_fine ? 16 : 0)));
+    tail_token_grad_kernel<<<148 * 8, 256, 0, s>>>(g_emb, dA, g_fine, out, B, C);
+    return check_cuda(cudaGetLastError(), "tail_token_grad launch");
+}
+
 int tscam_im2col(const float* normed, __nv_bfloat16* A, int B, int C, cudaStream_t s) {
     tscam_im2col_kernel<<<148 * 8, 256, 0, s>>>(normed, A, B, C);
     return check_cuda(cudaGetLastError(), "tscam_im2col launch");

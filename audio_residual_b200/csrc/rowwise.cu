@@ -295,11 +295,13 @@ namespace ard {
 //   dx = rstd * (gg - mean(gg) - xhat * mean(gg * xhat)),  gg = g * gamma;   out = (add ? add : 0) + dx   (fp32)
 // Rows may be the PatchMerging gather (MergeRows): x is read and dx written through the same row map.
 //   out = add_scale * add + dx  (fp32);   out_bf = bf16(add + dx)  (optional: the next dgrad GEMM's A operand)
-template <int VEC, int NV, class Rows>
+// EXT: out_bf = bf16(add + dx + ext), ext read at row r = clip * ext.T + t from ext.p + clip * ext.bstride + t * C (a block's rows of a
+// layers_residuals gradient, which reaches the dgrad operand only, never the fp32 shortcut gradient `out`).
+template <int VEC, int NV, class Rows, bool EXT = false>
 __global__ void __launch_bounds__(256) layernorm_bwd_kernel(Rows xrows, Rows orows, float* __restrict__ out_base,
                                                            const float* __restrict__ g, const float* __restrict__ gamma,
                                                            const float* __restrict__ add, float add_scale,
-                                                           __nv_bfloat16* __restrict__ out_bf, long long nrows) {
+                                                           __nv_bfloat16* __restrict__ out_bf, long long nrows, RowAddend ext = RowAddend()) {
     constexpr int C = 32 * VEC * NV;
     const int lane = threadIdx.x & 31;
     const long long row = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
@@ -350,19 +352,27 @@ __global__ void __launch_bounds__(256) layernorm_bwd_kernel(Rows xrows, Rows oro
             const float d = rstd * (gg[i][k] - m1 - v[i][k] * m2);
             const float a = add != nullptr ? add[op - out_base + k] : 0.f;
             op[k] = fmaf(add_scale, a, d);
-            if (out_bf != nullptr) out_bf[op - out_base + k] = __float2bfloat16_rn(a + d);
+            if constexpr (EXT) {
+                out_bf[op - out_base + k] = __float2bfloat16_rn(a + d + ext.p[(row / ext.T) * ext.bstride + (row % ext.T) * C + e + k]);
+            } else {
+                if (out_bf != nullptr) out_bf[op - out_base + k] = __float2bfloat16_rn(a + d);
+            }
         }
     }
 }
 
 template <class Rows>
 static int launch_ln_bwd(Rows xr, Rows orr, float* out, const float* g, const float* gamma, const float* add, float add_scale,
-                         __nv_bfloat16* out_bf, long long nrows, int C, cudaStream_t s) {
+                         __nv_bfloat16* out_bf, long long nrows, int C, cudaStream_t s, RowAddend ext = RowAddend()) {
     const int wpb = 8;
     const unsigned grid = (unsigned)((nrows + wpb - 1) / wpb);
-    ProfScope ps(PROF_LN, s, 16.0 * nrows * C, ((add ? 16.0 : 12.0) + (out_bf ? 2.0 : 0.0)) * nrows * C);
-#define ARD_LNB_CASE(c, vec, nv) \
-    case c: layernorm_bwd_kernel<vec, nv, Rows><<<grid, wpb * 32, 0, s>>>(xr, orr, out, g, gamma, add, add_scale, out_bf, nrows); break;
+    if (ext.p && !out_bf) return set_error(ARD_ERR_SHAPE, "layernorm_bwd: the addend goes to the bf16 copy only");
+    ProfScope ps(PROF_LN, s, 16.0 * nrows * C, ((add ? 16.0 : 12.0) + (out_bf ? 2.0 : 0.0) + (ext.p ? 4.0 : 0.0)) * nrows * C);
+#define ARD_LNB_CASE(c, vec, nv)                                                                                                           \
+    case c:                                                                                                                                \
+        if (ext.p) layernorm_bwd_kernel<vec, nv, Rows, true><<<grid, wpb * 32, 0, s>>>(xr, orr, out, g, gamma, add, add_scale, out_bf, nrows, ext); \
+        else layernorm_bwd_kernel<vec, nv, Rows><<<grid, wpb * 32, 0, s>>>(xr, orr, out, g, gamma, add, add_scale, out_bf, nrows);         \
+        break;
     switch (C) {
         ARD_LNB_CASE(96, 1, 3)
         ARD_LNB_CASE(128, 4, 1)
@@ -381,9 +391,9 @@ static int launch_ln_bwd(Rows xr, Rows orr, float* out, const float* g, const fl
 }
 
 int layernorm_bwd(const float* x, const float* g, const float* gamma, const float* add, float* out, long long rows, int C, cudaStream_t s,
-                  float add_scale, __nv_bfloat16* out_bf) {
+                  float add_scale, __nv_bfloat16* out_bf, RowAddend ext) {
     if (rows <= 0) return 0;
-    return launch_ln_bwd(PlainRows{x, C}, PlainRows{out, C}, out, g, gamma, add, add_scale, out_bf, rows, C, s);
+    return launch_ln_bwd(PlainRows{x, C}, PlainRows{out, C}, out, g, gamma, add, add_scale, out_bf, rows, C, s, ext);
 }
 
 // PatchMerging backward of the gather + LayerNorm(4C): g [B*(H/2)*(W/2), 4C] -> dx [B, H*W, C] (every source element appears once)

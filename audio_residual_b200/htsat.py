@@ -367,8 +367,11 @@ class HTSAT_Swin_Transformer(nn.Module):
     def encode(self, waveform=None, mel_fusion=None, quantize=False, want_dict=False, want_audio_embed=False,
                want_capture=True, save_for_backward=False, want_head_outputs=False, precision=None):
         """Single entry to ard_encoder_forward. Returns a dict of freshly allocated CUDA tensors.
-        With grad enabled and trainable ResiDual lambdas, `embedding` / `audio_embed` come back attached to the autograd graph
-        (backward = ard_encoder_backward, filling `learnable.grad` as loss.backward() does in src/training.py:30-32).
+        With grad enabled and trainable ResiDual lambdas, every output the reference can differentiate w.r.t. the lambdas comes back
+        attached to the autograd graph: `embedding`, `audio_embed`, `framewise_output`, `clipwise_output`, `fine_grained_embedding`
+        and each tensor of `layers_residuals` and `layers_attention` (backward = ard_encoder_backward_outputs, filling
+        `learnable.grad` as loss.backward() does in src/training.py:30-32; a lambda no used output depends on gets no gradient).
+        `head_outputs` is not a reference output and is never differentiable.
         want_head_outputs: also return `head_outputs`, per layer [depth, B*nW, nH, 64, hd]: every block's per-head `attn @ v`
         (htsat.py:354). precision: "bf16" (default) or "fp32" (3-term split-bf16 GEMMs + fp32 attention, rel. err <= 1e-4);
         None takes the encoder's `precision` attribute. The autograd route runs at the encoder's `train_precision` instead;
@@ -474,21 +477,31 @@ class HTSAT_Swin_Transformer(nn.Module):
         return L.load().ard_last_launch_count(self._hb.h) if self._hb.h is not None else 0
 
 
+_TAIL_KEYS = ("framewise_output", "clipwise_output", "fine_grained_embedding")
+
+
 class _EncodeFn(torch.autograd.Function):
-    """autograd node around ard_encoder_forward(save_for_backward=1) / ard_encoder_backward. Inputs: the per-layer lambda
-    parameters (only to receive gradients; their values reach the library through _sync_residuals)."""
+    """autograd node around ard_encoder_forward(save_for_backward=1) / ard_encoder_backward_outputs. Inputs: the per-layer lambda
+    parameters (only to receive gradients; their values reach the library through _sync_residuals). Outputs: every tensor of the
+    forward's output dict that the reference can differentiate w.r.t. ResiDual.learnable (htsat.py:797-832): `embedding`,
+    `audio_embed`, the tail keys and the per-layer captures. Unused outputs get no gradient tensor (set_materialize_grads(False))
+    and reach the library as NULL."""
 
     @staticmethod
     def forward(ctx, enc, kw, holder, *lams):
+        ctx.set_materialize_grads(False)
         out = enc.encode(save_for_backward=True, **kw)
         holder.update(out)
         ctx.enc, ctx.B = enc, out["embedding"].shape[0]
         ctx.generation = out["_tape_generation"]   # the handle keeps ONE tape: a later training forward invalidates this node
         ctx.layers = [i for i, p in enumerate(enc._lambda_params()) if p is not None]
         ctx.ks = [p.shape[0] for p in enc._lambda_params() if p is not None]
-        ctx.has_audio = "audio_embed" in out
         ctx.devs = [p.device for p in enc._lambda_params() if p is not None]
-        return (out["embedding"], out["audio_embed"]) if ctx.has_audio else (out["embedding"],)
+        # lambda_l acts from the first patched block of layer l on; a layer's attention maps are those of blocks after it
+        ctx.attn_reach = {l: next(b for b, blk in enumerate(enc.layers[l].blocks) if blk._residual is not None) < enc.depths[l] - 1
+                          for l in ctx.layers}
+        ctx.keys = _output_keys(out, enc.num_layers)
+        return tuple(out[k] if l is None else out[k][l] for k, l in ctx.keys)
 
     @staticmethod
     def backward(ctx, *grads):
@@ -498,23 +511,41 @@ class _EncodeFn(torch.autograd.Function):
         a = L.ArdBackwardArgs()
         a.B = ctx.B
         a.generation = ctx.generation
+        o = L.ArdOutputGrads()
         keep = []
-        g_emb = grads[0]
-        g_ae = grads[1] if ctx.has_audio else None
-        if g_emb is not None:
-            g_emb = g_emb.detach().to(dev, torch.float32).contiguous()
-            a.grad_embedding = g_emb.data_ptr()
-        if g_ae is not None:
-            g_ae = g_ae.detach().to(dev, torch.float32).contiguous()
-            a.grad_audio_embed = g_ae.data_ptr()
+        # what the given gradients reach: everything (a head / tail key), the lambdas of layers <= top_res (residuals: the
+        # patched blocks' own r), and those of layers < top_attn, or == top_attn with a block after the first patched one
+        head, top_res, top_attn = False, -1, -1
+        for (k, l), g in zip(ctx.keys, grads):
+            if g is None:
+                continue
+            g = g.detach().to(dev, torch.float32).contiguous()
+            keep.append(g)
+            if k == "layers_residuals":
+                o.grad_layers_residuals[l] = g.data_ptr()
+                top_res = max(top_res, l)
+                continue
+            if k == "layers_attention":
+                o.grad_layers_attention[l] = g.data_ptr()
+                top_attn = max(top_attn, l)
+                continue
+            head = True
+            if k == "embedding":
+                a.grad_embedding = g.data_ptr()
+            elif k == "audio_embed":
+                a.grad_audio_embed = g.data_ptr()
+            else:
+                setattr(o, "grad_" + k, g.data_ptr())
+        # lambda_l reaches every output from its first patched block on: the head and tail, and the residuals of layers >= l
+        reached = [head or l <= top_res or l < top_attn or (l == top_attn and ctx.attn_reach[l]) for l in ctx.layers]
         outs = {}
         for l, k in zip(ctx.layers, ctx.ks):
             outs[l] = torch.empty(k, device=dev, dtype=torch.float32)
             a.grad_lambda[l] = outs[l].data_ptr()
-        with torch.cuda.device(dev):
-            L.check(lib.ard_encoder_backward(enc._hb.h, C.byref(a), L.stream_ptr()))
-        keep.extend([g_emb, g_ae])
-        return (None, None, None) + tuple(outs[l].to(d) for l, d in zip(ctx.layers, ctx.devs))
+        if any(reached):
+            with torch.cuda.device(dev):
+                L.check(lib.ard_encoder_backward_outputs(enc._hb.h, C.byref(a), C.byref(o), L.stream_ptr()))
+        return (None, None, None) + tuple(outs[l].to(d) if r else None for l, d, r in zip(ctx.layers, ctx.devs, reached))
 
 
 def _encode_with_grad(enc, lams, waveform, mel_fusion, quantize, want_dict, want_audio_embed, want_capture, precision):
@@ -523,11 +554,21 @@ def _encode_with_grad(enc, lams, waveform, mel_fusion, quantize, want_dict, want
     holder = {}
     live = [p for p in lams if p is not None]
     res = _EncodeFn.apply(enc, kw, holder, *live)
-    out = dict(holder)
-    out["embedding"] = res[0]
-    if want_audio_embed:
-        out["audio_embed"] = res[1]
+    out = {k: list(v) if isinstance(v, list) else v for k, v in holder.items()}
+    for i, (k, l) in enumerate(_output_keys(holder, enc.num_layers)):
+        if l is None:
+            out[k] = res[i]
+        else:
+            out[k][l] = res[i]
     return out
+
+
+def _output_keys(out, num_layers):
+    """The differentiable outputs of _EncodeFn in order (the same list its forward builds)."""
+    keys = [("embedding", None)] + [(k, None) for k in ("audio_embed",) + _TAIL_KEYS if k in out]
+    if "layers_residuals" in out:
+        keys += [(k, l) for k in ("layers_residuals", "layers_attention") for l in range(num_layers)]
+    return keys
 
 
 def create_htsat_model(audio_cfg, enable_fusion=False, fusion_type="None"):

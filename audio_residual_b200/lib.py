@@ -37,6 +37,11 @@ class ArdBackwardArgs(C.Structure):
                 ("generation", C.c_longlong)]
 
 
+class ArdOutputGrads(C.Structure):
+    _fields_ = [("grad_framewise_output", C.c_void_p), ("grad_clipwise_output", C.c_void_p), ("grad_fine_grained_embedding", C.c_void_p),
+                ("grad_layers_residuals", C.c_void_p * 4), ("grad_layers_attention", C.c_void_p * 4)]
+
+
 _lib = None
 
 
@@ -69,6 +74,10 @@ def load(check_symbols=False):
         lib.ard_set_layer_lambda.argtypes = [vp, i, vp, vp]
         lib.ard_encoder_forward.argtypes = [vp, C.POINTER(ArdForwardArgs), vp]
         lib.ard_encoder_backward.argtypes = [vp, C.POINTER(ArdBackwardArgs), vp]
+        lib.ard_encoder_backward_outputs.argtypes = [vp, C.POINTER(ArdBackwardArgs), C.POINTER(ArdOutputGrads), vp]
+        lib.ard_window_attention_bwd_pgrad.argtypes = [vp, vp, vp, f, vp, vp, i, i, i, i, i, i, vp]
+        lib.ard_window_attention_f32_bwd_pgrad.argtypes = [vp, vp, vp, f, vp, vp, i, i, i, i, i, i, vp]
+        lib.ard_tail_backward.argtypes = [vp, vp, i, vp, vp, vp, vp, i, i, vp, vp]
         lib.ard_block_forward.argtypes = [vp, i, i, vp, i, vp, vp, vp, vp]
         lib.ard_attention_block.argtypes = [vp, i, i, vp, i, vp, vp]
         lib.ard_workspace_bytes.argtypes = [vp]

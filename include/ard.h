@@ -113,7 +113,7 @@ int ard_encoder_forward(ard_handle* h, const ard_forward_args* args, void* strea
  * vectors. The encoder is frozen and in eval mode (src/training.py:105-108), so no weight gradients exist.
  * It runs at the precision of that forward: bf16 tensor-core dgrads (precision 0), or fp32-grade (precision 1: 3-term
  * split-bf16 dgrads, fp32 attention backward / gelu' / LayerNorm backward; rel. err <= 1e-4 vs the reference's fp32 autograd).
- * Inputs are dL/d(audio_embed) and/or dL/d(embedding); grad_lambda[l] (device [K_l] fp32, required for every layer that
+ * Inputs are dL/d(audio_embed) and/or dL/d(embedding) (the other output keys: ard_encoder_backward_outputs); grad_lambda[l] (device [K_l] fp32, required for every layer that
  * carries a ResiDual) is OVERWRITTEN with the gradient summed over the layer's patched blocks, which share one
  * ResiDual module in the reference (src/residual.py:186-197). */
 typedef struct ard_backward_args {
@@ -125,6 +125,30 @@ typedef struct ard_backward_args {
                                               * different saved forward on the handle since then -> ARD_ERR_STATE. 0: unchecked */
 } ard_backward_args;
 int ard_encoder_backward(ard_handle* h, const ard_backward_args* args, void* stream);
+/* Gradients of the other keys of output_dict (htsat.py:825-832) for ard_encoder_backward_outputs; every one of them is
+ * differentiable w.r.t. ResiDual.learnable in the reference (htsat.py:797-832, src/residual.py:58-98). All device fp32, NULL when
+ * the loss does not use that output. The tail keys need a saved forward that computed them (ARD_ERR_STATE otherwise). */
+typedef struct ard_output_grads {
+    const float* grad_framewise_output;       /* [B, 1024, 527]          sigmoid(tscam_conv) repeated x32, htsat.py:813-818 */
+    const float* grad_clipwise_output;        /* [B, 527]                sigmoid(mean_t tscam_conv), htsat.py:820-821 */
+    const float* grad_fine_grained_embedding; /* [B, 1024, 8*embed_dim]  frequency-bin mean repeated x32, htsat.py:807-808 */
+    const float* grad_layers_residuals[ARD_MAX_LAYERS]; /* [B, depth_l*T_l, C_l]: block b's residual_x (post-ResiDual r of a patched
+                                               * block, src/residual.py:88-89; the projected attention branch of a plain one,
+                                               * htsat.py:476) at rows b*T_l .. (b+1)*T_l of each clip (htsat.py:589-596) */
+    const float* grad_layers_attention[ARD_MAX_LAYERS]; /* [B*nW_l, nH_l, 64, 64] block-mean maps (htsat.py:589-595): every
+                                               * block's probabilities receive grad / depth_l, in that block's window order */
+} ard_output_grads;
+/* ard_encoder_backward with the gradients of the other output_dict keys added to the loss (outs may be NULL: then it is exactly
+ * ard_encoder_backward). At least one gradient in args or outs is required. The walk starts at the highest block a given gradient
+ * reaches (a loss on layers_residuals[1] alone never touches stages 2-3 or the tail); grad_lambda of a layer no given gradient
+ * reaches is written with zeros. */
+int ard_encoder_backward_outputs(ard_handle* h, const ard_backward_args* args, const ard_output_grads* outs, void* stream);
+/* Op-level tail backward (the tail part of ard_encoder_backward_outputs, on the handle's tscam_conv weights): grad_normed
+ * [B, 64, 8*embed_dim] = dL / d(final LayerNorm output) for the loss terms given (each NULL when unused): framewise / clipwise
+ * through y = tscam_conv pre-activation [B*32, ldy] fp32 (ldy >= 527, column o of row b*32+t = y[b, o, t]), fine-grained, and
+ * grad_embedding [B, 8*embed_dim] (the token mean). precision 0: bf16 tensor-core dgrad; 1: 3-term split-bf16 dgrad. */
+int ard_tail_backward(ard_handle* h, const float* y, int ldy, const float* grad_framewise, const float* grad_clipwise, const float* grad_fine,
+                      const float* grad_embedding, int B, int precision, float* grad_normed, void* stream);
 /* Serial number of the last ard_encoder_forward(save_for_backward=1) on this handle (0: none). The handle keeps ONE tape:
  * a second training forward overwrites it, and a backward carrying the older number is refused instead of silently using
  * the newer activations. */
@@ -198,6 +222,13 @@ int ard_window_attention_bwd(const void* qkv_bf16, const void* dout_bf16, void* 
  * order (q pre-scaled), dout [B*H*W, C] fp32 -> dqkv [B*H*W, 3C] fp32. H == W, head dim C/nH of 24 or 32; no shift when H == 8. */
 int ard_window_attention_f32_bwd(const float* qkv_f32, const float* dout_f32, float* dqkv_f32, const float* bias_table, int B, int H, int W,
                                  int C, int nH, int shift, void* stream);
+/* The two backwards above with a gradient w.r.t. the attention probabilities as well (a loss on the captured maps,
+ * layers_attention = the block mean of BasicLayer.forward, htsat.py:589-595): dP = dO V^T + pscale * pgrad before the softmax
+ * backward. pgrad fp32 [B*nW, nH, 64, 64], window order of the block (shifted blocks: windows of the rolled image). */
+int ard_window_attention_bwd_pgrad(const void* qkv_bf16, const void* dout_bf16, const float* pgrad, float pscale, void* dqkv_bf16,
+                                   const float* bias_table, int B, int H, int W, int C, int nH, int shift, void* stream);
+int ard_window_attention_f32_bwd_pgrad(const float* qkv_f32, const float* dout_f32, const float* pgrad, float pscale, float* dqkv_f32,
+                                       const float* bias_table, int B, int H, int W, int C, int nH, int shift, void* stream);
 /* Backward of nn.LayerNorm over the last dim: grad_in = (add ? add : 0) + dLN(x)^T grad_out; all fp32 [rows, C]. */
 int ard_layernorm_bwd(const float* x, const float* grad_out, const float* gamma, const float* add, float* grad_in, long long rows, int C,
                       void* stream);
